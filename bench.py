@@ -174,6 +174,14 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------ GPU arm
+def dump_outputs(dirname: str, out: dict):
+    """Write what one step returns to its caller, one float64 DIR/<name>.npy per array: u, ext [B, N], axial [B, M],
+    weight [B] and the per-system status codes info [B] (0: solved).  For bar-942 x 1024 that is 20 MB."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy().astype(np.float64))
+
+
 def run_gpu(args):
     # libraries (NCCL's version banner) may write to fd 1: keep the real stdout for the one JSON line
     real_stdout = os.dup(1)
@@ -337,6 +345,8 @@ def run_gpu(args):
     barrier()
     wall = time.perf_counter() - wall0
     launches = launches_per_step * args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs2[(step_no[0] - 1) & 1] if pipelined else out)
     # instrumented pass: CUDA events around every kernel (they cost a few microseconds per step, hence not in the timed pass)
     _lib.profile_enable(True)
     _lib.profile_read()
@@ -608,7 +618,14 @@ def main():
     ap.add_argument("--configs", default="3,4,5", help="which of the other BASELINE.json configurations to measure as well")
     ap.add_argument("--headline-only", action="store_true",
                     help="skip the shared-factor extra (profiler runs: the launch list then holds the headline step only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (rank 0's batch) to DIR/<name>.npy; the inputs are "
+                         "seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

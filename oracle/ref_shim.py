@@ -1,9 +1,7 @@
 """Import the live reference (``/root/reference``) read-only under a harness shim.
 
-TEST INFRASTRUCTURE ONLY, and only usable in the build container: the GPU box
-has no ``/root/reference``.  Used by ``tests/golden/make_golden.py`` to produce
-the committed ``tests/golden/live_*`` vectors and by the container-only tests
-that validate ``oracle/truss_oracle.py`` against the real thing.
+TEST INFRASTRUCTURE ONLY: used by ``tests/golden/make_golden.py`` to produce the
+committed ``tests/golden/live_*`` vectors, which the tests compare against.
 
 The reference does not import as-is here (SURVEY.md section 8c): ``utils.py:1``
 needs tkinter (``from turtle import position``), ``utils.py:3-4`` / ``plot.py:2,9``

@@ -1,8 +1,6 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -10,14 +8,3 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the live reference at /root/reference (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    from oracle import ref_shim
-
-    if not ref_shim.available():
-        skip = pytest.mark.skip(reason="live reference not present (GPU box)")
-        for item in items:
-            if "reference" in item.keywords:
-                item.add_marker(skip)

@@ -14,10 +14,19 @@ Writes, next to this file:
   live_random.json       seeded random 2D/3D trusses (all support types, parallel members, loads on supports), live results
   live_cube7_aug.json    generator + full augmentation list (example.py:239-267 recipe, 7 cubes), live results
   live_cube7_seed42.json GenerateRandomCubeTrusses(seed=42) inputs as regenerated today (must equal ref_generate inputs)
+  live_kmatrix.npz       GetKMatrix (non-zeros as <case>.i / .j / .v) and the unknown-displacement DOFs (<case>.free) of
+                         every ref_data input
+  live_generate_modes.json.gz  GenerateRandomCubeTrusses in every method / link type / parallel rule (helpers.generator_modes)
+  live_ga_stub_bar25.json   GA.Evolve on bar-25 with a stand-in fitness (helpers.ga_stub_evolve)
+
+The last three were first written by running live_reference_checks() over this package's own truss / generate / ga /
+type modules in place of the reference's, at a revision (d711202) whose tests compared exactly these results with the
+live reference and passed; live_reference_checks(ref_shim.load()) rewrites them from the reference itself.
 """
 from __future__ import annotations
 
 import glob
+import gzip
 import json
 import os
 import random
@@ -184,6 +193,24 @@ def live_cube7(ref, n_aug=48):
     json.dump([t.Serialize() for t in lst], open(os.path.join(HERE, "live_cube7_aug.json"), "w"))
 
 
+def live_reference_checks(ref):
+    from tests import helpers as H
+
+    kmat = {}
+    for f in sorted(glob.glob(os.path.join(HERE, "ref_data", "*_input_*.json"))):
+        name = os.path.basename(f)[:-5]
+        t = ref.truss.Truss(dim_of(name)).LoadFromJSON(f)
+        K = t.GetKMatrix()
+        i, j = np.nonzero(K)
+        kmat.update({name + ".i": i.astype(np.int32), name + ".j": j.astype(np.int32), name + ".v": K[i, j],
+                     name + ".free": np.nonzero(t.GetDisplacementUnknownMask())[0].astype(np.int32)})
+    np.savez_compressed(os.path.join(HERE, "live_kmatrix.npz"), **kmat)
+    modes = {label: [t.Serialize() for t in ref.generate.GenerateRandomCubeTrusses(**kw)] for label, kw in H.generator_modes()}
+    with gzip.open(os.path.join(HERE, "live_generate_modes.json.gz"), "wt") as f:
+        json.dump(modes, f)
+    json.dump(H.ga_stub_evolve(ref.ga, ref.truss, ref.type), open(os.path.join(HERE, "live_ga_stub_bar25.json"), "w"))
+
+
 def main():
     ref = ref_shim.load()
     copy_shipped()
@@ -192,6 +219,7 @@ def main():
     live_loadcases(ref)
     live_random(ref)
     live_cube7(ref)
+    live_reference_checks(ref)
     print("done")
 
 

@@ -4,6 +4,7 @@ from __future__ import annotations
 import glob
 import json
 import os
+import random
 
 import numpy as np
 
@@ -49,6 +50,40 @@ def cube7_shipped():
 
 def load_json(name):
     return json.load(open(os.path.join(GOLDEN, name)))
+
+
+def generator_modes():
+    """[(label, GenerateRandomCubeTrusses kwargs)] over every generation method x link type x parallel-member rule."""
+    from python_stable_3d_truss_analysis_b200.type import GenerateMethod, LinkType
+
+    out = []
+    for method in (GenerateMethod.DFS, GenerateMethod.BFS, GenerateMethod.Random):
+        for link in (LinkType.LeftBottom_RightTop, LinkType.Cross, LinkType.Random):
+            for par in (False, True):
+                kw = dict(gridRange=(4, 3, 3), numCubeRange=(2, 5), numEachRange=(1, 2), method=method, linkType=link,
+                          isAllowParallel=par, isPrintMessage=False, seed=11, nForceRange=(2, None),
+                          memberTypes=[[1., 1e7, 0.1], [2., 2e7, 0.2]])
+                out.append((f"method={method} link={link} parallel={par}", kw))
+    return out
+
+
+def ga_stub_evolve(ga_mod, truss_mod, type_mod):
+    """GA.Evolve on bar-25 with a deterministic stand-in fitness (no solve), given the ga / truss / type modules of an
+    implementation.  The GA operators draw from `random` like ga.py:151-190, so two implementations seeded alike must
+    walk the same populations.  Returns [best gene, its fitness info, final population, history] as JSON-ready lists."""
+    def stub(self, gene):
+        w = float(sum((g + 1) * ((i % 7) + 1) for i, g in enumerate(gene)))
+        return w, (gene[0] % 2 == 0), True
+
+    class StubGA(ga_mod.GA):
+        GetFitness = stub
+
+    data = json.load(open(os.path.join(GOLDEN, "ref_data", "bar-25_input_0.json")))
+    mts = [type_mod.MemberType(i, 1e7, 0.1 * i) for i in range(1, 6)]
+    random.seed(3)
+    gene, info, pop, history = StubGA(truss_mod.Truss(3).LoadFromJSON(data=data), mts, nIteration=6, nPop=30,
+                                      nElite=8).Evolve(False)
+    return [list(gene), list(info), [list(p) for p in pop], list(history)]
 
 
 def assert_close(got: dict, want: dict, tol=TOL, what=""):

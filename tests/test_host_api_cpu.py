@@ -1,11 +1,10 @@
 """Host-side mirror of the reference API, CPU only (nothing here launches a kernel)."""
+import gzip
 import json
-import random
 
 import numpy as np
 import pytest
 
-from oracle import ref_shim
 from oracle import truss_oracle as orc
 from python_stable_3d_truss_analysis_b200.generate import (AddJointNoise, GenerateRandomCubeTrusses, MoveToCentroid,
                                                              NoChange, RandomResetPin, RandomTranslation,
@@ -156,44 +155,18 @@ def test_generator_other_modes_are_deterministic():
             assert all(t.isStable for t in a) and len(a) == 4
 
 
-@pytest.mark.reference
 def test_generator_matches_live_reference_all_modes():
-    ref = ref_shim.load()
-    from python_stable_3d_truss_analysis_b200.type import GenerateMethod, LinkType
-    for method in (GenerateMethod.DFS, GenerateMethod.BFS, GenerateMethod.Random):
-        for link in (LinkType.LeftBottom_RightTop, LinkType.Cross, LinkType.Random):
-            for par in (False, True):
-                kw = dict(gridRange=(4, 3, 3), numCubeRange=(2, 5), numEachRange=(1, 2), method=method, linkType=link,
-                          isAllowParallel=par, isPrintMessage=False, seed=11, nForceRange=(2, None),
-                          memberTypes=[[1., 1e7, 0.1], [2., 2e7, 0.2]])
-                mine = GenerateRandomCubeTrusses(**kw)
-                theirs = ref.generate.GenerateRandomCubeTrusses(**kw)
-                assert [t.Serialize() for t in mine] == [t.Serialize() for t in theirs]
+    with gzip.open(f"{H.GOLDEN}/live_generate_modes.json.gz", "rt") as f:
+        theirs = json.load(f)
+    modes = H.generator_modes()
+    assert list(theirs) == [label for label, _ in modes]
+    for label, kw in modes:
+        assert [t.Serialize() for t in GenerateRandomCubeTrusses(**kw)] == theirs[label], label
 
 
-@pytest.mark.reference
 def test_ga_trajectory_matches_live_reference_with_stub_fitness():
     """The GA operators draw from `random` exactly like ga.py:151-190: with a deterministic stand-in
     fitness (no solve) both implementations must walk the same populations."""
-    ref = ref_shim.load()
-    from python_stable_3d_truss_analysis_b200.ga import GA
+    from python_stable_3d_truss_analysis_b200 import ga, truss, type as types
 
-    def stub(self, gene):
-        w = float(sum((g + 1) * ((i % 7) + 1) for i, g in enumerate(gene)))
-        return w, (gene[0] % 2 == 0), True
-
-    data = json.load(open(f"{H.GOLDEN}/ref_data/bar-25_input_0.json"))
-    mts = [(i, 1e7, 0.1 * i) for i in range(1, 6)]
-
-    class MineGA(GA):
-        GetFitness = stub
-
-    class TheirGA(ref.ga.GA):
-        GetFitness = stub
-
-    random.seed(3)
-    mine = MineGA(Truss(3).LoadFromJSON(data=data), [MemberType(*m) for m in mts], nIteration=6, nPop=30, nElite=8).Evolve(False)
-    random.seed(3)
-    theirs = TheirGA(ref.truss.Truss(3).LoadFromJSON(data=data), [ref.type.MemberType(*m) for m in mts], nIteration=6,
-                     nPop=30, nElite=8).Evolve(False)
-    assert mine[0] == theirs[0] and mine[1] == theirs[1] and mine[2] == theirs[2] and mine[3] == theirs[3]
+    assert H.ga_stub_evolve(ga, truss, types) == H.load_json("live_ga_stub_bar25.json")

@@ -1,11 +1,11 @@
 """Pin the oracle (oracle/truss_oracle.py) against every known-answer vector the reference ships
 and against vectors produced by the live reference (SURVEY.md section 8c).  CPU only."""
 import json
+import os
 
 import numpy as np
 import pytest
 
-from oracle import ref_shim
 from oracle import truss_oracle as orc
 from tests import helpers as H
 
@@ -90,23 +90,24 @@ def test_not_stable_rule():
     orc.solve(3, joints, np.array([1, 1, 1, 0], dtype=np.uint8), conn, aed, f)
 
 
-@pytest.mark.reference
 def test_oracle_vs_live_reference_in_container():
-    """Container-only: the oracle against the real reference imported under the shim."""
-    ref = ref_shim.load()
+    """The oracle against what the reference's Solve(), GetDisplacementUnknownMask() and GetKMatrix() returned
+    (live_solve.json, live_kmatrix.npz; the mask and K bit for bit)."""
+    live_solve = H.load_json("live_solve.json")
+    kmat = np.load(os.path.join(H.GOLDEN, "live_kmatrix.npz"))
     for name, dim, data, _ in H.shipped_cases():
-        t = ref.truss.Truss(dim).LoadFromJSON(data=data)
-        t.Solve()
-        live = ref_shim.dense_results(t)
-        r = orc.solve(dim, *orc.arrays_from_json(data, dim))
+        joints, support, conn, aed, force = orc.arrays_from_json(data, dim)
+        r = orc.solve(dim, joints, support, conn, aed, force)
+        live = {k: np.array(v) if k != "weight" else v for k, v in live_solve[name].items()}
         # 1e-12, not 0: the live dicts drop entries below the 1e-10 cutoff (truss.py:358), the oracle is dense
         H.assert_close(r, live, tol=1e-12, what=name)
-        free_idx, _, _ = orc.dof_maps(dim, orc.arrays_from_json(data, dim)[1])
-        assert np.array_equal(free_idx, np.nonzero(t.GetDisplacementUnknownMask())[0])
-        assert np.array_equal(orc.assemble_K(dim, *[orc.arrays_from_json(data, dim)[i] for i in (0, 2, 3)]), t.GetKMatrix())
+        free_idx, _, _ = orc.dof_maps(dim, support)
+        assert np.array_equal(free_idx, kmat[name + ".free"])
+        K = np.zeros((len(joints) * dim,) * 2)
+        K[kmat[name + ".i"], kmat[name + ".j"]] = kmat[name + ".v"]
+        assert np.array_equal(orc.assemble_K(dim, joints, conn, aed), K), name
 
 
-@pytest.mark.reference
 def test_seed42_generator_inputs_reproduce_shipped():
     regen = H.load_json("live_cube7_seed42.json")
     for (name, _, shipped, _), mine in zip(H.cube7_shipped(), regen):
