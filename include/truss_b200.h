@@ -170,6 +170,22 @@ typedef struct {
   double* react;   /* [B][s]  reaction at supported DOF r     = ext[sup_idx[r]]          */
 } tb_batch_out;
 
+/* Cotangents of tb_solve's outputs for tb_adjoint (device pointers, rows contiguous per system); any may be NULL (= 0). */
+typedef struct {
+  const double* u;          /* [B][N]  entries at supported DOFs are ignored (u is 0 there) */
+  const double* ext;        /* [B][N]  free DOFs flow to the load, supported DOFs through the reactions */
+  const double* axial;      /* [B][M] */
+  const double* weight;     /* [B]    */
+} tb_adj_in;
+
+/* Per-system gradients written by tb_adjoint (device pointers); any but member_aed may be NULL to skip it. */
+typedef struct {
+  double* joint_xyz;        /* [B][nJ][d] */
+  double* member_aed;       /* [B][M][3]  (a, e, density) -- required */
+  double* force;            /* [B][N]     0 at supported DOFs (truss.py:349 overwrites those loads) */
+  int32_t* info;            /* [B]        per-system status (same K, so the forward's); failed system: gradients 0 */
+} tb_adj_out;
+
 /* GA fitness outputs (ga.py:139-149): fitness = weight + penalties; flags[b][0] = stress
  * allowed, flags[b][1] = displacement allowed (truss.py:429-462 with isGetSumViolation). */
 typedef struct {
@@ -200,6 +216,17 @@ int tb_host_wait(tb_plan* plan, uint64_t ticket);
  * tb_solve on the same arguments factorises every system independently (the bench's headline mode). */
 int tb_solve_loadcases(tb_plan* plan, const tb_batch_in* in, const tb_batch_out* out, void* cuda_stream);
 int tb_solve_loadcases_host(tb_plan* plan, const tb_batch_in* in, const tb_batch_out* out);
+
+/* Reverse mode of tb_solve (truss.py:329-364) for B systems: the gradients of L = <grad.u, u> + <grad.ext, ext> +
+ * <grad.axial, axial> + grad.weight * weight with respect to the joint positions, the member properties and the loads,
+ * by one adjoint solve with the same stiffness matrix (K is symmetric) through the plan's own pipeline.  `u` = the
+ * forward's dense displacements of the same inputs (device, [B][N]).  Explicit member properties only (member_aed; a
+ * gene / type-table batch returns TB_ERR_NULL).  Gradients are written per system even for an input shared with stride 0
+ * (reducing them is the caller's job).  shared_factor: the systems are load cases of one truss, as tb_solve_loadcases
+ * (joint_stride and member_stride must be 0; on the band path one factorisation and B substitutions).  Enqueues on the
+ * stream without synchronising; the adjoint scratch is the plan's (grow-only, grown in stream order). */
+int tb_adjoint(tb_plan* plan, const tb_batch_in* in, const double* u, const tb_adj_in* grad, const tb_adj_out* out,
+               int32_t shared_factor, void* cuda_stream);
 
 /* GA.GetFitness for B genes (ga.py:139-149); `full` may be NULL or receive the full results. */
 int tb_fitness(tb_plan* plan, const tb_batch_in* in, double allow_stress, double allow_displace,

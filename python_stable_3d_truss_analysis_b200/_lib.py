@@ -17,7 +17,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_PATH = os.environ.get("TB_LIB_PATH") or os.path.join(CSRC, "libtruss_b200.so")   # TB_LIB_PATH: instrumented builds (tools/)
-SOURCES = ["tb_plan.cu", "tb_tsplan.cu", "tb_small.cu", "tb_dense16.cu", "tb_large.cu", "tb_band.cu", "tb_bandts.cu", "tb_api.cu", "tb_peak.cu",
+SOURCES = ["tb_plan.cu", "tb_tsplan.cu", "tb_small.cu", "tb_dense16.cu", "tb_large.cu", "tb_band.cu", "tb_bandts.cu", "tb_api.cu", "tb_adjoint.cu", "tb_peak.cu",
            "tb_ga.cu", "tb_augment.cu", "tb_json.cu", "tb_gencube.cu"]
 
 TB_ERR_NO_DEVICE = -7
@@ -144,6 +144,14 @@ class TbBatchOut(C.Structure):
                 ("info", C.c_void_p), ("u_free", C.c_void_p), ("react", C.c_void_p)]
 
 
+class TbAdjIn(C.Structure):
+    _fields_ = [("u", C.c_void_p), ("ext", C.c_void_p), ("axial", C.c_void_p), ("weight", C.c_void_p)]
+
+
+class TbAdjOut(C.Structure):
+    _fields_ = [("joint_xyz", C.c_void_p), ("member_aed", C.c_void_p), ("force", C.c_void_p), ("info", C.c_void_p)]
+
+
 class TbFitOut(C.Structure):
     _fields_ = [("fitness", C.c_void_p), ("flags", C.c_void_p), ("info", C.c_void_p)]
 
@@ -155,7 +163,7 @@ class TbRaggedIn(C.Structure):
 
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
-           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
+           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
            "tb_solve_ragged_host", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
@@ -186,6 +194,7 @@ def lib():
     L.tb_host_wait.argtypes = [vp, C.c_uint64]
     L.tb_solve_loadcases.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBatchOut), vp]
     L.tb_solve_loadcases_host.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBatchOut)]
+    L.tb_adjoint.argtypes = [vp, C.POINTER(TbBatchIn), vp, C.POINTER(TbAdjIn), C.POINTER(TbAdjOut), i32, vp]
     L.tb_fitness.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut), vp]
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
@@ -566,6 +575,22 @@ class Plan:
                         _ptr(out.get("info")), _ptr(out.get("u_free")), _ptr(out.get("react")))
         fn = lib().tb_solve_loadcases if shared_factor else lib().tb_solve
         check(fn(self._h, C.byref(bi), C.byref(bo), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def adjoint_device(self, B, xyz, force, aed, u, grads, out, stream=None, shared_factor=False):
+        """Reverse mode of ``solve_device`` (tb_adjoint) on torch CUDA tensors.  ``u`` is the forward's dense [B, N]
+        displacements of the same inputs; ``grads`` maps "u" / "ext" / "axial" / "weight" to cotangents (missing or
+        None = 0); ``out`` maps "joint_xyz" [B, nJ, d], "member_aed" [B, M, 3] (required), "force" [B, N] and "info" [B]
+        to preallocated tensors (missing or None = skipped).  Gradients are per system, also for shared inputs."""
+        import torch
+
+        keep = []
+        bi = self._batch_in(B, xyz, aed, None, None, force, keep)
+        st = torch.cuda.current_stream() if stream is None else stream
+        gi = TbAdjIn(_ptr(grads.get("u")), _ptr(grads.get("ext")), _ptr(grads.get("axial")), _ptr(grads.get("weight")))
+        go = TbAdjOut(_ptr(out.get("joint_xyz")), _ptr(out.get("member_aed")), _ptr(out.get("force")), _ptr(out.get("info")))
+        check(lib().tb_adjoint(self._h, C.byref(bi), _ptr(u), C.byref(gi), C.byref(go), 1 if shared_factor else 0,
+                               C.c_void_p(st.cuda_stream)))
         return out
 
     def fitness_device(self, B, xyz, force, gene, type_table, allow_stress, allow_displace, out, aed=None, stream=None):

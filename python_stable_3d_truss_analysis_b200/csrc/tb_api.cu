@@ -883,6 +883,68 @@ extern "C" int tb_debug_assemble_host(tb_plan* p, const tb_batch_in* in, double*
   return TB_OK;
 }
 
+// Reverse mode of tb_solve (DESIGN.md section 9): adjoint load, the adjoint solve through the plan's own pipeline
+// (K is symmetric: the forward system with force := r), sensitivities.  Everything on the caller's stream.
+extern "C" int tb_adjoint(tb_plan* p, const tb_batch_in* in, const double* u, const tb_adj_in* grad, const tb_adj_out* out,
+                          int32_t shared_factor, void* cuda_stream) {
+  if (!p || !in) return TB_ERR_NULL;
+  if (in->batch > 0 && !in->member_aed) return TB_ERR_NULL;      // (no gradients with respect to a type table)
+  int rc = check_batch_in(p, in);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  if (!u || !grad || !out || !out->member_aed) return TB_ERR_NULL;
+  if (shared_factor) {
+    rc = check_loadcases(in);
+    if (rc) return rc;
+  }
+  rc = check_device(p);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  const int B = in->batch;
+  std::lock_guard<std::mutex> lock(p->mu);
+  rc = ws_acquire(p, st);
+  if (rc) return rc;
+  const bool smem = tb_adjoint_vec_in_smem(p->dim, p->M);
+  const size_t rowN = (size_t)B * p->N * 8, nvec = smem ? 0 : (size_t)B * p->M * p->dim * 8;
+  const size_t need = 2 * Arena::al(rowN) + Arena::al((size_t)B * 4) + nvec;
+  if (p->adj_bytes < need) {                    // stream-ordered: the previous call's kernels are ahead on this stream
+    if (p->adj_buf) TB_CUDA(cudaFreeAsync(p->adj_buf, st));
+    p->adj_buf = nullptr;
+    p->adj_bytes = 0;
+    TB_CUDA(cudaMallocAsync(&p->adj_buf, need, st));
+    p->adj_bytes = need;
+  }
+  char* cur = (char*)p->adj_buf;
+  double* r = take<double>(cur, (size_t)B * p->N);
+  double* lam = take<double>(cur, (size_t)B * p->N);
+  int32_t* info_tmp = take<int32_t>(cur, (size_t)B);
+  TbAdjArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = B; a.dim = p->dim; a.nJ = p->nJ; a.M = p->M; a.N = p->N;
+  a.xyz = in->joint_xyz; a.xyz_stride = in->joint_stride;
+  a.aed = in->member_aed; a.aed_stride = in->member_stride;
+  a.conn = p->d_conn; a.dof2free = p->d_dof2free; a.inc_ptr = p->d_inc_ptr; a.inc_mem = p->d_inc_mem;
+  a.g_u = grad->u; a.g_ext = grad->ext; a.g_axial = grad->axial; a.g_w = grad->weight;
+  a.r = r;
+  a.u = u;
+  a.lam = lam;
+  a.info = out->info ? out->info : info_tmp;
+  a.vec = smem ? nullptr : (double*)cur;
+  a.g_xyz = out->joint_xyz; a.g_aed = out->member_aed; a.g_force = out->force;
+  const int num_sm = p->num_sm > 0 ? p->num_sm : 148;
+  rc = tb_launch_adj_rhs(a, num_sm, st);
+  if (rc) return rc;
+  tb_batch_in ain = *in;                        // same systems, load := r (its supported rows are ignored)
+  ain.force = r;
+  ain.force_stride = p->N;
+  const tb_batch_out aout = {lam, nullptr, nullptr, nullptr, const_cast<int32_t*>(a.info), nullptr, nullptr};
+  rc = run_plan_unlocked(p, &ain, &aout, nullptr, 0.0, 0.0, st, shared_factor ? 1 : 0);
+  if (rc) return rc;
+  rc = tb_launch_sens(a, num_sm, st);
+  if (rc) return rc;
+  return ws_release(p, st);
+}
+
 // pinned host buffers for callers that want full-speed H2D/D2H through the *_host entry points
 extern "C" int tb_pinned_alloc(void** ptr, size_t bytes) {
   if (!ptr) return TB_ERR_NULL;

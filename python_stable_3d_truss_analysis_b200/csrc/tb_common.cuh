@@ -155,6 +155,10 @@ struct tb_plan {
   double* compact_u = nullptr;
   double* compact_ext = nullptr;
   size_t compact_cap_u = 0, compact_cap_ext = 0;   // systems
+  // tb_adjoint scratch (grow-only, grown stream-ordered on the caller's stream): adjoint load and solution [B][N] each,
+  // status [B], and the per-member vectors [B][M][d] when they do not fit shared memory
+  void* adj_buf = nullptr;
+  size_t adj_bytes = 0;
   // pipelined host calls (tb_solve_host_async): TB_ASYNC_SLOTS more staging arenas used in turn by consecutive calls,
   // the events that chain a call's copies and kernels, and the ticket counters (submitted / known to be complete)
   void* stage_async[TB_ASYNC_SLOTS] = {};
@@ -189,6 +193,26 @@ struct TbDivisor {
     return a == 0.0 ? q : __fma_rn(r, y, q);                   // (a zero keeps its sign: the correction would turn -0 into +0)
   }
 };
+
+// Geometry of member (j0, j1) with the reference's roundings (truss.py:19,56-63): dx = x_j1 - x_j0, the length (squares
+// summed in axis order), k = EA/L and the cosines through one shared divisor, and the weight term (a L) density.  Returns
+// the length; k and c are not finite for a zero-length member (the caller checks the length).
+template <int DIM>
+__device__ __forceinline__ double tb_member_geom(const double* xyz, int j0, int j1, double ar, double e, double rho,
+                                                 double dx[DIM], double c[DIM], double& k, double& w) {
+#pragma unroll
+  for (int i = 0; i < DIM; ++i) dx[i] = __dsub_rn(xyz[j1 * DIM + i], xyz[j0 * DIM + i]);
+  double l2 = __dmul_rn(dx[0], dx[0]);
+#pragma unroll
+  for (int i = 1; i < DIM; ++i) l2 = __dadd_rn(l2, __dmul_rn(dx[i], dx[i]));
+  const double len = __dsqrt_rn(l2);
+  const TbDivisor dv(len);                  // (one reciprocal for the four quotients of the member)
+  k = dv.div(__dmul_rn(e, ar));
+#pragma unroll
+  for (int i = 0; i < DIM; ++i) c[i] = dv.div(dx[i]);
+  w = __dmul_rn(__dmul_rn(ar, len), rho);
+  return len;
+}
 #endif
 
 // ---------------------------------------------------------------------------------------------
@@ -274,6 +298,24 @@ int tb_launch_band_chol(const LargeArgs& a, int num_sm, cudaStream_t st);
 int tb_launch_assemble_only(const LargeArgs& a, int num_sm, cudaStream_t st);   // member products + K_ff values (a.kv) through a.q_*
 int tb_launch_band_subst(const LargeArgs& a, int num_sm, cudaStream_t st);   // load cases against the factor of system 0
 int tb_band_smem_bytes(int NB);
+
+// Reverse mode (tb_adjoint.cu): the adjoint load before the adjoint solve, the sensitivities after it
+struct TbAdjArgs {
+  int batch, dim, nJ, M, N;
+  const double* xyz; int64_t xyz_stride;
+  const double* aed; int64_t aed_stride;
+  const int32_t* conn; const int32_t* dof2free; const int32_t* inc_ptr; const int32_t* inc_mem;
+  const double* g_u; const double* g_ext; const double* g_axial; const double* g_w;   // cotangents, null = 0
+  double* r;             // [B][N] adjoint load (k_adj_rhs)
+  const double* u;       // [B][N] forward displacements (k_sens)
+  const double* lam;     // [B][N] adjoint solution (k_sens)
+  const int32_t* info;   // [B]    status of the solve (k_sens)
+  double* vec;           // [B][M][dim] per-member vectors in HBM, or null: shared memory (tb_adjoint_vec_in_smem)
+  double* g_xyz; double* g_aed; double* g_force;                                      // outputs (g_aed required)
+};
+bool tb_adjoint_vec_in_smem(int dim, int M);
+int tb_launch_adj_rhs(const TbAdjArgs& a, int num_sm, cudaStream_t st);
+int tb_launch_sens(const TbAdjArgs& a, int num_sm, cudaStream_t st);
 
 // fragment-major offset of element (r, c) inside one 64x64 tile:
 //   [k-half 2][row-block 8][k-slab 8][lane 32], lane = (r%8)*4 + c%4

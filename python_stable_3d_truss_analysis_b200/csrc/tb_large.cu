@@ -938,20 +938,9 @@ __global__ void __launch_bounds__(256) k_recover(const LargeArgs a) {
           ar = tt[0]; e = tt[1]; rho = tt[2];
         }
         double dx[DIM];
+        tb_member_geom<DIM>(xyz, j0, j1, ar, e, rho, dx, cm, km, wm);
 #pragma unroll
-        for (int i = 0; i < DIM; ++i) dx[i] = __dsub_rn(xyz[j1 * DIM + i], xyz[j0 * DIM + i]);
-        double l2 = __dmul_rn(dx[0], dx[0]);
-#pragma unroll
-        for (int i = 1; i < DIM; ++i) l2 = __dadd_rn(l2, __dmul_rn(dx[i], dx[i]));
-        const double len = __dsqrt_rn(l2);
-        const TbDivisor dv(len);                  // (one reciprocal for the four quotients of the member)
-        km = dv.div(__dmul_rn(e, ar));
-#pragma unroll
-        for (int i = 0; i < DIM; ++i) {
-          cm[i] = dv.div(dx[i]);
-          sRec[a.M + m * DIM + i] = cm[i];
-        }
-        wm = __dmul_rn(__dmul_rn(ar, len), rho);
+        for (int i = 0; i < DIM; ++i) sRec[a.M + m * DIM + i] = cm[i];
       } else {
         km = mk[m];
         wm = mw[m];

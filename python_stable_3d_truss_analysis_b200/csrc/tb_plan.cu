@@ -539,7 +539,11 @@ extern "C" void tb_plan_destroy(tb_plan* p) {
   cudaFree(p->d_prod_k);
   cudaFree(p->d_inc_ptr);
   cudaFree(p->d_inc_mem);
-  if (p->ws_event) cudaEventDestroy(p->ws_event);
+  if (p->ws_event) {
+    cudaEventSynchronize(p->ws_event);          // (the last call's kernels may still read the adjoint scratch)
+    cudaEventDestroy(p->ws_event);
+  }
+  cudaFree(p->adj_buf);
   cudaFree(p->ws);
   cudaFree(p->stage_dev);
   for (int i = 0; i < TB_ASYNC_SLOTS; ++i) {
