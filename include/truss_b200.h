@@ -20,7 +20,10 @@
  *        0  solved
  *        k>0  leading minor k of the reduced stiffness matrix is not positive definite
  *             (LAPACK potrf convention; the reference would raise numpy LinAlgError or
- *             return garbage for a singular K, truss.py:343)
+ *             return garbage for a singular K, truss.py:343).  The two-sided band kernel
+ *             (k_band_ts) eliminates its top part top-down and its bottom part bottom-up
+ *             at once: k - 1 is the plan-order row of the first non-positive pivot of the
+ *             part that failed, and of the bottom part when both fail (DESIGN.md section 3)
  *        -1  fails the counting rule of truss.py:158-164 (reference: TrussNotStableError)
  *        -2  a member has zero length (reference: ZeroDivisionError, truss.py:58)
  *        -3  invalid support code for this dim (device-side check; type.py:48-74)

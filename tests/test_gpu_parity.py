@@ -14,7 +14,9 @@ from python_stable_3d_truss_analysis_b200.batch import (FitnessBatch, SolveBatch
 from python_stable_3d_truss_analysis_b200.truss import Truss
 from python_stable_3d_truss_analysis_b200.type import MemberType, SupportType
 from python_stable_3d_truss_analysis_b200.utils import TrussNotStableError
+from tests import band_catalogue as BC
 from tests import helpers as H
+from tests.helpers import tower as _tower
 
 pytestmark = pytest.mark.gpu
 
@@ -334,47 +336,71 @@ def test_config5_cube12_tiled_vs_oracle():
         assert np.abs(tot).max() <= 1e-7 * np.abs(force).sum()
 
 
-def test_band_kernels_agree_bitwise_across_batch_sizes():
-    """The band path picks a three-warp-per-system kernel while the batch fits in one wave and a two-warp-per-system
-    kernel beyond (tb_band.cu: launch_band); both sum in the same order, so a system's result does not depend on the
-    batch it is in (SURVEY.md section 4 (iv): bit-identical per truss across GPU counts / shard sizes)."""
-    t = Truss(3).LoadFromJSON(f"{H.GOLDEN}/ref_data/bar-942_input_0.json")
-    rng = np.random.default_rng(3)
-    N = t.nJoint * 3
-    F = rng.uniform(-10, 10, size=(4096, N))
-    big = SolveLoadCases(t, F, independent=True)                 # 4096 systems: two-warp kernel, chunked host pipeline
-    small = SolveLoadCases(t, F[1000:1032], independent=True)    # 32 systems: three-warp kernel
-    for k in H.FIELDS:
+def test_band_kernels_agree_bitwise_across_batch_sizes(tmp_path):
+    """A system's band-path result does not depend on the batch it is in (SURVEY.md section 4 (iv): bit-identical per
+    truss across GPU counts / shard sizes).  k_band_ts: 4096 systems (seven CTAs per SM, several systems per CTA in the
+    grid-stride loop) against 32 of them (one system per CTA).  The 16x16 kernels (TB_BAND_LEGACY=1, a fresh process):
+    the two-warp k_band2 at 4096 systems against the three-warp k_band3 at 32, same arithmetic in the same order."""
+    e = BC.get("bar-942")
+    plan = BC.plan_for(e)
+    NB16, nb = plan.info.band_blocks, BC.ts_nb(plan.ts_program())
+    xyz, aed, F = BC.inputs(plan, e, 4096, seed=3)
+    big, seen_big = H.cuda_kernels(lambda: H.solve_device_np(plan, 4096, xyz, aed, F))
+    small, seen_small = H.cuda_kernels(lambda: H.solve_device_np(plan, 32, xyz, aed[1000:1032], F[1000:1032]))
+    print(f"k_band_ts: {seen_big} | {seen_small}")
+    assert H.band_kernels(seen_big) == H.band_kernels(seen_small) == [f"k_band_ts<{nb}>"], (seen_big, seen_small)
+    for k in ("u", "ext", "axial", "weight", "info"):
         assert np.array_equal(big[k][1000:1032], small[k]), k
-
-
-_BAND_VARIANT_SCRIPT = """
-import sys, numpy as np
-sys.path.insert(0, {root!r})
-from python_stable_3d_truss_analysis_b200.truss import Truss
-from python_stable_3d_truss_analysis_b200.batch import SolveLoadCases
-t = Truss(3).LoadFromJSON({inp!r})
-F = np.random.default_rng(5).uniform(-10, 10, size=(40, t.nJoint * 3))
-out = SolveLoadCases(t, F, independent=True)
-np.savez({dst!r}, u=out["u"], ext=out["ext"], axial=out["axial"])
-"""
+    (lbig, lseen_big), (lsmall, lseen_small) = H.run_band_child(tmp_path, {"TB_BAND_LEGACY": "1"}, [
+        {"label": "bar-942", "B": 4096, "seed": 3}, {"label": "bar-942", "B": 4096, "seed": 3, "slice": [1000, 1032]}])
+    print(f"legacy: {lseen_big} | {lseen_small}")
+    assert H.band_kernels(lseen_big) == [f"k_band2<{NB16}>"] and H.band_kernels(lseen_small) == [f"k_band3<{NB16}>"]
+    for k in ("u", "ext", "axial", "weight", "info"):
+        assert np.array_equal(lbig[k][1000:1032], lsmall[k]), k
+    assert not big["info"].any() and not lbig["info"].any()
+    joints, support, conn, _, _ = BC.arrays(e)
+    for b in (0, 1000, 4095):
+        want = orc.solve(3, joints, support, conn, aed[b], F[b])
+        for name, got in (("k_band_ts", big), ("k_band2", lbig)):
+            H.assert_close({k: got[k][b] for k in H.FIELDS} | {"weight": got["weight"][b]}, want, what=f"{name}[{b}]")
 
 
 def test_band_kernel_variants_agree_bitwise(tmp_path):
-    """k_band1 (one warp per system), k_band2 (two) and k_band3 (three) are the same arithmetic in the same order:
-    forced one after the other through TB_BAND_WARPS (read once per process, hence the subprocesses) they return the
-    same bits."""
-    import os, subprocess, sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    """k_band1 (one warp per system), k_band2 (two) and k_band3 (three) are the same arithmetic in the same order.
+    Under TB_BAND_LEGACY=1 (systems with a two-sided program take the 16x16 kernels too) each is forced in turn through
+    TB_BAND_WARPS (both are read once per process, hence the subprocesses) on the band catalogue's systems of
+    NB16 = 1 .. 5: they return the same bits, and each matches the oracle.  NB16 = 6 .. 8 run on k_band1 alone, at 5
+    systems: not a multiple of its systems per CTA (4 for NB16 <= 6, 2 for 7 and 8)."""
+    systems = [e for e in BC.catalogue() if "/" not in e.label]
+    NB16 = {e.label: BC.plan_for(e).info.band_blocks for e in systems}
+    narrow = [e.label for e in systems if NB16[e.label] <= 5]
+    assert sorted({NB16[x] for x in narrow}) == [1, 2, 3, 4, 5]
+    assert sorted({v for v in NB16.values() if v > 5}) == [6, 7, 8]
+    B = 5
     res = {}
     for w in (1, 2, 3):
-        dst = str(tmp_path / f"w{w}.npz")
-        code = _BAND_VARIANT_SCRIPT.format(root=root, inp=f"{H.GOLDEN}/ref_data/bar-942_input_0.json", dst=dst)
-        subprocess.run([sys.executable, "-c", code], check=True, env=dict(os.environ, TB_BAND_WARPS=str(w)), timeout=600)
-        res[w] = np.load(dst)
-    for w in (2, 3):
-        for k in ("u", "ext", "axial"):
-            assert np.array_equal(res[1][k], res[w][k]), (w, k)
+        labels = [e.label for e in systems] if w == 1 else narrow
+        runs = H.run_band_child(tmp_path, {"TB_BAND_LEGACY": "1", "TB_BAND_WARPS": str(w)},
+                                [{"label": x, "B": B, "seed": 11} for x in labels])
+        for x, (out, seen) in zip(labels, runs):
+            print(f"TB_BAND_WARPS={w} {x}: {seen}")
+            assert H.band_kernels(seen) == [f"k_band{w}<{NB16[x]}>"], (w, x, seen)
+            assert not out["info"].any(), (w, x)
+            res[w, x] = out
+    for x in narrow:
+        for w in (2, 3):
+            for k in ("u", "ext", "axial", "weight"):
+                assert np.array_equal(res[1, x][k], res[w, x][k]), (x, w, k)
+    for e in systems:
+        plan = BC.plan_for(e)
+        joints, support, conn, _, _ = BC.arrays(e)
+        xyz, aed, F = BC.inputs(plan, e, B, seed=11)
+        for b in range(B):
+            want = orc.solve(e.dim, joints, support, conn, aed[b], F[b])
+            got = res[1, e.label]
+            H.assert_close({k: got[k][b] for k in H.FIELDS} | {"weight": got["weight"][b]}, want, what=f"k_band1 {e.label}[{b}]")
+            be = H.backward_error(e.dim, joints, support, conn, aed[b], F[b], got["u"][b])
+            assert be <= 1e-14, (e.label, b, be)
 
 
 def test_pivot_rsqrt_accuracy():
@@ -382,46 +408,6 @@ def test_pivot_rsqrt_accuracy():
     (tb_blocks.cuh: rsqrt_pos); it must stay within 2 ulp of 1/sqrt(d) over the whole accepted pivot range."""
     from python_stable_3d_truss_analysis_b200 import _lib
     assert _lib.rsqrt_probe(1 << 22) <= 4.5e-16
-
-
-def _tower(dim, per_level, levels, seed):
-    """A lattice tower: `per_level` joints per level on a ring (2D: a ladder), every level braced to the next; the bottom
-    level is pinned.  Half-bandwidth of K_ff ~ 2 * dim * per_level, so per_level sweeps the band width."""
-    rng = np.random.default_rng(seed)
-    joints, members = [], []
-    for lv in range(levels):
-        for k in range(per_level):
-            if dim == 2:
-                p = [float(k) * 2.0 + 0.1 * rng.standard_normal(), float(lv) * 1.5]
-            else:
-                ang = 2 * np.pi * k / per_level
-                p = [3.0 * np.cos(ang) + 0.1 * rng.standard_normal(), 3.0 * np.sin(ang) + 0.1 * rng.standard_normal(), 2.0 * lv]
-            joints.append([p, "PIN" if lv == 0 else "NO"])
-    jid = lambda lv, k: lv * per_level + (k % per_level)
-    mt = lambda: [float(rng.uniform(0.5, 2.0)), 1e4, 0.1]
-    for lv in range(levels):
-        ring = per_level if (dim == 3 and per_level > 2) else per_level - 1
-        for k in range(ring):
-            if lv > 0:
-                members.append([[jid(lv, k), jid(lv, k + 1)], mt()])
-        if dim == 3 and per_level > 3 and lv > 0:                  # cross bracing inside the level
-            for k in range(per_level - 2):
-                members.append([[jid(lv, 0), jid(lv, k + 2)], mt()]) if k + 2 != per_level - 1 or per_level == 4 else None
-        if lv + 1 < levels:
-            for k in range(per_level):
-                members.append([[jid(lv, k), jid(lv + 1, k)], mt()])
-                members.append([[jid(lv, k), jid(lv + 1, k + 1)], mt()])
-                if dim == 3:
-                    members.append([[jid(lv, k + 1), jid(lv + 1, k)], mt()])
-    members = [m for m in members if m is not None and m[0][0] != m[0][1]]
-    seen, uniq = set(), []
-    for m in members:
-        key = tuple(sorted(m[0]))
-        if key not in seen:
-            seen.add(key)
-            uniq.append(m)
-    forces = [[jid(levels - 1, k), [float(x) for x in rng.uniform(-5, 5, size=dim)]] for k in range(per_level)]
-    return {"joint": joints, "force": forces, "member": uniq}
 
 
 @pytest.mark.parametrize("dim,per_level,levels", [(2, 2, 40), (3, 3, 30), (3, 5, 24), (3, 8, 16), (3, 11, 12), (3, 13, 10),
