@@ -290,6 +290,23 @@ typedef struct {
 int tb_solve_ragged(const tb_ragged_in* in, const tb_batch_out* out, void* cuda_stream);
 int tb_solve_ragged_host(const tb_ragged_in* in, const tb_batch_out* out);
 
+/* Reverse mode of tb_solve_ragged: the gradients of L (as tb_adjoint) for every truss of a ragged batch, by one adjoint
+ * ragged solve (the same kernel as the forward of the batch) between two warp-per-truss kernels.  Device pointers in the
+ * packed layout: `u` (the forward's displacements of the same inputs), grad->u / grad->ext, out->joint_xyz / out->force
+ * [d * sum nJ]; grad->axial [sum M]; out->member_aed [sum M][3]; grad->weight, out->info [B].  Required (TB_ERR_NULL
+ * otherwise, when B > 0): in and its packed arrays as for tb_solve_ragged, u, grad, out, out->member_aed, out->info (the
+ * solve's per-truss status, the forward's; a failed truss gets zero gradients) and work.  Optional (NULL = a zero
+ * cotangent, or the gradient is skipped): grad->u / ext / axial / weight, out->joint_xyz, out->force.
+ * `work` is caller-provided device scratch of at least d * joint_off[B] doubles (the adjoint
+ * load, overwritten in place by the adjoint solution): the offsets live on the device, so only the caller knows sum nJ.
+ * Argument errors as tb_solve_ragged (TB_ERR_NULL / TB_ERR_DIM / TB_ERR_SIZE / TB_ERR_TOO_LARGE; B = 0 is a no-op),
+ * TB_ERR_NO_DEVICE without a GPU.  The offsets and arrays are not validated on the host: a truss larger than max_joint /
+ * max_member, with a joint id outside [0, nJ) or an unknown support code gets zero gradients (and its status), and
+ * nothing is read out of range; the rows of a truss whose offsets do not lie inside [0, joint_off[B]] / [0,
+ * member_off[B]] are not written.  Enqueues on the stream without synchronising (capturable into a CUDA graph). */
+int tb_adjoint_ragged(const tb_ragged_in* in, const double* u, const tb_adj_in* grad, const tb_adj_out* out, double* work,
+                      void* cuda_stream);
+
 /* ---- Dataset generation on the device (slientruss3d/generate.py:12-148; SURVEY.md section 8 f-2) ------------------
  * Expands a pool of trusses (a tb_ragged_in with DEVICE pointers) into n_out augmented trusses in the same packed layout,
  * ready for tb_solve_ragged: output truss o is pool truss src[o] after MoveToCentroid, RandomTranslation, AddJointNoise,

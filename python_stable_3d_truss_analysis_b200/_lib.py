@@ -164,7 +164,7 @@ class TbRaggedIn(C.Structure):
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
            "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
-           "tb_solve_ragged_host", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
+           "tb_solve_ragged_host", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
 _lib = None
@@ -199,6 +199,7 @@ def lib():
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
     L.tb_solve_ragged_host.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut)]
+    L.tb_adjoint_ragged.argtypes = [C.POINTER(TbRaggedIn), vp, C.POINTER(TbAdjIn), C.POINTER(TbAdjOut), vp, vp]
     L.tb_pinned_alloc.argtypes = [C.POINTER(vp), C.c_size_t]
     L.tb_pinned_free.argtypes = [vp]
     L.tb_small_path_limits.argtypes = [C.POINTER(i32), C.POINTER(i32)]
@@ -648,6 +649,63 @@ def solve_ragged_host(dim, joint_off, member_off, xyz, support, conn, aed, force
     return out
 
 
+def _ragged_in(dim, packed, max_joint=None, max_member=None):
+    """tb_ragged_in over the CUDA tensors of a packed dict (joint_off, member_off, xyz, support, conn, aed, force).  The
+    maxima come from the offsets (one device-to-host read) unless given."""
+    import torch
+
+    jo, mo = packed["joint_off"], packed["member_off"]
+    B = int(jo.shape[0]) - 1
+    if max_joint is None or max_member is None:
+        mx = [0, 0]
+        if B > 0:
+            mx = torch.stack([(jo[1:] - jo[:-1]).max(), (mo[1:] - mo[:-1]).max()]).tolist()
+        max_joint = mx[0] if max_joint is None else max_joint
+        max_member = mx[1] if max_member is None else max_member
+    return TbRaggedIn(int(dim), B, _ptr(jo), _ptr(mo), _ptr(packed["xyz"]), _ptr(packed["support"]), _ptr(packed["conn"]),
+                      _ptr(packed["aed"]), _ptr(packed["force"]), int(max_joint), int(max_member))
+
+
+def solve_ragged_device(dim, packed, out=None, stream=None, max_joint=None, max_member=None):
+    """tb_solve_ragged on torch CUDA tensors: ``packed`` holds joint_off, member_off [B+1] (int64), xyz [d sum nJ],
+    support [sum nJ] (uint8), conn [2 sum M] (int32, local joint ids), aed [3 sum M] and force [d sum nJ] (float64), as
+    ``gencube_device`` / ``augment_and_solve_device`` return them.  ``out`` may hold preallocated u, ext [d sum nJ],
+    axial [sum M], weight [B] and info [B] tensors; missing ones are allocated.  Enqueues on ``stream`` (None = current)
+    and returns ``out``."""
+    import torch
+
+    ri = _ragged_in(dim, packed, max_joint, max_member)
+    dev = packed["xyz"].device
+    SJ, SM, B = int(packed["support"].numel()), int(packed["conn"].numel()) // 2, ri.batch
+    out = {} if out is None else out
+    for k, n, dt in (("u", SJ * dim, torch.float64), ("ext", SJ * dim, torch.float64), ("axial", SM, torch.float64),
+                     ("weight", B, torch.float64), ("info", B, torch.int32)):
+        if out.get(k) is None:
+            out[k] = torch.empty(n, dtype=dt, device=dev)
+    st = torch.cuda.current_stream() if stream is None else stream
+    bo = TbBatchOut(_ptr(out["u"]), _ptr(out["ext"]), _ptr(out["axial"]), _ptr(out["weight"]), _ptr(out["info"]))
+    check(lib().tb_solve_ragged(C.byref(ri), C.byref(bo), C.c_void_p(st.cuda_stream)))
+    return out
+
+
+def adjoint_ragged_device(dim, packed, u, grads, out, stream=None, max_joint=None, max_member=None, work=None):
+    """Reverse mode of ``solve_ragged_device`` (tb_adjoint_ragged) on torch CUDA tensors.  ``u`` is the forward's
+    displacements [d sum nJ] of the same inputs; ``grads`` maps "u" / "ext" / "axial" / "weight" to cotangents in the
+    packed layout (missing or None = 0); ``out`` maps "joint_xyz" [d sum nJ], "member_aed" [3 sum M] (required),
+    "force" [d sum nJ] and "info" [B] (required) to preallocated tensors.  ``work``: device scratch of d sum nJ doubles
+    (allocated when None)."""
+    import torch
+
+    ri = _ragged_in(dim, packed, max_joint, max_member)
+    if work is None:
+        work = torch.empty(max(int(packed["support"].numel()) * dim, 1), dtype=torch.float64, device=packed["xyz"].device)
+    st = torch.cuda.current_stream() if stream is None else stream
+    gi = TbAdjIn(_ptr(grads.get("u")), _ptr(grads.get("ext")), _ptr(grads.get("axial")), _ptr(grads.get("weight")))
+    go = TbAdjOut(_ptr(out.get("joint_xyz")), _ptr(out.get("member_aed")), _ptr(out.get("force")), _ptr(out.get("info")))
+    check(lib().tb_adjoint_ragged(C.byref(ri), _ptr(u), C.byref(gi), C.byref(go), _ptr(work), C.c_void_p(st.cuda_stream)))
+    return out
+
+
 def augment_and_solve_device(dim, pool, n_out, params: "TbAugmentParams", src=None, solve=True, device=None):
     """Dataset generation on the device: expand the packed pool (dict of numpy arrays: joint_off, member_off, xyz,
     support, conn, aed, force) into ``n_out`` augmented trusses (tb_augment_ragged) and, if ``solve``, run
@@ -681,13 +739,7 @@ def augment_and_solve_device(dim, pool, n_out, params: "TbAugmentParams", src=No
                                   C.byref(params), _ptr(out["xyz"]), _ptr(out["support"]), _ptr(out["conn"]), _ptr(out["aed"]),
                                   _ptr(out["force"]), st))
     if solve:
-        out.update({"u": torch.empty(SJ * dim, dtype=torch.float64, device=dev), "ext": torch.empty(SJ * dim, dtype=torch.float64, device=dev),
-                    "axial": torch.empty(SM, dtype=torch.float64, device=dev), "weight": torch.empty(n_out, dtype=torch.float64, device=dev),
-                    "info": torch.empty(n_out, dtype=torch.int32, device=dev)})
-        ro = TbRaggedIn(int(dim), int(n_out), _ptr(out["joint_off"]), _ptr(out["member_off"]), _ptr(out["xyz"]), _ptr(out["support"]),
-                        _ptr(out["conn"]), _ptr(out["aed"]), _ptr(out["force"]), maxj, maxm)
-        bo = TbBatchOut(_ptr(out["u"]), _ptr(out["ext"]), _ptr(out["axial"]), _ptr(out["weight"]), _ptr(out["info"]))
-        check(lib().tb_solve_ragged(C.byref(ro), C.byref(bo), st))
+        solve_ragged_device(dim, out, out=out, max_joint=maxj, max_member=maxm)
     out["_keep"] = d
     return out
 
@@ -726,11 +778,7 @@ def gencube_device(params: "TbGencubeParams", n, type_table, solve=True, export=
                                 _ptr(out["conn"]), _ptr(out["aed"]), st))
     out.update(ex)
     if solve and n > 0:
-        out.update({"u": e(SJ * 3), "ext": e(SJ * 3), "axial": e(SM), "weight": e(n), "info": e(n, dt=torch.int32)})
-        ro = TbRaggedIn(3, n, _ptr(jo), _ptr(mo), _ptr(out["xyz"]), _ptr(out["support"]), _ptr(out["conn"]), _ptr(out["aed"]),
-                        _ptr(out["force"]), int(s["nj"].max()), int(s["nm"].max()))
-        bo = TbBatchOut(_ptr(out["u"]), _ptr(out["ext"]), _ptr(out["axial"]), _ptr(out["weight"]), _ptr(out["info"]))
-        check(lib().tb_solve_ragged(C.byref(ro), C.byref(bo), st))
+        solve_ragged_device(3, out, out=out, max_joint=int(s["nj"].max()), max_member=int(s["nm"].max()))
     return out
 
 

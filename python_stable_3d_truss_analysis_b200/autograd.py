@@ -12,13 +12,18 @@ Example -- compliance gradient of bar-72 with respect to the member areas::
     out = autograd.solve(truss, aed=aed, force=f)
     (f * out["u"]).sum().backward()                   # compliance C = f.u
     dC_dA = aed.grad[:, 0]
+
+``solve_ragged(packed, xyz, aed, force)`` does the same for a ragged batch -- every truss with its own topology, packed
+back to back as ``gencube_device`` / ``augment_and_solve_device`` return them (``tb_adjoint_ragged``).
 """
 from __future__ import annotations
 
 import numpy as np
 import torch
 
-__all__ = ["solve"]
+from . import _lib
+
+__all__ = ["solve", "solve_ragged"]
 
 
 class _Solve(torch.autograd.Function):
@@ -99,3 +104,87 @@ def solve(truss, xyz=None, aed=None, force=None, shared_factor=False):
     if bx is None and ba is None and bf is None:
         out = {k: v[0] for k, v in out.items()}
     return out
+
+
+class _SolveRagged(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, xyz, aed, force, joint_off, member_off, support, conn, dim, maxj, maxm):
+        p = dict(joint_off=joint_off, member_off=member_off, support=support, conn=conn, xyz=xyz, aed=aed, force=force)
+        out = _lib.solve_ragged_device(dim, p, max_joint=maxj, max_member=maxm)
+        # (the topology tensors too: the version counter then refuses a backward after an in-place change to them)
+        ctx.save_for_backward(xyz, aed, force, out["u"], joint_off, member_off, support, conn)
+        ctx.dim, ctx.maxj, ctx.maxm = dim, maxj, maxm
+        ctx.mark_non_differentiable(out["info"])
+        ctx.set_materialize_grads(False)          # an output without a cotangent is passed to the library as NULL
+        return out["u"], out["ext"], out["axial"], out["weight"], out["info"]
+
+    @staticmethod
+    def backward(ctx, g_u, g_ext, g_axial, g_w, _g_info):
+        xyz, aed, force, u, joint_off, member_off, support, conn = ctx.saved_tensors
+        grads = {k: None if g is None else g.contiguous()
+                 for k, g in (("u", g_u), ("ext", g_ext), ("axial", g_axial), ("weight", g_w))}
+        need_x, _, need_f = ctx.needs_input_grad[:3]
+        res = {"joint_xyz": torch.empty_like(xyz) if need_x else None, "member_aed": torch.empty_like(aed),
+               "force": torch.empty_like(force) if need_f else None,
+               "info": torch.empty(joint_off.shape[0] - 1, dtype=torch.int32, device=u.device)}
+        p = dict(joint_off=joint_off, member_off=member_off, support=support, conn=conn, xyz=xyz, aed=aed, force=force)
+        _lib.adjoint_ragged_device(ctx.dim, p, u, grads, res, max_joint=ctx.maxj, max_member=ctx.maxm)
+        return (res["joint_xyz"], res["member_aed"] if ctx.needs_input_grad[1] else None, res["force"]) + (None,) * 7
+
+
+def _packed_input(t, default, shapes, name):
+    """``t`` (the packed default when None) after checking that it is a float64 tensor of one of ``shapes``."""
+    if t is None:
+        t = default
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.float64:
+        raise TypeError(f"{name} must be a float64 CUDA tensor")
+    if tuple(t.shape) not in shapes:
+        raise ValueError(f"{name} must have shape {' or '.join(str(list(s)) for s in shapes)}, not {list(t.shape)}")
+    return t
+
+
+def solve_ragged(packed, xyz=None, aed=None, force=None, max_joint=None, max_member=None):
+    """``Truss.Solve()`` for a ragged batch (every truss its own topology), differentiable with respect to ``xyz``,
+    ``aed`` and ``force``.
+
+    ``packed`` is a dict of CUDA tensors in the layout of ``tb_ragged_in``: ``joint_off`` / ``member_off`` [B+1] int64,
+    ``support`` [sum nJ] uint8, ``conn`` [2 sum M] int32 (local joint ids) and optionally ``xyz`` / ``aed`` / ``force``
+    -- what ``_lib.gencube_device`` and ``_lib.augment_and_solve_device`` return (a ``PackedDataset``'s arrays moved to
+    the device work too).  ``xyz`` [sum nJ, d] or [d sum nJ], ``aed`` [sum M, 3] or [3 sum M] and ``force`` [d sum nJ] are
+    float64 CUDA tensors; None means the packed value, held constant.  ``max_joint`` / ``max_member`` size the kernels;
+    None reads them from the offsets (one device-to-host copy).
+
+    Returns ``{"u": [d sum nJ], "ext": [d sum nJ], "axial": [sum M], "weight": [B], "info": [B] int32}`` in the packed
+    layout.  ``info`` is the per-truss status of ``include/truss_b200.h`` and is not differentiable; a failed truss has
+    zero outputs and zero gradients.  Every input row belongs to one truss, so the gradients need no batch reduction."""
+    for k, dt in (("joint_off", torch.int64), ("member_off", torch.int64), ("support", torch.uint8), ("conn", torch.int32)):
+        t = packed.get(k)
+        if not isinstance(t, torch.Tensor) or t.dtype != dt or t.dim() != 1:
+            raise TypeError(f"packed[{k!r}] must be a 1-D {dt} CUDA tensor")
+    SJ, SM = int(packed["support"].numel()), int(packed["conn"].numel()) // 2
+    src = xyz if xyz is not None else packed.get("xyz")
+    if isinstance(src, torch.Tensor) and src.dim() == 2:
+        dim = int(src.shape[1])
+    elif isinstance(src, torch.Tensor) and SJ > 0 and src.numel() % SJ == 0:
+        dim = src.numel() // SJ
+    else:
+        raise ValueError("xyz must have shape [sum nJ, d] or [d * sum nJ] with d = 2 or 3")
+    if dim not in (2, 3):
+        raise ValueError(f"xyz must have d = 2 or 3 columns, not {dim}")
+    xyz = _packed_input(xyz, packed.get("xyz"), [(SJ, dim), (SJ * dim,)], "xyz")
+    aed = _packed_input(aed, packed.get("aed"), [(SM, 3), (SM * 3,)], "aed")
+    force = _packed_input(force, packed.get("force"), [(SJ * dim,)], "force")
+    base = {k: packed[k] for k in ("joint_off", "member_off", "support", "conn")}
+    for k, t in list(base.items()) + [("xyz", xyz), ("aed", aed), ("force", force)]:   # (dtypes and shapes first)
+        if not t.is_cuda or t.device != xyz.device:
+            raise TypeError(f"{k} must be a CUDA tensor on the device of xyz")
+    xyz, aed, force = xyz.contiguous(), aed.contiguous(), force.contiguous()
+    jo, mo = base["joint_off"], base["member_off"]
+    if (max_joint is None or max_member is None) and jo.shape[0] > 1:      # one device-to-host read for both passes
+        mj, mm = torch.stack([(jo[1:] - jo[:-1]).max(), (mo[1:] - mo[:-1]).max()]).tolist()
+        max_joint = mj if max_joint is None else max_joint
+        max_member = mm if max_member is None else max_member
+    with torch.cuda.device(xyz.device):
+        u, ext, axial, weight, info = _SolveRagged.apply(xyz, aed, force, base["joint_off"], base["member_off"], base["support"],
+                                                         base["conn"], dim, max_joint, max_member)
+    return {"u": u, "ext": ext, "axial": axial, "weight": weight, "info": info}

@@ -945,6 +945,39 @@ extern "C" int tb_adjoint(tb_plan* p, const tb_batch_in* in, const double* u, co
   return ws_release(p, st);
 }
 
+// Reverse mode of tb_solve_ragged: adjoint load, the adjoint solve through run_ragged (the same kernel as the forward of
+// the batch; K is symmetric: force := r), sensitivities.  The adjoint solution overwrites the load in `work`: every solve
+// kernel stages a truss's load rows before it writes that truss's displacement rows, and a truss's rows belong to one
+// warp (or CTA), so the host never needs the device-resident total joint count to place a second array.
+extern "C" int tb_adjoint_ragged(const tb_ragged_in* in, const double* u, const tb_adj_in* grad, const tb_adj_out* out,
+                                 double* work, void* cuda_stream) {
+  int rc = check_ragged(in);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  if (!u || !grad || !out || !out->member_aed || !out->info || !work) return TB_ERR_NULL;
+  if (!have_device()) return TB_ERR_NO_DEVICE;
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  TbAdjRaggedArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.dim = in->dim; a.max_joint = in->max_joint; a.max_member = in->max_member;
+  a.joint_off = in->joint_off; a.member_off = in->member_off;
+  a.xyz = in->joint_xyz; a.support = in->support; a.conn = in->conn; a.aed = in->member_aed;
+  a.g_u = grad->u; a.g_ext = grad->ext; a.g_axial = grad->axial; a.g_w = grad->weight;
+  a.r = work;
+  a.u = u;
+  a.lam = work;
+  a.info = out->info;
+  a.g_xyz = out->joint_xyz; a.g_aed = out->member_aed; a.g_force = out->force;
+  rc = tb_launch_adj_rhs_ragged(a, st);
+  if (rc) return rc;
+  tb_ragged_in ain = *in;                       // same trusses, load := r (its supported rows are ignored)
+  ain.force = work;
+  const tb_batch_out aout = {work, nullptr, nullptr, nullptr, out->info, nullptr, nullptr};
+  rc = run_ragged(&ain, &aout, st);
+  if (rc) return rc;
+  return tb_launch_sens_ragged(a, st);
+}
+
 // pinned host buffers for callers that want full-speed H2D/D2H through the *_host entry points
 extern "C" int tb_pinned_alloc(void** ptr, size_t bytes) {
   if (!ptr) return TB_ERR_NULL;

@@ -15,6 +15,11 @@ struct TsPlan;   // two-sided band program (tb_ts.cuh)
 // SupportType codes, slientruss3d/type.py:30-35
 enum : int { SUP_NO = 0, SUP_PIN = 1, SUP_ROLLER_X = 2, SUP_ROLLER_Y = 3, SUP_ROLLER_Z = 4 };
 
+// Support code -> DOF rule (type.py:48-74): axis `ax` of a joint is restrained by a pin or by the roller of that axis
+__host__ __device__ __forceinline__ bool tb_dof_free(int s, int ax) { return !((s == SUP_PIN) || (s == SUP_ROLLER_X + ax)); }
+// a code the dim does not know (TB_INFO_BAD_SUPPORT)
+__host__ __device__ __forceinline__ bool tb_support_bad(int dim, int s) { return s > SUP_ROLLER_Z || (dim == 2 && s == SUP_ROLLER_Z); }
+
 // utils.py:79-84 IsZero / IsZeroVector default eps
 #define TB_ZERO_EPS 1e-10
 
@@ -316,6 +321,21 @@ struct TbAdjArgs {
 bool tb_adjoint_vec_in_smem(int dim, int M);
 int tb_launch_adj_rhs(const TbAdjArgs& a, int num_sm, cudaStream_t st);
 int tb_launch_sens(const TbAdjArgs& a, int num_sm, cudaStream_t st);
+
+// Reverse mode of a ragged batch (tb_adjoint_ragged): packed layout of tb_ragged_in, local joint ids, one warp per truss
+struct TbAdjRaggedArgs {
+  int batch, dim, max_joint, max_member;
+  const int64_t* joint_off; const int64_t* member_off;
+  const double* xyz; const uint8_t* support; const int32_t* conn; const double* aed;
+  const double* g_u; const double* g_ext; const double* g_axial; const double* g_w;   // cotangents, null = 0
+  double* r;             // [d sum nJ] adjoint load (k_adj_rhs_ragged)
+  const double* u;       // [d sum nJ] forward displacements (k_sens_ragged)
+  const double* lam;     // [d sum nJ] adjoint solution (k_sens_ragged)
+  const int32_t* info;   // [B]        status of the solve (k_sens_ragged)
+  double* g_xyz; double* g_aed; double* g_force;                                      // outputs (g_aed required)
+};
+int tb_launch_adj_rhs_ragged(const TbAdjRaggedArgs& a, cudaStream_t st);
+int tb_launch_sens_ragged(const TbAdjRaggedArgs& a, cudaStream_t st);
 
 // fragment-major offset of element (r, c) inside one 64x64 tile:
 //   [k-half 2][row-block 8][k-slab 8][lane 32], lane = (r%8)*4 + c%4

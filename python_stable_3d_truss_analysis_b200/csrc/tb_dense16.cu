@@ -144,8 +144,8 @@ __global__ void __launch_bounds__(128) k_dense16(const SmallArgs a, const int nb
         if (dof < N) {
           const int j = dof / DIM, ax = dof - j * DIM;
           const int s = sSup[j];
-          badsup |= (s > SUP_ROLLER_Z || (DIM == 2 && s == SUP_ROLLER_Z));
-          fr = !((s == SUP_PIN) || (s == SUP_ROLLER_X + ax));
+          badsup |= tb_support_bad(DIM, s);
+          fr = tb_dof_free(s, ax);
         }
         const unsigned bal = __ballot_sync(FULL, fr);
         const int pos = n + __popc(bal & ((1u << lane) - 1u));

@@ -125,12 +125,12 @@ extern "C" int tb_plan_create(const tb_topology* topo, tb_plan** plan_out) {
   p->n_resist = 0;
   for (int j = 0; j < p->nJ; ++j) {
     int s = p->support[j];
-    if (s > SUP_ROLLER_Z || (d == 2 && s == SUP_ROLLER_Z)) {  // type.py:62,74
+    if (tb_support_bad(d, s)) {  // type.py:62,74
       delete p;
       return TB_ERR_SUPPORT;
     }
     for (int ax = 0; ax < d; ++ax) {
-      bool resist = (s == SUP_PIN) || (s == SUP_ROLLER_X + ax);
+      bool resist = !tb_dof_free(s, ax);
       int dof = j * d + ax;
       if (resist) {
         p->sup_idx.push_back(dof);

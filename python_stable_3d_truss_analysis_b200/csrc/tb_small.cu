@@ -116,8 +116,8 @@ __global__ void __launch_bounds__(SMALL_MAX_THREADS) k_small(const SmallArgs a) 
         if (dof < N) {
           const int j = dof / DIM, ax = dof - j * DIM;
           const int s = sSup[j];
-          if (s > SUP_ROLLER_Z || (DIM == 2 && s == SUP_ROLLER_Z)) atomicMin(&sMeta[1], TB_INFO_BAD_SUPPORT);
-          fr = !((s == SUP_PIN) || (s == SUP_ROLLER_X + ax));
+          if (tb_support_bad(DIM, s)) atomicMin(&sMeta[1], TB_INFO_BAD_SUPPORT);
+          fr = tb_dof_free(s, ax);
         }
         const unsigned bal = __ballot_sync(0xffffffffu, fr);
         const int pos = run + __popc(bal & ((1u << lane) - 1u));
