@@ -23,11 +23,15 @@
  *             return garbage for a singular K, truss.py:343).  The two-sided band kernel
  *             (k_band_ts) eliminates its top part top-down and its bottom part bottom-up
  *             at once: k - 1 is the plan-order row of the first non-positive pivot of the
- *             part that failed, and of the bottom part when both fail (DESIGN.md section 3)
+ *             part that failed, and of the bottom part when both fail (DESIGN.md section 3).
+ *             The envelope kernel of ragged batches: k - 1 is the position of the first
+ *             non-positive (or subnormal) pivot in the truss's elimination order
+ *             (tb_ragged_env_order)
  *        -1  fails the counting rule of truss.py:158-164 (reference: TrussNotStableError)
  *        -2  a member has zero length (reference: ZeroDivisionError, truss.py:58)
  *        -3  invalid support code for this dim (device-side check; type.py:48-74)
- *        -4  a member or gene index is out of range (device-side check)
+ *        -4  a member or gene index is out of range (device-side check), or a ragged truss is larger
+ *            than the batch's max_joint / max_member
  *     outputs of a system with info != 0 are zero-filled (fitness: +inf), never NaN
  *   - "device" entry points take device pointers, enqueue on the given stream and do not
  *     synchronise; "_host" entry points take host pointers and perform the H2D copies,
@@ -287,8 +291,35 @@ typedef struct {
   int32_t max_member;         /* max M over the batch */
 } tb_ragged_in;
 
+/* Routing: a batch whose (max_joint, max_member) fits the fused shared-memory kernels (tb_small_path_fits) runs on them
+ * in one launch.  Any other batch is split by truss: the trusses up to 48 joints and 192 members (3D; 2D: 72 joints, 224
+ * members) run in one launch of the fused warp-per-truss kernel sized at those limits, and every larger truss runs on the
+ * envelope kernel (one CTA per truss: its own reverse Cuthill-McKee order, row-envelope Cholesky; DESIGN.md section 10),
+ * which overwrites that truss's rows and status.  Either kernel gives a truss the same bits wherever it sits in the
+ * batch.  Accepted sizes: d * max_joint <= 1536 and max_member <= 8192 (tb_ragged_limits); larger: TB_ERR_TOO_LARGE.
+ * The compact outputs (u_free / react) are refused (TB_ERR_SIZE): a ragged batch has no common n and s.
+ * Scratch of the envelope kernel: one grow-only device arena per device, one slot per CTA of its persistent grid (a
+ * slot holds a dense lower-triangle bound of d * max_joint DOFs, the truss's incidence and adjacency lists and member
+ * geometry: about 9.4 MB at 1536 DOFs, under 1 MB for a batch of 40-cube trusses).  It is grown stream-ordered on the
+ * caller's stream (cudaFreeAsync / cudaMallocAsync).  Threads and streams: calls on one device that need it do not
+ * overlap (a mutex), and a call on another stream than the previous one waits for it (an event).  A captured call must
+ * stay on one stream, and a call inside a stream capture never grows the arena: it returns TB_ERR_ALLOC with nothing
+ * enqueued; a warm-up call of the same sizes outside the capture grows it (and a later growth invalidates graphs
+ * captured before it).  Batches that fit the fused kernels use no scratch. */
 int tb_solve_ragged(const tb_ragged_in* in, const tb_batch_out* out, void* cuda_stream);
 int tb_solve_ragged_host(const tb_ragged_in* in, const tb_batch_out* out);
+/* Largest sizes tb_solve_ragged accepts: max_joint = 1536 / dim, max_member = 8192.  TB_ERR_DIM / TB_ERR_NULL. */
+int tb_ragged_limits(int32_t dim, int32_t* max_joint, int32_t* max_member);
+/* Every truss of the batch through the envelope kernel, whatever its size (tests and tools: the ragged counterpart of
+ * tb_plan_set_path).  Device pointers; arguments, outputs, scratch and errors as tb_solve_ragged. */
+int tb_solve_ragged_env(const tb_ragged_in* in, const tb_batch_out* out, void* cuda_stream);
+/* Ordering mode of the envelope kernel: nothing is solved.  order [sum nJ] receives each truss's joints in elimination
+ * order (local ids; 0..nJ-1 when the reverse Cuthill-McKee order does not shrink sum (i - first_i + 1)^2 below 0.85x
+ * that of the natural order -- the rule of tb_plan_create), envelope [B] the row-envelope entries of its K_ff in that
+ * order (tb_plan_info.envelope_size of a plan of the same topology).  A truss over max_joint / max_member gets envelope
+ * -1 and its order rows are not written; one with a joint id outside [0, nJ) gets -1 in both.  order and envelope are
+ * required device pointers (TB_ERR_NULL); other argument errors as tb_solve_ragged. */
+int tb_ragged_env_order(const tb_ragged_in* in, int32_t* order, int64_t* envelope, void* cuda_stream);
 
 /* Reverse mode of tb_solve_ragged: the gradients of L (as tb_adjoint) for every truss of a ragged batch, by one adjoint
  * ragged solve (the same kernel as the forward of the batch) between two warp-per-truss kernels.  Device pointers in the
@@ -396,8 +427,9 @@ int tb_pinned_free(void* ptr);
 /* Largest system (free DOFs are bounded by d*nJ) the fused shared-memory kernel accepts. */
 int tb_small_path_limits(int32_t* max_dof, int32_t* max_member);
 /* 1 when a truss of n_joint joints and n_member members (every DOF possibly free, as in a ragged batch) fits the shared
- * memory of the fused kernels -- the test tb_solve_ragged applies to (max_joint, max_member); the size limits above are
- * necessary, not sufficient (many members on few joints run out of shared memory first). */
+ * memory of the fused kernels -- the test tb_solve_ragged applies to (max_joint, max_member) to keep a batch on them
+ * alone (otherwise it routes by truss, see tb_solve_ragged), and the limit of tb_adjoint_ragged; the size limits above
+ * are necessary, not sufficient (many members on few joints run out of shared memory first). */
 int tb_small_path_fits(int32_t dim, int32_t n_joint, int32_t n_member);
 
 /* FP64 pipe microbenchmarks used as roofline denominators (MEASURED_PEAKS.json has no FP64

@@ -18,7 +18,7 @@ CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_PATH = os.environ.get("TB_LIB_PATH") or os.path.join(CSRC, "libtruss_b200.so")   # TB_LIB_PATH: instrumented builds (tools/)
 SOURCES = ["tb_plan.cu", "tb_tsplan.cu", "tb_small.cu", "tb_dense16.cu", "tb_large.cu", "tb_band.cu", "tb_bandts.cu", "tb_api.cu", "tb_adjoint.cu", "tb_peak.cu",
-           "tb_ga.cu", "tb_augment.cu", "tb_json.cu", "tb_gencube.cu"]
+           "tb_ga.cu", "tb_augment.cu", "tb_json.cu", "tb_gencube.cu", "tb_ragenv.cu"]
 
 TB_ERR_NO_DEVICE = -7
 TB_ERR_TOO_LARGE = -6
@@ -164,7 +164,7 @@ class TbRaggedIn(C.Structure):
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
            "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
-           "tb_solve_ragged_host", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
+           "tb_solve_ragged_host", "tb_solve_ragged_env", "tb_ragged_env_order", "tb_ragged_limits", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
 _lib = None
@@ -199,6 +199,9 @@ def lib():
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
     L.tb_solve_ragged_host.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut)]
+    L.tb_solve_ragged_env.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
+    L.tb_ragged_env_order.argtypes = [C.POINTER(TbRaggedIn), vp, vp, vp]
+    L.tb_ragged_limits.argtypes = [i32, C.POINTER(i32), C.POINTER(i32)]
     L.tb_adjoint_ragged.argtypes = [C.POINTER(TbRaggedIn), vp, C.POINTER(TbAdjIn), C.POINTER(TbAdjOut), vp, vp]
     L.tb_pinned_alloc.argtypes = [C.POINTER(vp), C.c_size_t]
     L.tb_pinned_free.argtypes = [vp]
@@ -622,6 +625,13 @@ def small_path_limits():
     return a.value, b.value
 
 
+def ragged_limits(dim: int):
+    """(max_joint, max_member): the largest trusses ``tb_solve_ragged`` accepts for this dim."""
+    a, b = C.c_int32(), C.c_int32()
+    check(lib().tb_ragged_limits(int(dim), C.byref(a), C.byref(b)))
+    return a.value, b.value
+
+
 def solve_ragged_host(dim, joint_off, member_off, xyz, support, conn, aed, force, want=("u", "ext", "axial", "weight"),
                       out=None):
     """B independent trusses with their own topology (generate.py:354-357), packed back to back.  ``out`` may hold
@@ -666,7 +676,7 @@ def _ragged_in(dim, packed, max_joint=None, max_member=None):
                       _ptr(packed["aed"]), _ptr(packed["force"]), int(max_joint), int(max_member))
 
 
-def solve_ragged_device(dim, packed, out=None, stream=None, max_joint=None, max_member=None):
+def solve_ragged_device(dim, packed, out=None, stream=None, max_joint=None, max_member=None, _entry="tb_solve_ragged"):
     """tb_solve_ragged on torch CUDA tensors: ``packed`` holds joint_off, member_off [B+1] (int64), xyz [d sum nJ],
     support [sum nJ] (uint8), conn [2 sum M] (int32, local joint ids), aed [3 sum M] and force [d sum nJ] (float64), as
     ``gencube_device`` / ``augment_and_solve_device`` return them.  ``out`` may hold preallocated u, ext [d sum nJ],
@@ -684,8 +694,28 @@ def solve_ragged_device(dim, packed, out=None, stream=None, max_joint=None, max_
             out[k] = torch.empty(n, dtype=dt, device=dev)
     st = torch.cuda.current_stream() if stream is None else stream
     bo = TbBatchOut(_ptr(out["u"]), _ptr(out["ext"]), _ptr(out["axial"]), _ptr(out["weight"]), _ptr(out["info"]))
-    check(lib().tb_solve_ragged(C.byref(ri), C.byref(bo), C.c_void_p(st.cuda_stream)))
+    check(getattr(lib(), _entry)(C.byref(ri), C.byref(bo), C.c_void_p(st.cuda_stream)))
     return out
+
+
+def solve_ragged_env_device(dim, packed, out=None, stream=None, max_joint=None, max_member=None):
+    """``solve_ragged_device`` with every truss on the envelope kernel (``tb_solve_ragged_env``), whatever its size."""
+    return solve_ragged_device(dim, packed, out, stream, max_joint, max_member, _entry="tb_solve_ragged_env")
+
+
+def ragged_env_order_device(dim, packed, stream=None, max_joint=None, max_member=None):
+    """The ordering mode of the envelope kernel (``tb_ragged_env_order``): returns ``(order, envelope)``, torch CUDA
+    tensors of each truss's joints in elimination order [sum nJ] (int32, local ids) and the row-envelope entries of its
+    K_ff in that order [B] (int64)."""
+    import torch
+
+    ri = _ragged_in(dim, packed, max_joint, max_member)
+    dev = packed["xyz"].device
+    order = torch.empty(max(int(packed["support"].numel()), 1), dtype=torch.int32, device=dev)
+    env = torch.empty(max(ri.batch, 1), dtype=torch.int64, device=dev)
+    st = torch.cuda.current_stream() if stream is None else stream
+    check(lib().tb_ragged_env_order(C.byref(ri), _ptr(order), _ptr(env), C.c_void_p(st.cuda_stream)))
+    return order[:int(packed["support"].numel())], env[:ri.batch]
 
 
 def adjoint_ragged_device(dim, packed, u, grads, out, stream=None, max_joint=None, max_member=None, work=None):

@@ -143,6 +143,13 @@ def _packed_input(t, default, shapes, name):
     return t
 
 
+def _refuse_beyond_fused(dim, joint_off, max_joint, max_member):
+    """Reverse mode exists for the fused kernels' trusses only: a batch beyond them (which the forward would solve on the
+    envelope kernel) is refused before any launch."""
+    if joint_off.shape[0] > 1 and not _lib.small_path_fits(dim, max_joint, max_member):
+        raise _lib.TrussLibError(_lib.TB_ERR_TOO_LARGE, "no reverse mode for a ragged batch beyond the fused kernels")
+
+
 def solve_ragged(packed, xyz=None, aed=None, force=None, max_joint=None, max_member=None):
     """``Truss.Solve()`` for a ragged batch (every truss its own topology), differentiable with respect to ``xyz``,
     ``aed`` and ``force``.
@@ -175,6 +182,8 @@ def solve_ragged(packed, xyz=None, aed=None, force=None, max_joint=None, max_mem
     aed = _packed_input(aed, packed.get("aed"), [(SM, 3), (SM * 3,)], "aed")
     force = _packed_input(force, packed.get("force"), [(SJ * dim,)], "force")
     base = {k: packed[k] for k in ("joint_off", "member_off", "support", "conn")}
+    if max_joint is not None and max_member is not None:                 # (sizes known: refused before anything else)
+        _refuse_beyond_fused(dim, base["joint_off"], max_joint, max_member)
     for k, t in list(base.items()) + [("xyz", xyz), ("aed", aed), ("force", force)]:   # (dtypes and shapes first)
         if not t.is_cuda or t.device != xyz.device:
             raise TypeError(f"{k} must be a CUDA tensor on the device of xyz")
@@ -184,6 +193,7 @@ def solve_ragged(packed, xyz=None, aed=None, force=None, max_joint=None, max_mem
         mj, mm = torch.stack([(jo[1:] - jo[:-1]).max(), (mo[1:] - mo[:-1]).max()]).tolist()
         max_joint = mj if max_joint is None else max_joint
         max_member = mm if max_member is None else max_member
+    _refuse_beyond_fused(dim, jo, max_joint, max_member)
     with torch.cuda.device(xyz.device):
         u, ext, axial, weight, info = _SolveRagged.apply(xyz, aed, force, base["joint_off"], base["member_off"], base["support"],
                                                          base["conn"], dim, max_joint, max_member)

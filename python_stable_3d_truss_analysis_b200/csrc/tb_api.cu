@@ -1,6 +1,7 @@
 // C-ABI entry points (include/truss_b200.h).  Device variants enqueue on the caller's stream;
 // *_host variants stage host buffers through a grow-only device arena owned by the plan (or a
 // process-wide one for ragged batches), run the same device path, and copy the results back.
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
@@ -661,6 +662,99 @@ int run_ragged(const tb_ragged_in* in, const tb_batch_out* out, cudaStream_t st)
 void* g_rag_dev[TB_MAX_DEVICES] = {};
 size_t g_rag_dev_bytes[TB_MAX_DEVICES] = {};
 
+// Argument checks of the ragged forward entry points: as check_ragged, up to the envelope kernel's limits
+int check_ragged_fwd(const tb_ragged_in* in) {
+  if (!in) return TB_ERR_NULL;
+  if (in->dim != 2 && in->dim != 3) return TB_ERR_DIM;
+  if (in->batch < 0 || in->max_joint < 0 || in->max_member < 0) return TB_ERR_SIZE;
+  if (in->batch == 0) return TB_OK;
+  if (!in->joint_off || !in->member_off || !in->joint_xyz || !in->support || !in->conn || !in->member_aed || !in->force)
+    return TB_ERR_NULL;
+  if ((int64_t)in->max_joint * in->dim > TB_RAGGED_MAX_DOF || in->max_member > TB_RAGGED_MAX_MEMBER) return TB_ERR_TOO_LARGE;
+  return TB_OK;
+}
+
+bool ragged_fits_fused(const tb_ragged_in* in) {
+  return tb_small_fits(in->dim, in->max_joint, in->max_member, in->max_joint * in->dim);
+}
+
+// Scratch of the envelope kernel: one grow-only arena per device (one slot per CTA of the persistent grid), grown
+// stream-ordered on the caller's stream.  `mu` serialises the calls on the device; `ev` orders the arena's use across
+// streams (recorded after a call's kernel; a call on another stream waits for it first).
+struct EnvScratch {
+  std::mutex mu;
+  void* buf = nullptr;
+  size_t bytes = 0;
+  cudaEvent_t ev = nullptr;
+  cudaStream_t last = nullptr;
+  bool used = false;
+};
+EnvScratch g_env[TB_MAX_DEVICES];
+
+// Envelope kernel over a batch: every truss (route = false), only the trusses above the fused launch's sizes (route:
+// those run first, in one fused launch of the batch), or the ordering mode (order != null).  Inside a stream capture
+// the arena is never grown: TB_ERR_ALLOC with nothing enqueued.
+int run_env(const tb_ragged_in* in, const tb_batch_out* out, bool route, int32_t* order, int64_t* envelope, cudaStream_t st) {
+  const int d = in->dim;
+  int dev = 0;
+  TB_CUDA(cudaGetDevice(&dev));
+  EnvScratch& S = g_env[dev & (TB_MAX_DEVICES - 1)];
+  std::lock_guard<std::mutex> lock(S.mu);       // (also keeps the kernel's shared-memory attribute until the launch)
+  int grid = 0, smem = 0, env_smem = 0;
+  int rc = tb_rag_env_config(d, in->max_joint, in->max_member, in->batch, &grid, &smem, &env_smem);
+  if (rc) return rc;
+  const size_t slot = tb_rag_env_slot_bytes(d, in->max_joint, in->max_member);
+  const size_t need = slot * (size_t)grid;
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
+  const bool capturing = cap != cudaStreamCaptureStatusNone;
+  if (S.bytes < need && capturing) return TB_ERR_ALLOC;          // (a warm-up call outside the capture grows it)
+  if (!capturing && S.used && S.last != st && S.ev) TB_CUDA(cudaStreamWaitEvent(st, S.ev, 0));
+  if (S.bytes < need) {                                          // stream-ordered: the previous call is ahead on st
+    if (S.buf) TB_CUDA(cudaFreeAsync(S.buf, st));
+    S.buf = nullptr;
+    S.bytes = 0;
+    TB_CUDA(cudaMallocAsync(&S.buf, need, st));
+    S.bytes = need;
+  }
+  const int rj = d == 3 ? TB_RAGGED_ROUTE_J3 : TB_RAGGED_ROUTE_J2, rm = d == 3 ? TB_RAGGED_ROUTE_M3 : TB_RAGGED_ROUTE_M2;
+  if (route) {                                   // the fused kernels first, sized at the routing limits (k_dense16)
+    tb_ragged_in fin = *in;
+    fin.max_joint = std::min(in->max_joint, rj);
+    fin.max_member = std::min(in->max_member, rm);
+    rc = run_ragged(&fin, out, st);
+    if (rc) return rc;
+  }
+  RagEnvArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.dim = d; a.max_joint = in->max_joint; a.max_member = in->max_member;
+  a.route_joint = route ? rj : 0;
+  a.route_member = route ? rm : 0;
+  a.joint_off = in->joint_off; a.member_off = in->member_off;
+  a.xyz = in->joint_xyz; a.support = in->support; a.conn = in->conn; a.aed = in->member_aed; a.force = in->force;
+  if (out) { a.u = out->u; a.ext = out->ext; a.axial = out->axial; a.weight = out->weight; a.info = out->info; }
+  a.order = order;
+  a.envelope = envelope;
+  a.scratch = S.buf;
+  a.slot_bytes = slot;
+  a.env_smem = env_smem;
+  rc = tb_launch_rag_env(a, grid, smem, st);
+  if (rc) return rc;
+  if (!capturing) {
+    if (!S.ev) TB_CUDA(cudaEventCreateWithFlags(&S.ev, cudaEventDisableTiming));
+    TB_CUDA(cudaEventRecord(S.ev, st));
+    S.last = st;
+    S.used = true;
+  }
+  return TB_OK;
+}
+
+// The forward of a ragged batch: today's fused launch when the whole batch fits the fused kernels, else split by truss
+int run_ragged_fwd(const tb_ragged_in* in, const tb_batch_out* out, cudaStream_t st) {
+  if (ragged_fits_fused(in)) return run_ragged(in, out, st);
+  return run_env(in, out, true, nullptr, nullptr, st);
+}
+
 }  // namespace
 
 extern "C" int tb_solve(tb_plan* plan, const tb_batch_in* in, const tb_batch_out* out, void* cuda_stream) {
@@ -733,17 +827,44 @@ extern "C" int tb_fitness_host(tb_plan* plan, const tb_batch_in* in, double allo
 
 extern "C" int tb_solve_ragged(const tb_ragged_in* in, const tb_batch_out* out, void* cuda_stream) {
   if (out && (out->u_free || out->react)) return TB_ERR_SIZE;   // (the compact layout needs one n and s for the whole batch)
-  int rc = check_ragged(in);
+  int rc = check_ragged_fwd(in);
   if (rc) return rc;
   if (!out) return TB_ERR_NULL;
   if (!have_device()) return TB_ERR_NO_DEVICE;
   if (in->batch == 0) return TB_OK;
-  return run_ragged(in, out, (cudaStream_t)cuda_stream);
+  return run_ragged_fwd(in, out, (cudaStream_t)cuda_stream);
+}
+
+extern "C" int tb_solve_ragged_env(const tb_ragged_in* in, const tb_batch_out* out, void* cuda_stream) {
+  if (out && (out->u_free || out->react)) return TB_ERR_SIZE;
+  int rc = check_ragged_fwd(in);
+  if (rc) return rc;
+  if (!out) return TB_ERR_NULL;
+  if (!have_device()) return TB_ERR_NO_DEVICE;
+  if (in->batch == 0) return TB_OK;
+  return run_env(in, out, false, nullptr, nullptr, (cudaStream_t)cuda_stream);
+}
+
+extern "C" int tb_ragged_env_order(const tb_ragged_in* in, int32_t* order, int64_t* envelope, void* cuda_stream) {
+  int rc = check_ragged_fwd(in);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  if (!order || !envelope) return TB_ERR_NULL;
+  if (!have_device()) return TB_ERR_NO_DEVICE;
+  return run_env(in, nullptr, false, order, envelope, (cudaStream_t)cuda_stream);
+}
+
+extern "C" int tb_ragged_limits(int32_t dim, int32_t* max_joint, int32_t* max_member) {
+  if (dim != 2 && dim != 3) return TB_ERR_DIM;
+  if (!max_joint || !max_member) return TB_ERR_NULL;
+  *max_joint = TB_RAGGED_MAX_DOF / dim;
+  *max_member = TB_RAGGED_MAX_MEMBER;
+  return TB_OK;
 }
 
 extern "C" int tb_solve_ragged_host(const tb_ragged_in* in, const tb_batch_out* out) {
   if (out && (out->u_free || out->react)) return TB_ERR_SIZE;
-  int rc = check_ragged(in);
+  int rc = check_ragged_fwd(in);
   if (rc) return rc;
   if (!out) return TB_ERR_NULL;
   if (!have_device()) return TB_ERR_NO_DEVICE;
@@ -798,7 +919,7 @@ extern "C" int tb_solve_ragged_host(const tb_ragged_in* in, const tb_batch_out* 
   dout.axial = out->axial ? take<double>(cur, SM) : nullptr;
   dout.weight = out->weight ? take<double>(cur, (size_t)B) : nullptr;
   dout.info = take<int32_t>(cur, (size_t)B);
-  rc = run_ragged(&din, &dout, st);
+  rc = run_ragged_fwd(&din, &dout, st);
   if (rc) return rc;
   if (out->u) TB_CUDA(cudaMemcpyAsync(out->u, dout.u, SJ * d * 8, cudaMemcpyDeviceToHost, st));
   if (out->ext) TB_CUDA(cudaMemcpyAsync(out->ext, dout.ext, SJ * d * 8, cudaMemcpyDeviceToHost, st));

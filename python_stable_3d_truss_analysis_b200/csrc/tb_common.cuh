@@ -35,6 +35,17 @@ constexpr int TB_SMALL_MAX_DOF = 160;     // max d*nJ (bounds the free-DOF count
 constexpr int TB_SMALL_MAX_MEMBER = 1024;
 constexpr int TB_SMALL_MAX_JOINT = 80;
 
+// Ragged batches beyond the fused kernels (tb_ragenv.cu): the envelope kernel k_rag_env takes trusses up to
+// TB_RAGGED_MAX_DOF = d*nJ and TB_RAGGED_MAX_MEMBER members (the generator's largest truss on a 6^3 grid is 343 joints
+// and 5184 members; bar-942 is 732 DOFs).  A batch that does not fit the fused kernels as a whole is split by truss: the
+// trusses up to (TB_RAGGED_ROUTE_J<d>, TB_RAGGED_ROUTE_M<d>) run on the fused kernels in one launch of that size (it stays
+// on k_dense16 -- at most 9 blocks of 16 free DOFs and 110 KB of shared memory per warp -- and cube-7's 32 joints / 119
+// members are under it), the others on k_rag_env.
+constexpr int TB_RAGGED_MAX_DOF = 1536;
+constexpr int TB_RAGGED_MAX_MEMBER = 8192;
+constexpr int TB_RAGGED_ROUTE_J3 = 48, TB_RAGGED_ROUTE_M3 = 192;
+constexpr int TB_RAGGED_ROUTE_J2 = 72, TB_RAGGED_ROUTE_M2 = 224;
+
 extern std::atomic<int64_t> g_tb_launches;
 inline void tb_count_launch(int n = 1) { g_tb_launches.fetch_add(n, std::memory_order_relaxed); }
 
@@ -336,6 +347,24 @@ struct TbAdjRaggedArgs {
 };
 int tb_launch_adj_rhs_ragged(const TbAdjRaggedArgs& a, cudaStream_t st);
 int tb_launch_sens_ragged(const TbAdjRaggedArgs& a, cudaStream_t st);
+
+// Envelope path of ragged batches (tb_ragenv.cu): one CTA per truss, one scratch slot per CTA
+struct RagEnvArgs {
+  int batch, dim, max_joint, max_member;   // the slots are sized from max_joint / max_member
+  int route_joint, route_member;           // > 0: skip the trusses up to these sizes (the fused kernels solved them)
+  const int64_t* joint_off; const int64_t* member_off;
+  const double* xyz; const uint8_t* support; const int32_t* conn; const double* aed; const double* force;
+  double* u; double* ext; double* axial; double* weight; int32_t* info;
+  int32_t* order;        // ordering mode when non-null: [sum nJ] joints in elimination order (local ids), nothing solved
+  int64_t* envelope;     // ordering mode: [B] row-envelope entries of K_ff in that order
+  void* scratch;         // grid * slot_bytes
+  size_t slot_bytes;
+  int env_smem;          // envelope doubles that fit the launch's dynamic shared memory
+};
+size_t tb_rag_env_slot_bytes(int dim, int max_joint, int max_member);
+// persistent grid (at most one CTA per truss), dynamic shared memory and its envelope budget of a launch
+int tb_rag_env_config(int dim, int max_joint, int max_member, int batch, int* grid, int* smem_bytes, int* env_smem);
+int tb_launch_rag_env(const RagEnvArgs& a, int grid, int smem_bytes, cudaStream_t st);
 
 // fragment-major offset of element (r, c) inside one 64x64 tile:
 //   [k-half 2][row-block 8][k-slab 8][lane 32], lane = (r%8)*4 + c%4
