@@ -39,7 +39,8 @@ def SolveLoadCases(truss: Truss, forces, raise_on_error=True, independent=False)
     """One truss under B load cases.  ``forces`` is [B, N] dense (index jointID*dim + axis).
 
     Equivalent to ``for f in forces: truss.SetForces(f); truss.Solve()`` (truss.py:329-364).  The stiffness matrix is the
-    same for every load case, so on the band path it is assembled and factorised once (tb_solve_loadcases_host);
+    same for every load case, so on the band path it is assembled and factorised once (tb_solve_loadcases_host) when
+    the member products fit shared memory (else every load case is factorised on its own);
     ``independent=True`` factorises every system on its own, as a batch of unrelated trusses would (tb_solve_host)."""
     xyz, support, conn, aed, _ = truss._pack()
     forces = np.ascontiguousarray(forces, dtype=np.float64).reshape(-1, truss.nJoint * truss.dim)

@@ -1255,8 +1255,10 @@ int tb_launch_large(const LargeArgs& a, int num_sm, cudaStream_t st, int path) {
   }
   if (use_ts) return launch_ts_path(a, num_sm, st);
   if (!prep) k_init_status<<<(a.batch + 255) / 256, 256, 0, st>>>(a.status, a.batch, 0);   // k_prep clears its own
-  // load cases of one truss (shared_k): assembly and factorisation run for system 0 only
-  const bool shared = a.shared_k && path == 2 && prep && a.batch > 1;
+  // load cases of one truss (shared_k): assembly and factorisation run for system 0 only.  A batch of one load case
+  // takes the same route (not the factorisation kernel's own substitution), so a load case's bits do not depend on the
+  // size of the batch or of the chunk it is solved in.  Without k_prep every load case is factorised on its own.
+  const bool shared = a.shared_k && path == 2 && prep;
   LargeArgs a1 = a;
   a1.batch = 1;
   if (prep) {

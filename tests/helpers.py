@@ -171,14 +171,19 @@ def tower(dim, per_level, levels, seed):
 
 
 # --------------------------------------------------------------------------- which CUDA kernels ran (GPU tests)
-_KERNEL_TAG = re.compile(r"(k_band_ts|k_band[123]|k_prep)(?:<|ILi)(\d+)")
+_KERNEL_TAG = re.compile(r"(k_band_subst8|k_band_subst|k_band_ts|k_band[123]|k_prep|k_geom|k_recover)"
+                         r"(?:<(\d+)(?:, (true|false))?|ILi(\d+)E(?:Lb([01])E)?)")
 
 
 def kernel_tag(name: str):
-    """'k_band_ts<7>', 'k_band2<4>' (the band kernels by NB), 'k_prep<3>' (by dim) from a demangled or mangled kernel
-    name; None for any other kernel."""
+    """'k_band_ts<7>', 'k_band2<4>' (the band kernels by NB), 'k_band_subst8<4>', 'k_band_subst<4>' (the shared-factor
+    substitutions by NB), 'k_prep<3>', 'k_geom<3>' (by dim), 'k_recover<3,false>' (by dim and member-product placement),
+    'k_kval' from a demangled or mangled kernel name; None for any other kernel."""
     m = _KERNEL_TAG.search(name)
-    return f"{m.group(1)}<{m.group(2)}>" if m else None
+    if m:
+        flag = m.group(3) or {"0": "false", "1": "true"}.get(m.group(5))
+        return f"{m.group(1)}<{m.group(2) or m.group(4)}" + (f",{flag}>" if m.group(1) == "k_recover" and flag else ">")
+    return "k_kval" if "k_kval" in name else None
 
 
 def cuda_kernels(fn):
@@ -200,11 +205,17 @@ def cuda_kernels(fn):
 
 def band_kernels(seen):
     """The band factorisation kernels among cuda_kernels()' tags."""
-    return sorted(t for t in seen if t.startswith("k_band"))
+    return sorted(t for t in seen if t.startswith("k_band") and not t.startswith("k_band_subst"))
 
 
-def solve_device_np(plan, B, xyz, aed, force):
-    """plan.solve_device on CUDA copies of numpy inputs (leading dimension B, or shared); returns numpy outputs."""
+def subst_kernels(seen):
+    """The shared-factor substitution kernels among cuda_kernels()' tags."""
+    return sorted(t for t in seen if t.startswith("k_band_subst"))
+
+
+def solve_device_np(plan, B, xyz, aed, force, shared_factor=False):
+    """plan.solve_device on CUDA copies of numpy inputs (leading dimension B, or shared); returns numpy outputs.
+    ``shared_factor``: the B systems are load cases of one truss (xyz and aed shared)."""
     import torch
 
     dev = torch.device("cuda:0")
@@ -212,7 +223,7 @@ def solve_device_np(plan, B, xyz, aed, force):
     f64 = dict(dtype=torch.float64, device=dev)
     out = {"u": torch.empty(B, plan.N, **f64), "ext": torch.empty(B, plan.N, **f64), "axial": torch.empty(B, plan.M, **f64),
            "weight": torch.empty(B, **f64), "info": torch.empty(B, dtype=torch.int32, device=dev)}
-    plan.solve_device(B, td(xyz), td(force), aed=td(aed), out=out)
+    plan.solve_device(B, td(xyz), td(force), aed=td(aed), out=out, shared_factor=shared_factor)
     torch.cuda.synchronize()
     return {k: v.cpu().numpy() for k, v in out.items()}
 
@@ -234,13 +245,23 @@ sys.path.insert(0, {root!r})
 from tests import band_catalogue as BC
 from tests import helpers as H
 seen_all = []
-for job in json.loads(sys.argv[1]):
-    e = BC.get(job["label"])
+for job in json.load(open(sys.argv[1])):
+    e = BC.get(job["label"]) if "data" not in job else BC.Entry(job["label"], job["dim"], job["data"], {{}})
     plan = BC.plan_for(e)
     plan.set_path(2)
     xyz, aed, F = BC.inputs(plan, e, job["B"], seed=job["seed"])
     lo, hi = job.get("slice", (0, job["B"]))
-    out, seen = H.cuda_kernels(lambda: H.solve_device_np(plan, hi - lo, xyz, aed[lo:hi], F[lo:hi]))
+    if job.get("shared"):
+        aed = BC.arrays(e)[3]
+        if "force" in job:
+            F = np.load(job["force"])
+        if job.get("host"):
+            run = lambda: plan.solve_host(hi - lo, xyz, F[lo:hi], aed=aed, shared_factor=True)
+        else:
+            run = lambda: H.solve_device_np(plan, hi - lo, xyz, aed, F[lo:hi], shared_factor=True)
+    else:
+        run = lambda: H.solve_device_np(plan, hi - lo, xyz, aed[lo:hi], F[lo:hi])
+    out, seen = H.cuda_kernels(run)
     np.savez(job["dst"], **out)
     seen_all.append(seen)
 json.dump(seen_all, open(sys.argv[2], "w"))
@@ -248,18 +269,25 @@ json.dump(seen_all, open(sys.argv[2], "w"))
 
 
 def run_band_child(tmp_dir, env, jobs):
-    """Band-path solves of catalogue entries (tests/band_catalogue.py) in a fresh process with `env` added: the
-    switches TB_BAND_LEGACY, TB_BAND_WARPS and TB_LARGE_SPLIT are read once per process.  Each job is {"label", "B",
-    "seed"} and optionally "slice": [lo, hi] (solve only systems lo .. hi-1 of the B-system inputs).  Returns
-    [(numpy outputs, {kernel tag: launches})] per job."""
+    """Band-path solves in a fresh process with `env` added: the switches TB_BAND_LEGACY, TB_BAND_WARPS,
+    TB_LARGE_SPLIT, TB_SUBST_TILE, TB_HOST_CHUNKS and TB_WORKSPACE_MAX_GB are read once per process.  Each job is
+    {"label", "B", "seed"}: a catalogue entry (tests/band_catalogue.py), or any truss when the job also has "dim" and
+    "data" (the reference's JSON form).  Optional fields:
+      "slice": [lo, hi]   solve only systems lo .. hi-1 of the B-system inputs;
+      "shared": true      the B systems are load cases of the truss as it is (tb_solve_loadcases): one xyz / aed;
+      "host": true        (with "shared") through the blocking host entry point tb_solve_loadcases_host;
+      "force": path       (with "shared") the load cases, a [B, N] .npy file, instead of band_catalogue.inputs'.
+    Returns [(numpy outputs, {kernel tag: launches})] per job."""
     import subprocess
     import sys
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     tag = "_".join(f"{k}{v}" for k, v in sorted(env.items())) or "default"
     jobs = [dict(j, dst=os.path.join(str(tmp_dir), f"{tag}_{i}.npz")) for i, j in enumerate(jobs)]
+    jobs_path = os.path.join(str(tmp_dir), f"{tag}_jobs.json")
     seen_path = os.path.join(str(tmp_dir), f"{tag}_kernels.json")
-    subprocess.run([sys.executable, "-c", _BAND_CHILD.format(root=root), json.dumps(jobs), seen_path], check=True,
+    json.dump(jobs, open(jobs_path, "w"))
+    subprocess.run([sys.executable, "-c", _BAND_CHILD.format(root=root), jobs_path, seen_path], check=True,
                    env=dict(os.environ, **env), timeout=600)
     seen = json.load(open(seen_path))
     return [(dict(np.load(j["dst"])), s) for j, s in zip(jobs, seen)]
