@@ -78,6 +78,8 @@ extern "C" {
 #define TB_INFO_ZERO_LENGTH (-2)
 #define TB_INFO_BAD_SUPPORT (-3)
 #define TB_INFO_BAD_INDEX (-4)
+#define TB_INFO_MASS (-5)            /* tb_modes: M_ff is not positive definite */
+#define TB_INFO_NO_CONVERGENCE (-6)  /* tb_modes: the tridiagonal QL iteration hit its cap */
 
 typedef struct tb_plan tb_plan; /* opaque */
 
@@ -234,6 +236,42 @@ int tb_solve_loadcases_host(tb_plan* plan, const tb_batch_in* in, const tb_batch
  * stream without synchronising; the adjoint scratch is the plan's (grow-only, grown in stream order). */
 int tb_adjoint(tb_plan* plan, const tb_batch_in* in, const double* u, const tb_adj_in* grad, const tb_adj_out* out,
                int32_t shared_factor, void* cuda_stream);
+
+/* ---- Modal analysis (free vibration; DESIGN.md section 11) ----------------------------------------------------------
+ * For each system of a uniform batch: the n_modes lowest eigenvalues lambda = omega^2 of K_ff phi = lambda M_ff phi over
+ * the free DOFs (supported DOFs dropped as in tb_solve), ascending, and optionally the mode shapes.  K_ff is the static
+ * solve's stiffness matrix (the same member geometry and ascending-member sums).  Member mass m_e = (a L) density, the
+ * weight term's product and rounding; its units are the caller's (a weight density must be divided by g first).
+ *   lumped (consistent = 0): m_e / 2 on every axis of both end joints;
+ *   consistent (consistent = 1): (m_e / 6) [[2, 1], [1, 2]] per member and axis over its two end joints;
+ *   joint_mass: a non-structural mass added on every axis of its joint (both models).
+ * Mode shapes are dense over the N DOFs (0 at supported DOFs, the layout of u), M-normalised (phi^T M_ff phi = 1), with
+ * the component of largest magnitude positive (on a tie the lowest DOF index decides).  K is never factorised: a
+ * mechanism that passes the counting rule is not an error, it shows as eigenvalues ~ 0 with info 0.
+ * info: 0, TB_INFO_NOT_STABLE (counting rule), TB_INFO_ZERO_LENGTH, TB_INFO_BAD_INDEX (a gene out of range) as tb_solve,
+ * TB_INFO_MASS (lumped: a free DOF has mass <= 0; consistent: the Cholesky factorisation of M_ff fails),
+ * TB_INFO_NO_CONVERGENCE; a failed system gets zero outputs.
+ * Plans with n <= 160 free DOFs (TB_SMALL_MAX_DOF); larger: TB_ERR_TOO_LARGE before any launch.  `in` as tb_solve
+ * (explicit member_aed or gene + type_table); in->force is ignored and may be NULL.  Required: m, out->eigval, out->info
+ * (TB_ERR_NULL); 1 <= n_modes <= n (TB_ERR_SIZE).  tb_modes enqueues on the stream and never synchronises.  Consistent
+ * mass uses the plan's modal scratch (one n x n slot per CTA of the persistent grid, grow-only, grown stream-ordered on
+ * the caller's stream); a call inside a stream capture never grows it: TB_ERR_ALLOC with nothing enqueued (a warm-up call
+ * outside the capture grows it).  Lumped mass needs no scratch. */
+typedef struct {
+  int32_t n_modes;            /* 1 <= n_modes <= n (free DOFs), else TB_ERR_SIZE */
+  int32_t consistent;         /* 0: lumped mass, 1: consistent mass */
+  const double* joint_mass;   /* [B][nJ] non-structural mass per joint, or NULL */
+  int64_t joint_mass_stride;  /* 0 = shared */
+} tb_modes_in;
+
+typedef struct {
+  double* eigval;             /* [B][n_modes] lambda = omega^2, ascending -- required */
+  double* modes;              /* [B][n_modes][N] M-normalised, 0 at supports -- or NULL */
+  int32_t* info;              /* [B] -- required */
+} tb_modes_out;
+
+int tb_modes(tb_plan* plan, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out, void* cuda_stream);
+int tb_modes_host(tb_plan* plan, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out);
 
 /* GA.GetFitness for B genes (ga.py:139-149); `full` may be NULL or receive the full results. */
 int tb_fitness(tb_plan* plan, const tb_batch_in* in, double allow_stress, double allow_displace,

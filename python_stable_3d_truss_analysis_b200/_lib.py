@@ -18,10 +18,14 @@ CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 LIB_PATH = os.environ.get("TB_LIB_PATH") or os.path.join(CSRC, "libtruss_b200.so")   # TB_LIB_PATH: instrumented builds (tools/)
 SOURCES = ["tb_plan.cu", "tb_tsplan.cu", "tb_small.cu", "tb_dense16.cu", "tb_large.cu", "tb_band.cu", "tb_bandts.cu", "tb_api.cu", "tb_adjoint.cu", "tb_peak.cu",
-           "tb_ga.cu", "tb_augment.cu", "tb_json.cu", "tb_gencube.cu", "tb_ragenv.cu"]
+           "tb_ga.cu", "tb_augment.cu", "tb_json.cu", "tb_gencube.cu", "tb_ragenv.cu", "tb_modes.cu"]
 
 TB_ERR_NO_DEVICE = -7
 TB_ERR_TOO_LARGE = -6
+TB_ERR_ALLOC = -8
+# per-system status codes of tb_modes beyond those of the static solve (include/truss_b200.h)
+TB_INFO_MASS = -5                # M_ff is not positive definite
+TB_INFO_NO_CONVERGENCE = -6      # the tridiagonal QL iteration hit its cap
 
 
 class TrussLibError(RuntimeError):
@@ -156,6 +160,15 @@ class TbFitOut(C.Structure):
     _fields_ = [("fitness", C.c_void_p), ("flags", C.c_void_p), ("info", C.c_void_p)]
 
 
+class TbModesIn(C.Structure):
+    _fields_ = [("n_modes", C.c_int32), ("consistent", C.c_int32), ("joint_mass", C.c_void_p),
+                ("joint_mass_stride", C.c_int64)]
+
+
+class TbModesOut(C.Structure):
+    _fields_ = [("eigval", C.c_void_p), ("modes", C.c_void_p), ("info", C.c_void_p)]
+
+
 class TbRaggedIn(C.Structure):
     _fields_ = [("dim", C.c_int32), ("batch", C.c_int32), ("joint_off", C.c_void_p), ("member_off", C.c_void_p),
                 ("joint_xyz", C.c_void_p), ("support", C.c_void_p), ("conn", C.c_void_p), ("member_aed", C.c_void_p),
@@ -163,7 +176,7 @@ class TbRaggedIn(C.Structure):
 
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
-           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
+           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
            "tb_solve_ragged_host", "tb_solve_ragged_env", "tb_ragged_env_order", "tb_ragged_limits", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
@@ -195,6 +208,8 @@ def lib():
     L.tb_solve_loadcases.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBatchOut), vp]
     L.tb_solve_loadcases_host.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBatchOut)]
     L.tb_adjoint.argtypes = [vp, C.POINTER(TbBatchIn), vp, C.POINTER(TbAdjIn), C.POINTER(TbAdjOut), i32, vp]
+    L.tb_modes.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbModesIn), C.POINTER(TbModesOut), vp]
+    L.tb_modes_host.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbModesIn), C.POINTER(TbModesOut)]
     L.tb_fitness.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut), vp]
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
@@ -595,6 +610,60 @@ class Plan:
         go = TbAdjOut(_ptr(out.get("joint_xyz")), _ptr(out.get("member_aed")), _ptr(out.get("force")), _ptr(out.get("info")))
         check(lib().tb_adjoint(self._h, C.byref(bi), _ptr(u), C.byref(gi), C.byref(go), 1 if shared_factor else 0,
                                C.c_void_p(st.cuda_stream)))
+        return out
+
+    def _modes_in(self, B, n_modes, consistent, joint_mass, keep):
+        """tb_modes_in; ``n_modes=None`` asks for all n modes, ``joint_mass`` is [nJ] (shared) or [B, nJ]."""
+        mi = TbModesIn()
+        mi.n_modes = self.n if n_modes is None else int(n_modes)
+        mi.consistent = 1 if consistent else 0
+        if joint_mass is not None:
+            jm = _np(joint_mass, np.float64) if isinstance(joint_mass, (np.ndarray, list, tuple)) else joint_mass
+            total = int(np.prod(jm.shape))
+            if total not in (self.nJ, self.nJ * B):
+                raise ValueError(f"joint_mass of {total} elements is neither [{self.nJ}] nor [{B},{self.nJ}]")
+            keep.append(jm)
+            mi.joint_mass, mi.joint_mass_stride = _ptr(jm), 0 if total == self.nJ else self.nJ
+        return mi
+
+    def modes_host(self, B, xyz, aed=None, gene=None, type_table=None, n_modes=None, consistent=False, joint_mass=None,
+                   out=None, want_modes=True):
+        """Modal analysis of B systems (tb_modes_host), host (numpy) buffers: ``eigval`` [B, n_modes] (lambda = omega^2,
+        ascending), ``modes`` [B, n_modes, N] (M-normalised, 0 at supported DOFs; skipped with ``want_modes=False``) and
+        ``info`` [B].  ``n_modes=None`` = all n modes."""
+        keep = []
+        bi = self._batch_in(B, xyz, aed, gene, type_table, np.zeros(self.N), keep)
+        bi.force, bi.force_stride = None, 0            # (ignored by tb_modes)
+        mi = self._modes_in(B, n_modes, consistent, joint_mass, keep)
+        nm = mi.n_modes
+        out = {} if out is None else out
+        out.setdefault("eigval", np.empty((B, nm), np.float64))
+        if want_modes:
+            out.setdefault("modes", np.empty((B, nm, self.N), np.float64))
+        out.setdefault("info", np.empty(B, np.int32))
+        mo = TbModesOut(_ptr(out["eigval"]), _ptr(out.get("modes")), _ptr(out["info"]))
+        check(lib().tb_modes_host(self._h, C.byref(bi), C.byref(mi), C.byref(mo)))
+        return out
+
+    def modes_device(self, B, xyz, aed=None, gene=None, type_table=None, n_modes=None, consistent=False, joint_mass=None,
+                     out=None, stream=None):
+        """tb_modes on torch CUDA tensors; enqueues on ``stream`` (a torch stream or None = current).  ``out`` maps
+        "eigval" [B, n_modes] and "info" [B] (allocated when missing) and optionally "modes" [B, n_modes, N]."""
+        import torch
+
+        keep = []
+        bi = self._batch_in(B, xyz, aed, gene, type_table, np.zeros(self.N), keep)
+        bi.force, bi.force_stride = None, 0            # (ignored by tb_modes)
+        mi = self._modes_in(B, n_modes, consistent, joint_mass, keep)
+        dev = xyz.device if hasattr(xyz, "device") else torch.device("cuda", torch.cuda.current_device())
+        out = {} if out is None else out
+        if out.get("eigval") is None:
+            out["eigval"] = torch.empty((B, mi.n_modes), dtype=torch.float64, device=dev)
+        if out.get("info") is None:
+            out["info"] = torch.empty(B, dtype=torch.int32, device=dev)
+        st = torch.cuda.current_stream() if stream is None else stream
+        mo = TbModesOut(_ptr(out["eigval"]), _ptr(out.get("modes")), _ptr(out["info"]))
+        check(lib().tb_modes(self._h, C.byref(bi), C.byref(mi), C.byref(mo), C.c_void_p(st.cuda_stream)))
         return out
 
     def fitness_device(self, B, xyz, force, gene, type_table, allow_stress, allow_displace, out, aed=None, stream=None):

@@ -9,6 +9,7 @@ hand the whole batch to the CUDA library in one call:
   ``SolveMemberTypes(truss, genes, types)``  one truss, many member-type assignments (GA population)
   ``FitnessBatch(...)``                      GA.GetFitness for a population (ga.py:139-149)
   ``SolveWithFixedMemberType(trusses, t)``   the graph-data converter's double solve (data.py:17-44, 108-114)
+  ``ModesBatch(truss, ...)``                 natural frequencies and mode shapes of many sizings of one truss
 
 All of them return dense numpy arrays (``u [B,N]``, ``ext [B,N]``, ``axial [B,M]``, ``weight [B]``,
 ``info [B]``); ``SolveBatch`` also stores the results back into the Truss objects.
@@ -18,7 +19,7 @@ from __future__ import annotations
 import numpy as np
 
 from . import _lib
-from .truss import ZERO_EPS, Truss, make_plan, raise_for_info
+from .truss import ZERO_EPS, Truss, make_plan, raise_for_info, raise_for_modes_info
 from .type import MemberType
 
 
@@ -69,6 +70,37 @@ def FitnessBatch(truss: Truss, genes, memberTypeList, allowStress, allowDisplace
     plan = truss._get_plan(support, conn)
     return plan.fitness_host(genes.shape[0], xyz, force, genes, type_table(memberTypeList), allowStress,
                              allowDisplace, full=full)
+
+
+def ModesBatch(truss: Truss, aed=None, genes=None, memberTypeList=None, nMode=None, isConsistentMass=False,
+               jointMasses=None, raise_on_error=True, want_modes=True):
+    """Modal analysis of B sizings of one truss in one call (tb_modes_host): ``Truss.SolveModes`` per design, e.g. the
+    frequency constraints of a GA population.  Member properties are either explicit, ``aed`` [B, M, 3] (a, e, density),
+    or ``genes`` int [B, M] of indices into ``memberTypeList``.  ``jointMasses``: {jointID: mass} shared by the batch, or
+    an array [nJ] / [B, nJ].  Returns dict(eigval [B, k] (lambda = omega^2, ascending), modes [B, k, N] (M-normalised, 0
+    at supported DOFs), info [B]); ``nMode=None`` = all modes."""
+    xyz, support, conn, _, _ = truss._pack()
+    plan = truss._get_plan(support, conn)
+    jm = jointMasses
+    if isinstance(jointMasses, dict):
+        jm = np.zeros(truss.nJoint)
+        for j, mass in jointMasses.items():
+            jm[j] = float(mass)
+    if (aed is None) == (genes is None):
+        raise ValueError("give either aed or genes (with memberTypeList)")
+    if aed is not None:
+        aed = np.ascontiguousarray(aed, dtype=np.float64).reshape(-1, truss.nMember * 3)
+        out = plan.modes_host(aed.shape[0], xyz, aed=aed, n_modes=nMode, consistent=isConsistentMass, joint_mass=jm,
+                              want_modes=want_modes)
+    else:
+        genes = np.ascontiguousarray(genes, dtype=np.int32).reshape(-1, truss.nMember)
+        out = plan.modes_host(genes.shape[0], xyz, gene=genes, type_table=type_table(memberTypeList), n_modes=nMode,
+                              consistent=isConsistentMass, joint_mass=jm, want_modes=want_modes)
+    if raise_on_error:
+        bad = np.nonzero(out["info"])[0]
+        if bad.size:
+            raise_for_modes_info(int(out["info"][bad[0]]))
+    return out
 
 
 def pack_ragged(trusses):

@@ -1099,6 +1099,149 @@ extern "C" int tb_adjoint_ragged(const tb_ragged_in* in, const double* u, const 
   return tb_launch_sens_ragged(a, st);
 }
 
+// ---- modal analysis (DESIGN.md section 11) ---------------------------------------------------------------------------
+namespace {
+
+// Argument checks of tb_modes / tb_modes_host: every argument error before the device checks
+int check_modes(const tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out) {
+  if (!p || !in || !m || !out) return TB_ERR_NULL;
+  if (!out->eigval || !out->info) return TB_ERR_NULL;
+  if (in->batch < 0 || m->n_modes < 1 || m->n_modes > p->n) return TB_ERR_SIZE;
+  if ((m->consistent != 0 && m->consistent != 1) || m->joint_mass_stride < 0) return TB_ERR_SIZE;
+  if (p->n > TB_SMALL_MAX_DOF) return TB_ERR_TOO_LARGE;
+  if (in->batch > 0) {
+    if (!in->joint_xyz) return TB_ERR_NULL;
+    if (!in->member_aed && !(in->gene && in->type_table && in->n_type > 0)) return TB_ERR_NULL;
+  }
+  if (p->device < 0 || !have_device()) return TB_ERR_NO_DEVICE;
+  return TB_OK;
+}
+
+// One k_modes launch over the batch (device pointers), with the plan lock held
+int run_modes(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out, cudaStream_t st) {
+  int threads = 0, smem = 0, per_sm = 0;
+  int rc = tb_modes_config(p->dim, p->n, &threads, &smem, &per_sm);
+  if (rc) return rc;
+  const int sms = p->num_sm > 0 ? p->num_sm : 148;
+  const int grid = (int)std::min<int64_t>(in->batch, (int64_t)sms * per_sm);
+  if (m->consistent) {                           // the consistent mass's slots: grow-only, stream-ordered, never in a capture
+    const size_t need = (size_t)grid * p->n * p->n * sizeof(double);
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
+    if (p->modes_bytes < need && cap != cudaStreamCaptureStatusNone) return TB_ERR_ALLOC;
+    rc = ws_acquire(p, st);
+    if (rc) return rc;
+    if (p->modes_bytes < need) {
+      if (p->modes_buf) TB_CUDA(cudaFreeAsync(p->modes_buf, st));
+      p->modes_buf = nullptr;
+      p->modes_bytes = 0;
+      TB_CUDA(cudaMallocAsync(&p->modes_buf, need, st));
+      p->modes_bytes = need;
+    }
+  }
+  ModesArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.nJ = p->nJ; a.M = p->M; a.N = p->N; a.n = p->n;
+  a.n_modes = m->n_modes; a.consistent = m->consistent; a.plan_stable = p->stable; a.n_type = in->n_type;
+  a.xyz = in->joint_xyz; a.xyz_stride = in->joint_stride;
+  a.aed = in->member_aed; a.aed_stride = in->member_stride;
+  a.gene = in->member_aed ? nullptr : in->gene; a.gene_stride = in->gene_stride;
+  a.type_table = in->type_table;
+  a.jmass = m->joint_mass; a.jmass_stride = m->joint_mass_stride;
+  a.conn = p->d_conn; a.free_ref = p->d_free_ref; a.dof2free = p->d_dof2free;
+  a.ent_row = p->d_ent_row; a.ent_col = p->d_ent_col; a.ent_ptr = p->d_ent_ptr; a.nnz = (int64_t)p->ent_row.size();
+  a.ctr_member = p->d_ctr_member; a.ctr_local = p->d_ctr_local;
+  a.inc_ptr = p->d_inc_ptr; a.inc_mem = p->d_inc_mem;
+  a.eigval = out->eigval; a.modes = out->modes; a.info = out->info;
+  a.slot = m->consistent ? (double*)p->modes_buf : nullptr;
+  rc = tb_launch_modes(a, p->dim, grid, threads, smem, st);
+  if (rc) return rc;
+  return m->consistent ? ws_release(p, st) : TB_OK;
+}
+
+}  // namespace
+
+extern "C" int tb_modes(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out, void* cuda_stream) {
+  int rc = check_modes(p, in, m, out);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  rc = check_device(p);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lock(p->mu);
+  return run_modes(p, in, m, out, (cudaStream_t)cuda_stream);
+}
+
+// Host buffers: staged through the plan's arena like the other *_host calls (plain cudaMemcpyAsync on the compute stream)
+extern "C" int tb_modes_host(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out) {
+  int rc = check_modes(p, in, m, out);
+  if (rc) return rc;
+  const int B = in->batch;
+  if (B == 0) return TB_OK;
+  const int64_t rowJ = (int64_t)p->nJ * p->dim, rowM3 = (int64_t)p->M * 3, rowM = p->M, nm = m->n_modes;
+  if (!stride_ok(in->joint_stride, rowJ)) return TB_ERR_SIZE;
+  if (in->member_aed && !stride_ok(in->member_stride, rowM3)) return TB_ERR_SIZE;
+  if (!in->member_aed && !stride_ok(in->gene_stride, rowM)) return TB_ERR_SIZE;
+  if (m->joint_mass && !stride_ok(m->joint_mass_stride, p->nJ)) return TB_ERR_SIZE;
+  rc = check_device(p);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> pipe_lock(g_pipe_mu);
+  std::lock_guard<std::mutex> plan_lock(p->mu);
+  HostPipe* hp = host_pipe();
+  if (!hp) return TB_ERR_ALLOC;
+  rc = async_drain(p);
+  if (rc) return rc;
+  auto cnt = [&](int64_t stride, int64_t row) { return (size_t)(stride == 0 ? row : row * B); };
+  const size_t nxyz = cnt(in->joint_stride, rowJ);
+  const size_t naed = in->member_aed ? cnt(in->member_stride, rowM3) : 0;
+  const size_t ngene = in->member_aed ? 0 : cnt(in->gene_stride, rowM);
+  const size_t ntab = in->member_aed ? 0 : (size_t)in->n_type * 3;
+  const size_t njm = m->joint_mass ? cnt(m->joint_mass_stride, p->nJ) : 0;
+  const size_t nval = (size_t)B * nm, nmode = out->modes ? (size_t)B * nm * p->N : 0;
+  size_t need = 0;
+  for (size_t bytes : {nxyz * 8, naed * 8, ngene * 4, ntab * 8, njm * 8, nval * 8, nmode * 8, (size_t)B * 4}) need += Arena::al(bytes);
+  cudaStream_t st = hp->comp;
+  auto body = [&]() -> int {
+    int r2 = arena_reserve(&p->stage_dev, &p->stage_dev_bytes, need + 4096);
+    if (r2) return r2;
+    char* cur = (char*)p->stage_dev;
+    double* dxyz = take<double>(cur, nxyz);
+    double* daed = take<double>(cur, naed);
+    int32_t* dgene = take<int32_t>(cur, ngene);
+    double* dtab = take<double>(cur, ntab);
+    double* djm = take<double>(cur, njm);
+    tb_modes_out dout = {take<double>(cur, nval), out->modes ? take<double>(cur, nmode) : nullptr, take<int32_t>(cur, (size_t)B)};
+    TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, nxyz * 8, cudaMemcpyHostToDevice, st));
+    tb_batch_in din = *in;
+    din.joint_xyz = dxyz;
+    din.force = nullptr;
+    if (in->member_aed) {
+      TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, naed * 8, cudaMemcpyHostToDevice, st));
+      din.member_aed = daed;
+      din.gene = nullptr;
+    } else {
+      TB_CUDA(cudaMemcpyAsync(dgene, in->gene, ngene * 4, cudaMemcpyHostToDevice, st));
+      TB_CUDA(cudaMemcpyAsync(dtab, in->type_table, ntab * 8, cudaMemcpyHostToDevice, st));
+      din.gene = dgene;
+      din.type_table = dtab;
+    }
+    tb_modes_in dm = *m;
+    if (m->joint_mass) {
+      TB_CUDA(cudaMemcpyAsync(djm, m->joint_mass, njm * 8, cudaMemcpyHostToDevice, st));
+      dm.joint_mass = djm;
+    }
+    r2 = run_modes(p, &din, &dm, &dout, st);
+    if (r2) return r2;
+    TB_CUDA(cudaMemcpyAsync(out->eigval, dout.eigval, nval * 8, cudaMemcpyDeviceToHost, st));
+    if (out->modes) TB_CUDA(cudaMemcpyAsync(out->modes, dout.modes, nmode * 8, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaStreamSynchronize(st));
+    return TB_OK;
+  };
+  rc = body();
+  if (rc) host_pipe_drain(hp);
+  return rc;
+}
+
 // pinned host buffers for callers that want full-speed H2D/D2H through the *_host entry points
 extern "C" int tb_pinned_alloc(void** ptr, size_t bytes) {
   if (!ptr) return TB_ERR_NULL;

@@ -175,6 +175,9 @@ struct tb_plan {
   // status [B], and the per-member vectors [B][M][d] when they do not fit shared memory
   void* adj_buf = nullptr;
   size_t adj_bytes = 0;
+  // tb_modes scratch of the consistent mass (grow-only, grown stream-ordered): one n x n slot per CTA of the launch
+  void* modes_buf = nullptr;
+  size_t modes_bytes = 0;
   // pipelined host calls (tb_solve_host_async): TB_ASYNC_SLOTS more staging arenas used in turn by consecutive calls,
   // the events that chain a call's copies and kernels, and the ticket counters (submitted / known to be complete)
   void* stage_async[TB_ASYNC_SLOTS] = {};
@@ -365,6 +368,26 @@ size_t tb_rag_env_slot_bytes(int dim, int max_joint, int max_member);
 // persistent grid (at most one CTA per truss), dynamic shared memory and its envelope budget of a launch
 int tb_rag_env_config(int dim, int max_joint, int max_member, int batch, int* grid, int* smem_bytes, int* env_smem);
 int tb_launch_rag_env(const RagEnvArgs& a, int grid, int smem_bytes, cudaStream_t st);
+
+// Modal analysis (tb_modes.cu): one CTA per system, the reduced matrix in shared memory
+struct ModesArgs {
+  int batch, nJ, M, N, n, n_modes, consistent, plan_stable, n_type;
+  const double* xyz; int64_t xyz_stride;
+  const double* aed; int64_t aed_stride;
+  const int32_t* gene; int64_t gene_stride;
+  const double* type_table;
+  const double* jmass; int64_t jmass_stride;     // [B][nJ] non-structural joint mass, or null
+  // plan maps (device): the scatter map's entries are in the internal order, free_ref / dof2free map them back
+  const int32_t* conn; const int32_t* free_ref; const int32_t* dof2free;
+  const int32_t* ent_row; const int32_t* ent_col; const int64_t* ent_ptr; int64_t nnz;
+  const int32_t* ctr_member; const int32_t* ctr_local;
+  const int32_t* inc_ptr; const int32_t* inc_mem;
+  double* eigval; double* modes; int32_t* info;  // outputs [B][n_modes], [B][n_modes][N] or null, [B]
+  double* slot;                                  // consistent mass: grid slots of n x n doubles, else null
+};
+// CTA size, dynamic shared memory and resident CTAs per SM of k_modes for n free DOFs (1 <= n <= TB_SMALL_MAX_DOF)
+int tb_modes_config(int dim, int n, int* threads, int* smem, int* per_sm);
+int tb_launch_modes(const ModesArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st);
 
 // fragment-major offset of element (r, c) inside one 64x64 tile:
 //   [k-half 2][row-block 8][k-slab 8][lane 32], lane = (r%8)*4 + c%4

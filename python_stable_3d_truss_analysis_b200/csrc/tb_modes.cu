@@ -1,0 +1,452 @@
+// Batched modal analysis (tb_modes, DESIGN.md section 11): the n_modes lowest eigenpairs of K_ff phi = lambda M_ff phi for
+// every system of a uniform batch, n <= TB_SMALL_MAX_DOF free DOFs.
+//
+// k_modes<DIM> runs one CTA per system in a persistent grid-stride loop, with the whole reduced matrix in dynamic shared
+// memory (n x P doubles, P = n | 1: an odd row pitch keeps row-strided and column-strided accesses free of bank
+// conflicts).  Per system:
+//   1. status guards of the static solve (counting rule, gene index, zero length), then K_ff assembled densely through the
+//      plan's scatter map (the same products and ascending-member sums as every other path: bit-identical to
+//      GetKMatrix()[mask][:, mask]) and the mass: lumped per free DOF in shared memory, consistent into the CTA's slot of
+//      the plan's modal scratch (global memory, L2-resident).
+//   2. standard problem: K~ = M^-1/2 K M^-1/2 (lumped) or K~ = L^-1 K L^-T with M = L L^T (consistent, both triangular
+//      solves column-parallel in shared memory).
+//   3. Householder tridiagonalisation, tred2 style, with Q accumulated in place.
+//   4. implicit QL with shifts, tql2 style: thread 0 runs a sweep's scalar recurrence and records its rotations, then every
+//      thread applies them to its own row of Z (three barriers per sweep).  tql2 keeps the vectors of a cluster of equal
+//      eigenvalues orthogonal with no extra work (bar-72 and bar-120 have exactly repeated frequencies).
+//   5. ascending ranks, back-transform of the requested vectors (M^-1/2 z or L^-T z), sign convention, outputs.
+// Every sum runs serially in one thread in a fixed order and no value depends on which thread computes it, so a system's
+// bits do not depend on its position in the batch, the batch size, the CTA size or the number of resident CTAs.
+#include <cfloat>
+
+#include "tb_common.cuh"
+
+namespace {
+
+constexpr int TQL_MAX_ITER = 30;   // QL sweeps per eigenvalue (EISPACK tql2's cap)
+
+struct ModesCtl {
+  double h;
+  int any, lo, status;
+};
+
+// (a, e, density) of member m from the explicit rows or the gene / type table; ok = false for a gene out of range
+__device__ __forceinline__ void member_props(const ModesArgs& a, const double* aed, const int32_t* gene, int m, double& ar,
+                                             double& e, double& rho, bool& ok) {
+  const double* t;
+  if (gene) {
+    const int g = gene[m];
+    ok = (unsigned)g < (unsigned)a.n_type;
+    t = a.type_table + 3 * (ok ? g : 0);
+  } else {
+    ok = true;
+    t = aed + 3 * m;
+  }
+  ar = t[0];
+  e = t[1];
+  rho = t[2];
+}
+
+// EA/L, direction cosines and weight term (a L) density of member m, the reference's roundings (tb_member_geom)
+template <int DIM>
+__device__ __forceinline__ double member_kcw(const ModesArgs& a, const double* xyz, const double* aed, const int32_t* gene,
+                                             int m, double& k, double c[DIM], double& w) {
+  double ar, e, rho, dx[DIM];
+  bool ok;
+  member_props(a, aed, gene, m, ar, e, rho, ok);
+  return tb_member_geom<DIM>(xyz, a.conn[2 * m], a.conn[2 * m + 1], ar, e, rho, dx, c, k, w);
+}
+
+__host__ __device__ inline size_t modes_smem_bytes(int n) {
+  const int P = n | 1;
+  return ((size_t)n * P + 8 * (size_t)n) * sizeof(double) + 2 * (size_t)n * sizeof(int);
+}
+
+template <int DIM>
+__global__ void __launch_bounds__(160) k_modes(const ModesArgs a) {
+  extern __shared__ __align__(16) double smem[];
+  __shared__ ModesCtl ctl;
+  const int n = a.n, P = n | 1, N = a.N, nm = a.n_modes;
+  const int tid = threadIdx.x, nth = blockDim.x, lane = tid & 31, wid = tid >> 5, nw = nth >> 5;
+  double* Z = smem;            // [n][P] K_ff -> K~ -> Householder data -> Q -> eigenvectors of K~ (columns)
+  double* dv = Z + (size_t)n * P;   // diagonal, then eigenvalues
+  double* ev = dv + n;         // sub-diagonal
+  double* pv = ev + n;         // tred2 scratch p = A u / H
+  double* qv = pv + n;         // tred2 scratch q = p - K u
+  double* sc = qv + n;         // lumped: M^-1/2 per free DOF
+  double* rc = sc + n;         // rotations of one QL sweep
+  double* rs = rc + n;
+  double* sg = rs + n;         // sign of each requested mode
+  int* i2r = (int*)(sg + n);   // internal row of the plan's scatter map -> free DOF in the reference's order
+  int* perm = i2r + n;         // ascending rank -> column of Z
+  for (int r = tid; r < n; r += nth) i2r[a.dof2free[a.free_ref[r]]] = r;
+  double* L = a.slot ? a.slot + (size_t)blockIdx.x * n * n : nullptr;   // consistent mass: M_ff, then its Cholesky factor
+
+  for (int b = blockIdx.x; b < a.batch; b += gridDim.x) {
+    const double* xyz = a.xyz + b * a.xyz_stride;
+    const double* aed = a.aed ? a.aed + b * a.aed_stride : nullptr;
+    const int32_t* gene = a.aed ? nullptr : a.gene + b * a.gene_stride;
+    const double* jm = a.jmass ? a.jmass + b * a.jmass_stride : nullptr;
+    __syncthreads();                           // the previous system's shared data is consumed (and i2r is complete)
+
+    // ---- status guards of the static solve, in its order of precedence
+    int bad = 0;
+    for (int m = tid; m < a.M; m += nth) {
+      double ar, e, rho;
+      bool ok;
+      member_props(a, aed, gene, m, ar, e, rho, ok);
+      if (!ok) {
+        bad |= 1;
+      } else {
+        double k, c[DIM], w;
+        if (!(member_kcw<DIM>(a, xyz, aed, gene, m, k, c, w) > 0.0)) bad |= 2;
+      }
+    }
+    const int anyidx = __syncthreads_or(bad & 1), anylen = __syncthreads_or(bad & 2);
+    int status = a.plan_stable ? 0 : TB_INFO_NOT_STABLE;
+    if (anyidx) status = min(status, TB_INFO_BAD_INDEX);
+    else if (anylen) status = min(status, TB_INFO_ZERO_LENGTH);
+
+    if (status == 0) {
+      // ---- K_ff (and consistent M_ff) densely, both triangles
+      for (int i = tid; i < n * P; i += nth) Z[i] = 0.0;
+      if (a.consistent)
+        for (int i = tid; i < n * n; i += nth) L[i] = 0.0;
+      __syncthreads();
+      for (int64_t e = tid; e < a.nnz; e += nth) {
+        const int r = i2r[a.ent_row[e]], c = i2r[a.ent_col[e]];
+        double kv = 0.0, mv = 0.0;
+        for (int64_t q = a.ent_ptr[e]; q < a.ent_ptr[e + 1]; ++q) {
+          const int m = a.ctr_member[q], loc = a.ctr_local[q];
+          const int la = loc / (2 * DIM), lb = loc - la * (2 * DIM);
+          const int A = la / DIM, i = la - A * DIM, B = lb / DIM, j = lb - B * DIM;
+          double k, cs[DIM], w;
+          member_kcw<DIM>(a, xyz, aed, gene, m, k, cs, w);
+          double pr = __dmul_rn(cs[i], cs[j]);   // truss.py:69,80
+          if (A != B) pr = -pr;
+          kv = __dadd_rn(kv, __dmul_rn(k, pr));  // truss.py:70,314
+          if (a.consistent && i == j) {          // (m_e / 6) [[2, 1], [1, 2]] per axis
+            const double me6 = __ddiv_rn(w, 6.0);
+            mv = __dadd_rn(mv, A == B ? __dmul_rn(2.0, me6) : me6);
+          }
+        }
+        Z[r * P + c] = kv;
+        Z[c * P + r] = kv;
+        if (a.consistent) {
+          L[r * n + c] = mv;
+          L[c * n + r] = mv;
+        }
+      }
+      int badm = 0;
+      if (!a.consistent) {                     // lumped: m_e / 2 per end joint and axis, ascending member, + joint mass
+        for (int r = tid; r < n; r += nth) {
+          const int J = a.free_ref[r] / DIM;
+          double ms = 0.0;
+          for (int q = a.inc_ptr[J]; q < a.inc_ptr[J + 1]; ++q) {
+            double k, cs[DIM], w;
+            member_kcw<DIM>(a, xyz, aed, gene, a.inc_mem[q] >> 1, k, cs, w);
+            ms = __dadd_rn(ms, __dmul_rn(w, 0.5));
+          }
+          if (jm) ms = __dadd_rn(ms, jm[J]);
+          if (!(ms > 0.0)) badm = 1;
+          sc[r] = ms > 0.0 ? 1.0 / sqrt(ms) : 0.0;
+        }
+      }
+      __syncthreads();
+      if (a.consistent && jm)
+        for (int r = tid; r < n; r += nth) L[r * n + r] = __dadd_rn(L[r * n + r], jm[a.free_ref[r] / DIM]);
+      if (__syncthreads_or(badm)) status = TB_INFO_MASS;
+    }
+
+    // ---- standard problem
+    if (status == 0 && !a.consistent) {
+      for (int r = wid; r < n; r += nw)
+        for (int c = lane; c <= r; c += 32) Z[r * P + c] = (Z[r * P + c] * sc[r]) * sc[c];
+    } else if (status == 0) {
+      // Cholesky M = L L^T in the slot, left-looking: pivot by thread 0, then the column below it in parallel
+      for (int j = 0; j < n; ++j) {
+        double* Lj = L + (size_t)j * n;
+        if (tid == 0) {
+          double x = Lj[j];
+          for (int k = 0; k < j; ++k) x -= Lj[k] * Lj[k];
+          ctl.status = x > 0.0 ? 0 : TB_INFO_MASS;
+          Lj[j] = x > 0.0 ? sqrt(x) : 0.0;
+        }
+        __syncthreads();
+        if (ctl.status) break;
+        const double djj = Lj[j];
+        for (int i = j + 1 + tid; i < n; i += nth) {
+          double* Li = L + (size_t)i * n;
+          double x = Li[j];
+          for (int k = 0; k < j; ++k) x -= Li[k] * Lj[k];
+          Li[j] = x / djj;
+        }
+        __syncthreads();
+      }
+      status = ctl.status;
+      __syncthreads();
+      if (status == 0) {
+        // K~ = L^-1 (L^-1 K)^T: two column-parallel forward substitutions around an in-place transpose
+        for (int pass = 0; pass < 2; ++pass) {
+          for (int j = tid; j < n; j += nth)
+            for (int i = 0; i < n; ++i) {
+              const double* Li = L + (size_t)i * n;
+              double x = Z[i * P + j];
+              for (int k = 0; k < i; ++k) x -= Li[k] * Z[k * P + j];
+              Z[i * P + j] = x / Li[i];
+            }
+          __syncthreads();
+          if (pass == 0) {
+            for (int r = wid; r < n; r += nw)
+              for (int c = lane; c < r; c += 32) {
+                const double t = Z[r * P + c];
+                Z[r * P + c] = Z[c * P + r];
+                Z[c * P + r] = t;
+              }
+            __syncthreads();
+          }
+        }
+      }
+    }
+
+    if (status == 0) {
+      // ---- Householder tridiagonalisation (tred2), lower triangle of Z
+      for (int i = n - 1; i > 0; --i) {
+        const int l = i - 1;
+        double* zi = Z + (size_t)i * P;
+        __syncthreads();
+        if (tid == 0) {
+          double h = 0.0, scale = 0.0;
+          int any = 0;
+          if (l > 0) {
+            for (int k = 0; k < i; ++k) scale += fabs(zi[k]);
+            if (scale == 0.0) {
+              ev[i] = zi[l];
+            } else {
+              for (int k = 0; k < i; ++k) {
+                zi[k] /= scale;
+                h += zi[k] * zi[k];
+              }
+              const double f = zi[l];
+              const double g = f >= 0.0 ? -sqrt(h) : sqrt(h);
+              ev[i] = scale * g;
+              h -= f * g;
+              zi[l] = f - g;
+              any = 1;
+            }
+          } else {
+            ev[i] = zi[l];
+          }
+          dv[i] = h;
+          ctl.h = h;
+          ctl.any = any;
+        }
+        __syncthreads();
+        if (!ctl.any) continue;
+        const double h = ctl.h;
+        for (int j = tid; j < i; j += nth) {   // p = A u / H, u / H stored in column i
+          const double* zj = Z + (size_t)j * P;
+          Z[j * P + i] = zi[j] / h;
+          double g = 0.0;
+          for (int k = 0; k <= j; ++k) g += zj[k] * zi[k];
+          for (int k = j + 1; k < i; ++k) g += Z[k * P + j] * zi[k];
+          pv[j] = g / h;
+        }
+        __syncthreads();
+        double f = 0.0;                        // (every thread, same order)
+        for (int j = 0; j < i; ++j) f += pv[j] * zi[j];
+        const double hh = f / (h + h);
+        for (int j = tid; j < i; j += nth) qv[j] = pv[j] - hh * zi[j];
+        __syncthreads();
+        for (int j = wid; j < i; j += nw) {    // rank-2 update A -= u q^T + q u^T, a warp per row
+          const double fj = zi[j], gj = qv[j];
+          double* zj = Z + (size_t)j * P;
+          for (int k = lane; k <= j; k += 32) zj[k] -= (fj * qv[k] + gj * zi[k]);
+        }
+      }
+      __syncthreads();
+      if (tid == 0) {
+        dv[0] = 0.0;
+        ev[0] = 0.0;
+      }
+      for (int i = 0; i < n; ++i) {           // accumulate Q in place, a thread per column
+        __syncthreads();
+        const bool acc = dv[i] != 0.0;
+        if (acc)
+          for (int j = tid; j < i; j += nth) {
+            double g = 0.0;
+            for (int k = 0; k < i; ++k) g += Z[i * P + k] * Z[k * P + j];
+            for (int k = 0; k < i; ++k) Z[k * P + j] -= g * Z[k * P + i];
+          }
+        __syncthreads();
+        if (tid == 0) {
+          dv[i] = Z[i * P + i];
+          Z[i * P + i] = 1.0;
+        }
+        for (int j = tid; j < i; j += nth) Z[j * P + i] = Z[i * P + j] = 0.0;
+      }
+      __syncthreads();
+
+      // ---- implicit QL with shifts (tql2)
+      if (tid == 0) {
+        for (int i = 1; i < n; ++i) ev[i - 1] = ev[i];
+        ev[n - 1] = 0.0;
+      }
+      int fail = 0;
+      for (int l = 0; l < n && !fail; ++l) {
+        int iter = 0;
+        for (;;) {
+          __syncthreads();
+          int m;
+          for (m = l; m < n - 1; ++m) {
+            const double dd = fabs(dv[m]) + fabs(dv[m + 1]);
+            if (fabs(ev[m]) <= DBL_EPSILON * dd) break;
+          }
+          if (m == l) break;
+          if (iter++ == TQL_MAX_ITER) {
+            fail = 1;
+            break;
+          }
+          __syncthreads();                     // every thread has read d and e
+          if (tid == 0) {
+            double g = (dv[l + 1] - dv[l]) / (2.0 * ev[l]);
+            double r = hypot(g, 1.0);
+            g = dv[m] - dv[l] + ev[l] / (g + copysign(r, g));
+            double s = 1.0, c = 1.0, p = 0.0;
+            int i;
+            bool brk = false;
+            for (i = m - 1; i >= l; --i) {
+              const double f = s * ev[i], bb = c * ev[i];
+              r = hypot(f, g);
+              ev[i + 1] = r;
+              if (r == 0.0) {
+                dv[i + 1] -= p;
+                ev[m] = 0.0;
+                brk = true;
+                break;
+              }
+              s = f / r;
+              c = g / r;
+              g = dv[i + 1] - p;
+              r = (dv[i] - g) * s + 2.0 * c * bb;
+              p = s * r;
+              dv[i + 1] = g + p;
+              g = c * r - bb;
+              rc[i] = c;
+              rs[i] = s;
+            }
+            ctl.lo = brk ? i + 1 : l;
+            if (!brk) {
+              dv[l] -= p;
+              ev[l] = g;
+              ev[m] = 0.0;
+            }
+          }
+          __syncthreads();
+          if (tid < n) {                       // thread k applies the sweep's rotations to row k of Z
+            double* zk = Z + (size_t)tid * P;
+            for (int i = m - 1; i >= ctl.lo; --i) {
+              const double c = rc[i], s = rs[i], f = zk[i + 1];
+              zk[i + 1] = s * zk[i] + c * f;
+              zk[i] = c * zk[i] - s * f;
+            }
+          }
+        }
+      }
+      if (fail) status = TB_INFO_NO_CONVERGENCE;
+      __syncthreads();
+    }
+
+    if (status == 0) {
+      // ---- ascending order (ties: lower column first), back-transform, sign convention
+      for (int i = tid; i < n; i += nth) {
+        const double di = dv[i];
+        int rank = 0;
+        for (int j = 0; j < n; ++j) rank += (dv[j] < di || (dv[j] == di && j < i)) ? 1 : 0;
+        perm[rank] = i;
+      }
+      __syncthreads();
+      for (int q = tid; q < nm; q += nth) {
+        const int col = perm[q];
+        if (!a.consistent) {
+          for (int r = 0; r < n; ++r) Z[r * P + col] *= sc[r];
+        } else {
+          for (int r = n - 1; r >= 0; --r) {  // L^T y = z
+            double x = Z[r * P + col];
+            for (int k = r + 1; k < n; ++k) x -= L[(size_t)k * n + r] * Z[k * P + col];
+            Z[r * P + col] = x / L[(size_t)r * n + r];
+          }
+        }
+        double best = 0.0;
+        int bi = 0;
+        for (int r = 0; r < n; ++r) {
+          const double v = fabs(Z[r * P + col]);
+          if (v > best) {
+            best = v;
+            bi = r;
+          }
+        }
+        sg[q] = Z[bi * P + col] < 0.0 ? -1.0 : 1.0;
+        a.eigval[(int64_t)b * nm + q] = dv[col];
+      }
+      __syncthreads();
+      if (a.modes) {
+        double* mo = a.modes + (int64_t)b * nm * N;
+        for (int64_t i = tid; i < (int64_t)nm * N; i += nth) mo[i] = 0.0;
+        __syncthreads();
+        for (int idx = tid; idx < nm * n; idx += nth) {
+          const int q = idx / n, r = idx - q * n;
+          mo[(int64_t)q * N + a.free_ref[r]] = sg[q] * Z[r * P + perm[q]];
+        }
+      }
+    } else {                                   // failed system: zero outputs, never NaN
+      for (int q = tid; q < nm; q += nth) a.eigval[(int64_t)b * nm + q] = 0.0;
+      if (a.modes) {
+        double* mo = a.modes + (int64_t)b * nm * N;
+        for (int64_t i = tid; i < (int64_t)nm * N; i += nth) mo[i] = 0.0;
+      }
+    }
+    if (tid == 0) a.info[b] = status;
+  }
+}
+
+template <int DIM>
+int modes_config(int n, int* threads, int* smem, int* per_sm) {
+  // CTA size and residency depend on n only: cached per device and n (the occupancy query costs more than the launch)
+  static int cache[64][TB_SMALL_MAX_DOF + 1];
+  static int attr[64];   // the kernel's dynamic shared-memory limit set so far (only ever raised)
+  static std::mutex mu;
+  int dev = 0;
+  TB_CUDA(cudaGetDevice(&dev));
+  *threads = ((n < 32 ? 32 : n) + 31) / 32 * 32;
+  *smem = (int)modes_smem_bytes(n);
+  std::lock_guard<std::mutex> lock(mu);
+  int& c = cache[dev & 63][n];
+  if (c == 0) {
+    if (*smem > attr[dev & 63]) {   // (the exact size: the opt-in limit also counts the kernel's static shared memory)
+      TB_CUDA(cudaFuncSetAttribute(k_modes<DIM>, cudaFuncAttributeMaxDynamicSharedMemorySize, *smem));
+      attr[dev & 63] = *smem;
+    }
+    int q = 0;
+    TB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&q, k_modes<DIM>, *threads, (size_t)*smem));
+    if (q < 1) return (int)cudaErrorInvalidConfiguration;
+    c = q;
+  }
+  *per_sm = c;
+  return 0;
+}
+
+}  // namespace
+
+int tb_modes_config(int dim, int n, int* threads, int* smem, int* per_sm) {
+  if (n < 1 || n > TB_SMALL_MAX_DOF) return (int)cudaErrorInvalidValue;
+  return dim == 3 ? modes_config<3>(n, threads, smem, per_sm) : modes_config<2>(n, threads, smem, per_sm);
+}
+
+int tb_launch_modes(const ModesArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st) {
+  if (a.batch <= 0) return 0;
+  if (dim == 3) k_modes<3><<<grid, threads, smem, st>>>(a);
+  else k_modes<2><<<grid, threads, smem, st>>>(a);
+  tb_count_launch();
+  return (int)cudaGetLastError();
+}

@@ -544,6 +544,7 @@ extern "C" void tb_plan_destroy(tb_plan* p) {
     cudaEventDestroy(p->ws_event);
   }
   cudaFree(p->adj_buf);
+  cudaFree(p->modes_buf);
   cudaFree(p->ws);
   cudaFree(p->stage_dev);
   for (int i = 0; i < TB_ASYNC_SLOTS; ++i) {

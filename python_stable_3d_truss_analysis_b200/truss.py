@@ -30,6 +30,25 @@ from .utils import (CheckDim, DimensionError, InvaildJointError, IsZero, IsZeroV
                     TrussNotSolvedError, TrussNotStableError, ZERO_EPS)
 
 INFO_NOT_STABLE, INFO_ZERO_LENGTH, INFO_BAD_SUPPORT, INFO_BAD_INDEX = -1, -2, -3, -4
+INFO_MASS, INFO_NO_CONVERGENCE = _lib.TB_INFO_MASS, _lib.TB_INFO_NO_CONVERGENCE   # tb_modes only
+
+
+class MassNotPositiveDefiniteError(ValueError):
+    """Modal analysis: the reduced mass matrix is not positive definite (a free DOF without mass)."""
+
+
+class ModesNotConvergedError(RuntimeError):
+    """Modal analysis: the tridiagonal QL iteration hit its cap."""
+
+
+def raise_for_modes_info(info: int):
+    """Map a per-system status code of tb_modes onto an exception (the static solve's codes as raise_for_info)."""
+    if info == INFO_MASS:
+        raise MassNotPositiveDefiniteError("Mass matrix is not positive definite: a free DOF has no positive mass "
+                                           "(give its members a density or its joint a joint mass)")
+    if info == INFO_NO_CONVERGENCE:
+        raise ModesNotConvergedError("The eigenvalue iteration did not converge")
+    raise_for_info(info)
 
 
 def raise_for_info(info: int):
@@ -149,9 +168,11 @@ class Truss:
         self._dense = None                      # dict(u, ext, axial) of dense float64 arrays
         self._displace = self._external = self._internal = None
         self._solved = False
+        self._modes = None                      # dict(eigval [k], modes [k, N]) of SolveModes()
 
     def _topology_changed(self):
         self._plan = None
+        self._modes = None
 
     def _pack(self):
         """Flat arrays in the layout of include/truss_b200.h."""
@@ -262,6 +283,7 @@ class Truss:
 
     def SetJointPosition(self, jointID, position):
         self._joints[jointID] = (position, self._joints[jointID][1])
+        self._modes = None
         for j0, j1, member in self._members.values():
             if j0 == jointID: member.SetPosition(0, position)
             if j1 == jointID: member.SetPosition(1, position)
@@ -280,6 +302,7 @@ class Truss:
 
     def SetMemberType(self, memberID, memberType):
         self._members[memberID][2].memberType = memberType
+        self._modes = None
 
     def SetMemberTypes(self, memberTypeDict, isCheckAllSet=False):
         if isCheckAllSet and self._members.keys() - memberTypeDict.keys():
@@ -408,6 +431,48 @@ class Truss:
         out = plan.solve_host(1, xyz, force, aed=aed, want=("u", "ext", "axial"))
         raise_for_info(int(out["info"][0]))
         self._set_dense_results(out["u"][0], out["ext"][0], out["axial"][0])
+
+    # ------------------------------------------------------------------ modal analysis
+    def SolveModes(self, nMode=None, isConsistentMass=False, jointMasses=None):
+        """Free vibration K_ff phi = lambda M_ff phi on the GPU (tb_modes, batch of one): the ``nMode`` lowest eigenpairs
+        (None = all).  Member mass is (a L) density in the caller's units (divide a weight density by g first); lumped
+        mass puts half of it on every axis of both end joints, ``isConsistentMass`` uses the consistent bar mass matrix.
+        ``jointMasses``: {jointID: mass} added on every axis of the joint.  A mechanism that passes the counting rule is
+        not an error: it shows as eigenvalues ~ 0."""
+        if not self.isStable:
+            raise TrussNotStableError("The truss is not stable !")
+        xyz, support, conn, aed, _ = self._pack()
+        plan = self._get_plan(support, conn)
+        jm = None
+        if jointMasses:
+            jm = np.zeros(self.nJoint)
+            for j, mass in jointMasses.items():
+                if j not in self._joints:
+                    raise InvaildJointError(f"No such joint [{j}], can't add a mass on it.")
+                jm[j] = float(mass)
+        out = plan.modes_host(1, xyz, aed=aed, n_modes=nMode, consistent=isConsistentMass, joint_mass=jm)
+        raise_for_modes_info(int(out["info"][0]))
+        self._modes = {"eigval": out["eigval"][0].copy(), "modes": out["modes"][0].copy()}
+
+    def _modes_or_raise(self):
+        if self._modes is None:
+            raise TrussNotSolvedError("Haven't done modal analysis yet (SolveModes).")
+        return self._modes
+
+    def GetEigenvalues(self):
+        """lambda = omega^2 of the solved modes, ascending (numpy array)."""
+        return self._modes_or_raise()["eigval"].copy()
+
+    def GetNaturalFrequencies(self):
+        """Natural frequencies omega / (2 pi) of the solved modes, ascending (numpy array)."""
+        return np.sqrt(np.maximum(self._modes_or_raise()["eigval"], 0.0)) / (2.0 * np.pi)
+
+    def GetModeShapes(self):
+        """One dict per mode, {jointID: displacement vector} over every joint (zero at supported DOFs), in the style of
+        GetDisplacements; M-normalised, the component of largest magnitude positive."""
+        modes = self._modes_or_raise()["modes"]
+        d = self._dim
+        return [{j: modes[k, j * d:(j + 1) * d].copy() for j in range(self.nJoint)} for k in range(modes.shape[0])]
 
     # ------------------------------------------------------------------ JSON
     def Serialize(self):
