@@ -273,6 +273,36 @@ typedef struct {
 int tb_modes(tb_plan* plan, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out, void* cuda_stream);
 int tb_modes_host(tb_plan* plan, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out);
 
+/* Reverse mode of tb_modes (DESIGN.md section 11): the gradients of L = sum_k g_eigval[k] lambda_k with respect to the
+ * joint positions, the member properties and the non-structural joint masses, from the forward's M-normalised modes:
+ *   dlambda/dp = phi^T (dK/dp - lambda dM/dp) phi           (simple eigenvalue, phi^T M_ff phi = 1)
+ * One pass over the members per system; nothing is solved.  `in` and `m` are the forward's arguments, of which only
+ * m->n_modes and m->consistent are read (the joint masses enter through the modes).  Explicit member properties only
+ * (member_aed; a gene / type-table batch returns TB_ERR_NULL: pass type_table[gene]).  Argument errors as tb_modes
+ * (TB_ERR_NULL / TB_ERR_SIZE, TB_ERR_TOO_LARGE for n > 160, TB_ERR_NO_DEVICE; B = 0 is a no-op).  phi is read at the
+ * free DOFs only (supported entries count as 0); a mode with g_eigval[k] == 0 is skipped.  A system whose forward info
+ * is not 0 gets zero gradients.  Gradients are written per system even for an input shared with stride 0 (reducing
+ * them is the caller's job).  Enqueues on the stream, never synchronises and uses no scratch (always capturable).
+ * Repeated eigenvalues: an eigenvalue of a cluster is not differentiable on its own.  A cotangent equal across the
+ * cluster (a loss symmetric in the cluster's eigenvalues, e.g. sum_k f(lambda_k)) gives the exact gradient whatever
+ * basis the forward chose; any other cotangent gives a basis-dependent directional value.  The same holds for a cluster
+ * cut by n_modes: ask for enough modes to keep it whole. */
+typedef struct {
+  const double* eigval;     /* [B][n_modes]     the forward's lambda -- required */
+  const double* modes;      /* [B][n_modes][N]  the forward's M-normalised modes -- required */
+  const int32_t* info;      /* [B]              the forward's status; info != 0: zero gradients -- required */
+  const double* g_eigval;   /* [B][n_modes]     cotangent -- required */
+} tb_modes_adj_in;
+
+typedef struct {
+  double* joint_xyz;        /* [B][nJ][d]  any may be NULL to skip it */
+  double* member_aed;       /* [B][M][3]   (a, e, density) */
+  double* joint_mass;       /* [B][nJ]     also when the forward had no joint_mass (the gradient at mu = 0) */
+} tb_modes_adj_out;
+
+int tb_modes_adjoint(tb_plan* plan, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_adj_in* a,
+                     const tb_modes_adj_out* out, void* cuda_stream);
+
 /* GA.GetFitness for B genes (ga.py:139-149); `full` may be NULL or receive the full results. */
 int tb_fitness(tb_plan* plan, const tb_batch_in* in, double allow_stress, double allow_displace,
                const tb_fit_out* fit, const tb_batch_out* full, void* cuda_stream);

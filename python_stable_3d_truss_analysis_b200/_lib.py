@@ -169,6 +169,14 @@ class TbModesOut(C.Structure):
     _fields_ = [("eigval", C.c_void_p), ("modes", C.c_void_p), ("info", C.c_void_p)]
 
 
+class TbModesAdjIn(C.Structure):
+    _fields_ = [("eigval", C.c_void_p), ("modes", C.c_void_p), ("info", C.c_void_p), ("g_eigval", C.c_void_p)]
+
+
+class TbModesAdjOut(C.Structure):
+    _fields_ = [("joint_xyz", C.c_void_p), ("member_aed", C.c_void_p), ("joint_mass", C.c_void_p)]
+
+
 class TbRaggedIn(C.Structure):
     _fields_ = [("dim", C.c_int32), ("batch", C.c_int32), ("joint_off", C.c_void_p), ("member_off", C.c_void_p),
                 ("joint_xyz", C.c_void_p), ("support", C.c_void_p), ("conn", C.c_void_p), ("member_aed", C.c_void_p),
@@ -176,7 +184,7 @@ class TbRaggedIn(C.Structure):
 
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
-           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
+           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_modes_adjoint", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
            "tb_solve_ragged_host", "tb_solve_ragged_env", "tb_ragged_env_order", "tb_ragged_limits", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
@@ -210,6 +218,8 @@ def lib():
     L.tb_adjoint.argtypes = [vp, C.POINTER(TbBatchIn), vp, C.POINTER(TbAdjIn), C.POINTER(TbAdjOut), i32, vp]
     L.tb_modes.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbModesIn), C.POINTER(TbModesOut), vp]
     L.tb_modes_host.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbModesIn), C.POINTER(TbModesOut)]
+    L.tb_modes_adjoint.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbModesIn), C.POINTER(TbModesAdjIn),
+                                   C.POINTER(TbModesAdjOut), vp]
     L.tb_fitness.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut), vp]
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
@@ -664,6 +674,32 @@ class Plan:
         st = torch.cuda.current_stream() if stream is None else stream
         mo = TbModesOut(_ptr(out["eigval"]), _ptr(out.get("modes")), _ptr(out["info"]))
         check(lib().tb_modes(self._h, C.byref(bi), C.byref(mi), C.byref(mo), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def modes_adjoint_device(self, B, xyz, aed, fwd, g_eigval, out, n_modes=None, consistent=False, stream=None):
+        """Reverse mode of ``modes_device`` (tb_modes_adjoint) on torch CUDA tensors: the gradients of
+        sum_k g_eigval[:, k] * lambda_k.  ``fwd`` is the dict ``modes_device`` returned for the same inputs (its "eigval",
+        "modes" and "info" are read); ``g_eigval`` is [B, n_modes]; ``out`` maps "joint_xyz" [B, nJ, d], "member_aed"
+        [B, M, 3] and "joint_mass" [B, nJ] to preallocated tensors (missing or None = skipped).  ``n_modes=None`` takes
+        the forward's count; ``consistent`` must be the forward's mass model.  Gradients are per system, also for shared
+        inputs.  With repeated eigenvalues only a cotangent equal across each cluster gives a basis-independent value."""
+        import torch
+
+        if aed is None:
+            raise ValueError("aed is required: there are no gradients with respect to a gene type table")
+        k = int(fwd["eigval"].shape[-1]) if n_modes is None else int(n_modes)
+        for name, t, shape in (("fwd['eigval']", fwd.get("eigval"), (B, k)), ("fwd['modes']", fwd.get("modes"), (B, k, self.N)),
+                               ("fwd['info']", fwd.get("info"), (B,)), ("g_eigval", g_eigval, (B, k))):
+            if t is None or tuple(t.shape) != shape or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous tensor of shape {list(shape)}")
+        keep = []
+        bi = self._batch_in(B, xyz, aed, None, None, np.zeros(self.N), keep)
+        bi.force, bi.force_stride = None, 0            # (not read)
+        mi = TbModesIn(k, 1 if consistent else 0, None, 0)
+        ai = TbModesAdjIn(_ptr(fwd["eigval"]), _ptr(fwd["modes"]), _ptr(fwd["info"]), _ptr(g_eigval))
+        ao = TbModesAdjOut(_ptr(out.get("joint_xyz")), _ptr(out.get("member_aed")), _ptr(out.get("joint_mass")))
+        st = torch.cuda.current_stream() if stream is None else stream
+        check(lib().tb_modes_adjoint(self._h, C.byref(bi), C.byref(mi), C.byref(ai), C.byref(ao), C.c_void_p(st.cuda_stream)))
         return out
 
     def fitness_device(self, B, xyz, force, gene, type_table, allow_stress, allow_displace, out, aed=None, stream=None):

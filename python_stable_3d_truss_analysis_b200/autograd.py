@@ -15,6 +15,14 @@ Example -- compliance gradient of bar-72 with respect to the member areas::
 
 ``solve_ragged(packed, xyz, aed, force)`` does the same for a ragged batch -- every truss with its own topology, packed
 back to back as ``gencube_device`` / ``augment_and_solve_device`` return them (``tb_adjoint_ragged``).
+
+``modes(truss, xyz, aed, joint_mass)`` runs the modal analysis (``tb_modes``, DESIGN.md section 11) and returns eigenvalues
+that backpropagate to the joint coordinates, the member properties and the joint masses (``tb_modes_adjoint``: one pass
+over the members, nothing solved).  Example -- a frequency penalty for sizing, symmetric in the eigenvalues::
+
+    out = autograd.modes(truss, aed=aed, n_modes=6)
+    penalty = torch.relu(lam_min - out["eigval"]).pow(2).sum()
+    penalty.backward()                                # aed.grad
 """
 from __future__ import annotations
 
@@ -23,7 +31,15 @@ import torch
 
 from . import _lib
 
-__all__ = ["solve", "solve_ragged"]
+__all__ = ["solve", "solve_ragged", "modes"]
+
+
+def per_input(g, x):
+    """The gradient of input ``x`` from per-system gradients ``g``: a shared (unbatched) input gets the sum over the
+    batch."""
+    if g is None:
+        return None
+    return g.reshape(x.shape) if x.dim() == g.dim() else g.sum(0)
 
 
 class _Solve(torch.autograd.Function):
@@ -52,12 +68,6 @@ class _Solve(torch.autograd.Function):
                "member_aed": torch.empty(B, plan.M, 3, **f64),
                "force": torch.empty(B, plan.N, **f64) if need_f else None}
         plan.adjoint_device(B, xyz, force, aed, u, grads, res, shared_factor=ctx.shared_factor)
-
-        def per_input(g, x):                      # a shared (unbatched) input gets the sum over the batch
-            if g is None:
-                return None
-            return g.reshape(x.shape) if x.dim() == g.dim() else g.sum(0)
-
         return (per_input(res["joint_xyz"], xyz), per_input(res["member_aed"], aed) if need_a else None,
                 per_input(res["force"], force), None, None, None)
 
@@ -198,3 +208,77 @@ def solve_ragged(packed, xyz=None, aed=None, force=None, max_joint=None, max_mem
         u, ext, axial, weight, info = _SolveRagged.apply(xyz, aed, force, base["joint_off"], base["member_off"], base["support"],
                                                          base["conn"], dim, max_joint, max_member)
     return {"u": u, "ext": ext, "axial": axial, "weight": weight, "info": info}
+
+
+class _Modes(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, xyz, aed, joint_mass, plan, B, n_modes, consistent):
+        out = {"modes": torch.empty(B, n_modes, plan.N, dtype=torch.float64, device=xyz.device)}   # (the backward needs them)
+        plan.modes_device(B, xyz, aed=aed, n_modes=n_modes, consistent=consistent, joint_mass=joint_mass, out=out)
+        ctx.save_for_backward(xyz, aed, joint_mass, out["eigval"], out["modes"], out["info"])
+        ctx.plan, ctx.B, ctx.n_modes, ctx.consistent = plan, B, n_modes, consistent
+        ctx.mark_non_differentiable(out["modes"], out["info"])
+        ctx.set_materialize_grads(False)
+        return out["eigval"], out["modes"], out["info"]
+
+    @staticmethod
+    def backward(ctx, g_eigval, _g_modes, _g_info):
+        if g_eigval is None:
+            return (None,) * 7
+        xyz, aed, joint_mass, eigval, modes_, info = ctx.saved_tensors
+        plan, B = ctx.plan, ctx.B
+        f64 = dict(dtype=torch.float64, device=xyz.device)
+        need_x, need_a, need_m = ctx.needs_input_grad[:3]
+        res = {"joint_xyz": torch.empty(B, plan.nJ, plan.dim, **f64) if need_x else None,
+               "member_aed": torch.empty(B, plan.M, 3, **f64) if need_a else None,
+               "joint_mass": torch.empty(B, plan.nJ, **f64) if need_m else None}
+        fwd = {"eigval": eigval, "modes": modes_, "info": info}
+        plan.modes_adjoint_device(B, xyz, aed, fwd, g_eigval.contiguous(), res, n_modes=ctx.n_modes, consistent=ctx.consistent)
+        return (per_input(res["joint_xyz"], xyz), per_input(res["member_aed"], aed),
+                per_input(res["joint_mass"], joint_mass) if need_m else None, None, None, None, None)
+
+
+def modes(truss, xyz=None, aed=None, joint_mass=None, n_modes=None, consistent=False):
+    """Modal analysis (``Truss.SolveModes``) for a uniform batch, with eigenvalues differentiable with respect to
+    ``xyz``, ``aed`` and ``joint_mass``.
+
+    Inputs are float64 CUDA tensors: ``xyz`` [nJ, d] joint positions, ``aed`` [M, 3] (a, e, density) per member and
+    ``joint_mass`` [nJ] non-structural mass per joint; each either unbatched (shared by every system) or with a leading
+    batch dimension B.  ``xyz`` / ``aed`` None mean the truss's own values, held constant; ``joint_mass`` None means no
+    non-structural mass.  ``n_modes`` (None = all n free DOFs) lowest modes; ``consistent`` selects the consistent mass
+    matrix instead of the lumped one.
+
+    Returns ``{"eigval": [B, k], "modes": [B, k, N], "info": [B] int32}`` (without the batch dimension when no input has
+    one): lambda = omega^2 ascending, M-normalised mode shapes (0 at supported DOFs) and the per-system status of
+    ``include/truss_b200.h``.  Only ``eigval`` is differentiable (dlambda/dp = phi^T (dK/dp - lambda dM/dp) phi); a
+    failed system has zero outputs and zero gradients.
+
+    Repeated eigenvalues (bar-72 and bar-120 have an exactly repeated lowest pair): a single eigenvalue of a cluster is
+    not differentiable, only functions symmetric in the cluster's eigenvalues are.  A loss that treats every mode alike
+    -- ``relu(lam_min - eigval).pow(2).sum()``, ``(1 / eigval).sum()`` -- sends equal cotangents to a cluster and gets
+    its exact gradient, whatever basis of the cluster the forward returned.  A loss that singles out one eigenvalue of a
+    cluster (``eigval[..., 0]`` on bar-72) gets a basis-dependent directional value; so does any loss when ``n_modes``
+    cuts a cluster in two.  Ask for enough modes to keep the clusters you use whole."""
+    pxyz, psup, pconn, paed, _ = truss._pack()
+    plan = truss._get_plan(psup, pconn)
+    given = [t for t in (xyz, aed, joint_mass) if isinstance(t, torch.Tensor)]
+    device = given[0].device if given else torch.device("cuda", torch.cuda.current_device())
+    xyz, bx = _input(xyz, pxyz, (plan.nJ, plan.dim), device, "xyz")
+    aed, ba = _input(aed, paed, (plan.M, 3), device, "aed")
+    bm = None
+    if joint_mass is not None:
+        joint_mass, bm = _input(joint_mass, None, (plan.nJ,), device, "joint_mass")
+    for name, t in (("xyz", xyz), ("aed", aed), ("joint_mass", joint_mass)):
+        if t is not None and t.device != device:
+            raise TypeError(f"{name} must be on the device of the other inputs ({device})")
+    sizes = {b for b in (bx, ba, bm) if b is not None}
+    if len(sizes) > 1:
+        raise ValueError(f"batched inputs disagree on the batch size: {sorted(sizes)}")
+    B = sizes.pop() if sizes else 1
+    k = plan.n if n_modes is None else int(n_modes)
+    with torch.cuda.device(device):
+        eigval, shapes, info = _Modes.apply(xyz, aed, joint_mass, plan, B, k, bool(consistent))
+    out = {"eigval": eigval, "modes": shapes, "info": info}
+    if bx is None and ba is None and bm is None:
+        out = {key: v[0] for key, v in out.items()}
+    return out

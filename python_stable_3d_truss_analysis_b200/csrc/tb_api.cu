@@ -1102,12 +1102,11 @@ extern "C" int tb_adjoint_ragged(const tb_ragged_in* in, const double* u, const 
 // ---- modal analysis (DESIGN.md section 11) ---------------------------------------------------------------------------
 namespace {
 
-// Argument checks of tb_modes / tb_modes_host: every argument error before the device checks
-int check_modes(const tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out) {
-  if (!p || !in || !m || !out) return TB_ERR_NULL;
-  if (!out->eigval || !out->info) return TB_ERR_NULL;
+// Argument checks shared by tb_modes, tb_modes_host and tb_modes_adjoint (p, in, m non-null): sizes, the free-DOF
+// limit, the inputs, then the device
+int check_modes_args(const tb_plan* p, const tb_batch_in* in, const tb_modes_in* m) {
   if (in->batch < 0 || m->n_modes < 1 || m->n_modes > p->n) return TB_ERR_SIZE;
-  if ((m->consistent != 0 && m->consistent != 1) || m->joint_mass_stride < 0) return TB_ERR_SIZE;
+  if (m->consistent != 0 && m->consistent != 1) return TB_ERR_SIZE;
   if (p->n > TB_SMALL_MAX_DOF) return TB_ERR_TOO_LARGE;
   if (in->batch > 0) {
     if (!in->joint_xyz) return TB_ERR_NULL;
@@ -1115,6 +1114,14 @@ int check_modes(const tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, c
   }
   if (p->device < 0 || !have_device()) return TB_ERR_NO_DEVICE;
   return TB_OK;
+}
+
+// Argument checks of tb_modes / tb_modes_host: every argument error before the device checks
+int check_modes(const tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out) {
+  if (!p || !in || !m || !out) return TB_ERR_NULL;
+  if (!out->eigval || !out->info) return TB_ERR_NULL;
+  if (m->joint_mass_stride < 0) return TB_ERR_SIZE;
+  return check_modes_args(p, in, m);
 }
 
 // One k_modes launch over the batch (device pointers), with the plan lock held
@@ -1169,6 +1176,28 @@ extern "C" int tb_modes(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m,
   if (rc) return rc;
   std::lock_guard<std::mutex> lock(p->mu);
   return run_modes(p, in, m, out, (cudaStream_t)cuda_stream);
+}
+
+// Reverse mode of tb_modes: one k_modes_sens launch, no scratch (so no plan lock and always capturable)
+extern "C" int tb_modes_adjoint(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_adj_in* g,
+                                const tb_modes_adj_out* out, void* cuda_stream) {
+  if (!p || !in || !m || !g || !out) return TB_ERR_NULL;
+  if (!g->eigval || !g->modes || !g->info || !g->g_eigval) return TB_ERR_NULL;
+  if (in->batch > 0 && !in->member_aed) return TB_ERR_NULL;      // (no gradients with respect to a type table)
+  int rc = check_modes_args(p, in, m);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  rc = check_device(p);
+  if (rc) return rc;
+  ModesSensArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.nJ = p->nJ; a.M = p->M; a.N = p->N; a.n_modes = m->n_modes; a.consistent = m->consistent;
+  a.xyz = in->joint_xyz; a.xyz_stride = in->joint_stride;
+  a.aed = in->member_aed; a.aed_stride = in->member_stride;
+  a.conn = p->d_conn; a.dof2free = p->d_dof2free; a.inc_ptr = p->d_inc_ptr; a.inc_mem = p->d_inc_mem;
+  a.eigval = g->eigval; a.modes = g->modes; a.info = g->info; a.g_eigval = g->g_eigval;
+  a.g_xyz = out->joint_xyz; a.g_aed = out->member_aed; a.g_jmass = out->joint_mass;
+  return tb_launch_modes_sens(a, p->dim, (cudaStream_t)cuda_stream);
 }
 
 // Host buffers: staged through the plan's arena like the other *_host calls (plain cudaMemcpyAsync on the compute stream)

@@ -389,6 +389,17 @@ struct ModesArgs {
 int tb_modes_config(int dim, int n, int* threads, int* smem, int* per_sm);
 int tb_launch_modes(const ModesArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st);
 
+// Reverse mode of the modal analysis (tb_modes_adjoint): one warp per system, no scratch
+struct ModesSensArgs {
+  int batch, nJ, M, N, n_modes, consistent;
+  const double* xyz; int64_t xyz_stride;
+  const double* aed; int64_t aed_stride;
+  const int32_t* conn; const int32_t* dof2free; const int32_t* inc_ptr; const int32_t* inc_mem;
+  const double* eigval; const double* modes; const int32_t* info; const double* g_eigval;   // [B][k], [B][k][N], [B], [B][k]
+  double* g_xyz; double* g_aed; double* g_jmass;                                            // outputs, null = skipped
+};
+int tb_launch_modes_sens(const ModesSensArgs& a, int dim, cudaStream_t st);
+
 // fragment-major offset of element (r, c) inside one 64x64 tile:
 //   [k-half 2][row-block 8][k-slab 8][lane 32], lane = (r%8)*4 + c%4
 // so that one DMMA m8n8k4 operand fragment (8 rows x 4 k) is 32 consecutive doubles and a

@@ -17,6 +17,8 @@
 //   5. ascending ranks, back-transform of the requested vectors (M^-1/2 z or L^-T z), sign convention, outputs.
 // Every sum runs serially in one thread in a fixed order and no value depends on which thread computes it, so a system's
 // bits do not depend on its position in the batch, the batch size, the CTA size or the number of resident CTAs.
+//
+// k_modes_sens<DIM> is the reverse mode (tb_modes_adjoint): eigenvalue gradients from the forward's modes, below.
 #include <cfloat>
 
 #include "tb_common.cuh"
@@ -436,6 +438,125 @@ int modes_config(int n, int* threads, int* smem, int* per_sm) {
   return 0;
 }
 
+// ---- reverse mode (tb_modes_adjoint): dlambda/dp = phi^T (dK/dp - lambda dM/dp) phi, summed with the cotangent
+// k_modes_sens<DIM> runs one warp per system (8 per CTA, persistent grid-stride loop).  Lanes first take members and
+// write the (a, e, density) row; then lanes take joints and gather the geometry vector of every incident member,
+// recomputed by the same member body (one more member evaluation per end instead of per-member scratch).  Per member
+// the modes are summed in ascending k, per joint the incidence list in ascending member*2+end order (gather_joint's
+// order), so a system's bits depend on nothing but its own inputs.  No atomics, no shared memory, any M.
+
+constexpr int SENS_WARPS = 8;
+
+// phi of joint J in one mode row, read at free DOFs only (supported entries count as 0)
+template <int DIM>
+__device__ __forceinline__ void mode_at(const ModesSensArgs& a, const double* phi, int J, double p[DIM]) {
+#pragma unroll
+  for (int i = 0; i < DIM; ++i) p[i] = a.dof2free[J * DIM + i] >= 0 ? phi[J * DIM + i] : 0.0;
+}
+
+// Member m of one system: ga = dL/d(a, e, density) and v = dL/d(x_j1) = -dL/d(x_j0), with t = c.dphi and w the mass
+// quadratic form per unit member mass (lumped (|phi0|^2 + |phi1|^2) / 2, consistent (|phi0|^2 + |phi1|^2 + phi0.phi1) / 3):
+//   dlambda/da = (e/L) t^2 - lambda L rho w,  dlambda/de = (a/L) t^2,  dlambda/drho = -lambda a L w,
+//   dlambda/dd = (k/L) (2 t dphi - 3 t^2 c) - lambda rho a w c
+template <int DIM>
+__device__ __forceinline__ void modes_sens_member(const ModesSensArgs& a, const double* xyz, const double* aed_m,
+                                                  const double* lam, const double* gl, const double* phi, int m,
+                                                  double ga[3], double v[DIM]) {
+  const int j0 = a.conn[2 * m], j1 = a.conn[2 * m + 1];
+  const double ar = aed_m[0], e = aed_m[1], rho = aed_m[2];
+  double dx[DIM], c[DIM], k, w;
+  const double len = tb_member_geom<DIM>(xyz, j0, j1, ar, e, rho, dx, c, k, w);
+  const double il = 1.0 / len, el = e * il, al = ar * il, kl = k * il, lr = len * rho, la = len * ar, ra = rho * ar;
+  ga[0] = ga[1] = ga[2] = 0.0;
+#pragma unroll
+  for (int i = 0; i < DIM; ++i) v[i] = 0.0;
+  for (int q = 0; q < a.n_modes; ++q) {
+    const double g = gl[q];
+    if (g == 0.0) continue;                    // (skipped, not multiplied by zero: a padded cotangent gives the same bits)
+    const double* ph = phi + (int64_t)q * a.N;
+    double p0[DIM], p1[DIM], dp[DIM], t = 0.0, s = 0.0, x = 0.0;
+    mode_at<DIM>(a, ph, j0, p0);
+    mode_at<DIM>(a, ph, j1, p1);
+#pragma unroll
+    for (int i = 0; i < DIM; ++i) {
+      dp[i] = p1[i] - p0[i];
+      t = fma(c[i], dp[i], t);
+      s = fma(p0[i], p0[i], fma(p1[i], p1[i], s));
+      x = fma(p0[i], p1[i], x);
+    }
+    const double wq = a.consistent ? (s + x) * (1.0 / 3.0) : 0.5 * s;
+    const double lq = lam[q], t2 = t * t, lw = lq * wq;
+    ga[0] += g * (el * t2 - lr * lw);
+    ga[1] += g * (al * t2);
+    ga[2] -= g * (la * lw);
+#pragma unroll
+    for (int i = 0; i < DIM; ++i) v[i] += g * (kl * (2.0 * t * dp[i] - 3.0 * t2 * c[i]) - ra * lw * c[i]);
+  }
+}
+
+template <int DIM>
+__global__ void __launch_bounds__(32 * SENS_WARPS) k_modes_sens(const ModesSensArgs a) {
+  const int lane = threadIdx.x & 31;
+  const int nm = a.n_modes;
+  for (int b = blockIdx.x * SENS_WARPS + (threadIdx.x >> 5); b < a.batch; b += gridDim.x * SENS_WARPS) {
+    double* gx = a.g_xyz ? a.g_xyz + (int64_t)b * a.N : nullptr;
+    double* ga = a.g_aed ? a.g_aed + (int64_t)b * a.M * 3 : nullptr;
+    double* gj = a.g_jmass ? a.g_jmass + (int64_t)b * a.nJ : nullptr;
+    if (a.info[b] != 0) {                      // failed system: zero gradients, never NaN
+      for (int i = lane; i < a.N; i += 32)
+        if (gx) gx[i] = 0.0;
+      for (int i = lane; i < 3 * a.M; i += 32)
+        if (ga) ga[i] = 0.0;
+      for (int i = lane; i < a.nJ; i += 32)
+        if (gj) gj[i] = 0.0;
+      continue;
+    }
+    const double* xyz = a.xyz + b * a.xyz_stride;
+    const double* aed = a.aed + b * a.aed_stride;
+    const double* lam = a.eigval + (int64_t)b * nm;
+    const double* gl = a.g_eigval + (int64_t)b * nm;
+    const double* phi = a.modes + (int64_t)b * nm * a.N;
+    if (ga)
+      for (int m = lane; m < a.M; m += 32) {
+        double r[3], v[DIM];
+        modes_sens_member<DIM>(a, xyz, aed + 3 * m, lam, gl, phi, m, r, v);
+        ga[3 * m] = r[0];
+        ga[3 * m + 1] = r[1];
+        ga[3 * m + 2] = r[2];
+      }
+    if (!gx && !gj) continue;
+    for (int J = lane; J < a.nJ; J += 32) {
+      if (gx) {
+        double s[DIM];
+#pragma unroll
+        for (int i = 0; i < DIM; ++i) s[i] = 0.0;
+        for (int p = a.inc_ptr[J]; p < a.inc_ptr[J + 1]; ++p) {   // (+) at the member's joint 1, (-) at its joint 0
+          const int me = a.inc_mem[p], m = me >> 1;
+          double r[3], v[DIM];
+          modes_sens_member<DIM>(a, xyz, aed + 3 * m, lam, gl, phi, m, r, v);
+#pragma unroll
+          for (int i = 0; i < DIM; ++i) s[i] += (me & 1) ? v[i] : -v[i];
+        }
+#pragma unroll
+        for (int i = 0; i < DIM; ++i) gx[J * DIM + i] = s[i];
+      }
+      if (gj) {                                // dlambda/dmu_J = -lambda |phi_J|^2
+        double s = 0.0;
+        for (int q = 0; q < nm; ++q) {
+          const double g = gl[q];
+          if (g == 0.0) continue;
+          double p[DIM], pp = 0.0;
+          mode_at<DIM>(a, phi + (int64_t)q * a.N, J, p);
+#pragma unroll
+          for (int i = 0; i < DIM; ++i) pp = fma(p[i], p[i], pp);
+          s += g * (lam[q] * pp);
+        }
+        gj[J] = -s;
+      }
+    }
+  }
+}
+
 }  // namespace
 
 int tb_modes_config(int dim, int n, int* threads, int* smem, int* per_sm) {
@@ -447,6 +568,34 @@ int tb_launch_modes(const ModesArgs& a, int dim, int grid, int threads, int smem
   if (a.batch <= 0) return 0;
   if (dim == 3) k_modes<3><<<grid, threads, smem, st>>>(a);
   else k_modes<2><<<grid, threads, smem, st>>>(a);
+  tb_count_launch();
+  return (int)cudaGetLastError();
+}
+
+int tb_launch_modes_sens(const ModesSensArgs& a, int dim, cudaStream_t st) {
+  if (a.batch <= 0) return 0;
+  // persistent grid: the resident CTAs of the device (the occupancy query costs more than the launch: cached per device)
+  static int cache[64][2];
+  static std::mutex mu;
+  int dev = 0;
+  TB_CUDA(cudaGetDevice(&dev));
+  int per_sm = 0, sms = 0;
+  {
+    std::lock_guard<std::mutex> lock(mu);
+    int& c = cache[dev & 63][dim == 3];
+    if (c == 0) {
+      int q = 0;
+      if (dim == 3) TB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&q, k_modes_sens<3>, 32 * SENS_WARPS, 0));
+      else TB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&q, k_modes_sens<2>, 32 * SENS_WARPS, 0));
+      if (q < 1) return (int)cudaErrorInvalidConfiguration;
+      c = q;
+    }
+    per_sm = c;
+  }
+  TB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const int grid = (int)std::min<int64_t>(((int64_t)a.batch + SENS_WARPS - 1) / SENS_WARPS, (int64_t)sms * per_sm);
+  if (dim == 3) k_modes_sens<3><<<grid, 32 * SENS_WARPS, 0, st>>>(a);
+  else k_modes_sens<2><<<grid, 32 * SENS_WARPS, 0, st>>>(a);
   tb_count_launch();
   return (int)cudaGetLastError();
 }
