@@ -406,6 +406,52 @@ int tb_ragged_env_order(const tb_ragged_in* in, int32_t* order, int64_t* envelop
 int tb_adjoint_ragged(const tb_ragged_in* in, const double* u, const tb_adj_in* grad, const tb_adj_out* out, double* work,
                       void* cuda_stream);
 
+/* ---- Modal analysis of a ragged batch (DESIGN.md section 11, "Ragged batches") -------------------------------------
+ * tb_modes for every truss of a ragged batch (tb_ragged_in, packed, local joint ids; in->force is ignored and may be
+ * NULL): per truss the same K_ff and M_ff as tb_modes on a plan of the same topology (ascending-member sums through the
+ * same member geometry, the same lumped and consistent rules), its free DOFs in ascending DOF order, and the same
+ * eigen-solve -- a truss gets the bits tb_modes gives a plan of its topology, wherever it sits in the batch.
+ * One CTA per truss; the launch is sized by a free-DOF bound (max_free, default min(d * max_joint, 160)).
+ * info per truss: the status tb_solve_ragged gives it for -1 ... -4 (counting rule, zero length, unknown support code,
+ * joint id out of range, nJ > max_joint or M > max_member), TB_INFO_BAD_INDEX also for more free DOFs than the bound,
+ * then TB_INFO_MASS / TB_INFO_NO_CONVERGENCE as tb_modes.  A mechanism that passes the counting rule is info 0 with
+ * eigenvalues ~ 0.  A failed truss gets zero outputs (its mode rows are written only when its offsets lie inside the
+ * packed arrays).  A truss with n_b < n_modes free DOFs is not an error: eigval[b][q] and mode row q are 0 for q >= n_b,
+ * and n_free[b] = n_b says how many are real (n_b = 0: info 0, all zeros).
+ * Errors: TB_ERR_NULL (in, m, out, out->eigval, out->info, the packed arrays but force when B > 0), TB_ERR_DIM,
+ * TB_ERR_SIZE (negative sizes, consistent not 0 / 1, max_free outside [0, 160], n_modes < 1 or, when B > 0, above the
+ * bound), TB_ERR_TOO_LARGE (d * max_joint > 1536 or max_member > 8192), then TB_ERR_NO_DEVICE; B = 0 is a no-op.
+ * Consistent mass uses one bound x bound slot per CTA in the device's envelope arena (tb_solve_ragged's scratch: same
+ * lock, event, stream-ordered growth; inside a stream capture a call that would grow it returns TB_ERR_ALLOC with nothing
+ * enqueued).  Lumped mass and the reverse mode use no scratch (always capturable). */
+typedef struct {
+  int32_t n_modes;          /* 1 <= n_modes <= the launch's free-DOF bound, else TB_ERR_SIZE */
+  int32_t consistent;       /* 0 lumped, 1 consistent (else TB_ERR_SIZE) */
+  const double* joint_mass; /* [sum nJ] non-structural mass per joint (packed), or NULL */
+  int32_t max_free;         /* upper bound on any truss's free DOFs, sizes the launch; 0 = min(d * max_joint, 160);
+                               > 160 or < 0: TB_ERR_SIZE */
+} tb_modes_ragged_in;
+
+typedef struct {
+  double* eigval;   /* [B][n_modes] ascending -- required */
+  double* modes;    /* [n_modes * d * joint_off[B]] packed, or NULL: truss b's block starts at n_modes*d*joint_off[b]
+                       and is [n_modes][d*nJ_b], M-normalised, 0 at supported DOFs, the sign convention of tb_modes */
+  int32_t* n_free;  /* [B] free DOFs of each truss (0 for a failed truss), or NULL */
+  int32_t* info;    /* [B] -- required */
+} tb_modes_ragged_out;
+
+int tb_modes_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_ragged_out* out, void* cuda_stream);
+/* Host pointers: the offsets are validated on the host (TB_ERR_SIZE / TB_ERR_TOO_LARGE as tb_solve_ragged_host). */
+int tb_modes_ragged_host(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_ragged_out* out);
+/* Reverse mode of tb_modes_ragged, the gradients of tb_modes_adjoint per truss.  `g` holds the forward's eigval, modes
+ * (required here), info and the cotangent [B][n_modes]; `out` joint_xyz [d sum nJ], member_aed [3 sum M], joint_mass
+ * [sum nJ] (any NULL to skip).  Reads m->n_modes, m->consistent and m->max_free (the forward's; the joint masses enter
+ * through the modes); argument errors as tb_modes_ragged.  Modes q >= n_b of a truss are padding and are skipped
+ * whatever their cotangent.  A failed truss gets zero gradients.  One warp per truss, no scratch; the repeated-eigenvalue
+ * caveat of tb_modes_adjoint applies. */
+int tb_modes_adjoint_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_adj_in* g,
+                            const tb_modes_adj_out* out, void* cuda_stream);
+
 /* ---- Dataset generation on the device (slientruss3d/generate.py:12-148; SURVEY.md section 8 f-2) ------------------
  * Expands a pool of trusses (a tb_ragged_in with DEVICE pointers) into n_out augmented trusses in the same packed layout,
  * ready for tb_solve_ragged: output truss o is pool truss src[o] after MoveToCentroid, RandomTranslation, AddJointNoise,

@@ -177,6 +177,14 @@ class TbModesAdjOut(C.Structure):
     _fields_ = [("joint_xyz", C.c_void_p), ("member_aed", C.c_void_p), ("joint_mass", C.c_void_p)]
 
 
+class TbModesRaggedIn(C.Structure):
+    _fields_ = [("n_modes", C.c_int32), ("consistent", C.c_int32), ("joint_mass", C.c_void_p), ("max_free", C.c_int32)]
+
+
+class TbModesRaggedOut(C.Structure):
+    _fields_ = [("eigval", C.c_void_p), ("modes", C.c_void_p), ("n_free", C.c_void_p), ("info", C.c_void_p)]
+
+
 class TbRaggedIn(C.Structure):
     _fields_ = [("dim", C.c_int32), ("batch", C.c_int32), ("joint_off", C.c_void_p), ("member_off", C.c_void_p),
                 ("joint_xyz", C.c_void_p), ("support", C.c_void_p), ("conn", C.c_void_p), ("member_aed", C.c_void_p),
@@ -184,7 +192,7 @@ class TbRaggedIn(C.Structure):
 
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
-           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_modes_adjoint", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
+           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_modes_adjoint", "tb_modes_ragged", "tb_modes_ragged_host", "tb_modes_adjoint_ragged", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
            "tb_solve_ragged_host", "tb_solve_ragged_env", "tb_ragged_env_order", "tb_ragged_limits", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
@@ -220,6 +228,10 @@ def lib():
     L.tb_modes_host.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbModesIn), C.POINTER(TbModesOut)]
     L.tb_modes_adjoint.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbModesIn), C.POINTER(TbModesAdjIn),
                                    C.POINTER(TbModesAdjOut), vp]
+    L.tb_modes_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbModesRaggedIn), C.POINTER(TbModesRaggedOut), vp]
+    L.tb_modes_ragged_host.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbModesRaggedIn), C.POINTER(TbModesRaggedOut)]
+    L.tb_modes_adjoint_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbModesRaggedIn), C.POINTER(TbModesAdjIn),
+                                          C.POINTER(TbModesAdjOut), vp]
     L.tb_fitness.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut), vp]
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
@@ -779,6 +791,117 @@ def _ragged_in(dim, packed, max_joint=None, max_member=None):
         max_member = mx[1] if max_member is None else max_member
     return TbRaggedIn(int(dim), B, _ptr(jo), _ptr(mo), _ptr(packed["xyz"]), _ptr(packed["support"]), _ptr(packed["conn"]),
                       _ptr(packed["aed"]), _ptr(packed["force"]), int(max_joint), int(max_member))
+
+
+def free_dofs_per_joint(dim, support):
+    """Free DOFs of each joint from its support code (tb_dof_free: a pin fixes every axis, a roller the axis it names; an
+    unknown code fixes none).  ``support`` is a numpy array or a torch tensor of uint8 codes; returns the same kind."""
+    table = np.array([dim, 0, dim - 1, dim - 1, dim - 1 if dim == 3 else dim] + [dim] * 251, np.int64)
+    if isinstance(support, np.ndarray):
+        return table[support.astype(np.int64)]
+    import torch
+    return torch.as_tensor(table, device=support.device)[support.long()]
+
+
+def _modes_ragged_sizes(dim, packed, n_modes, max_joint, max_member, max_free):
+    """(max_joint, max_member, max_free) of a packed batch of CUDA tensors, the missing ones in one device-to-host read.
+    The default free-DOF bound is the largest truss's free-DOF count (at least n_modes, at most 160: a larger truss gets
+    TB_INFO_BAD_INDEX)."""
+    import torch
+
+    jo, mo = packed["joint_off"], packed["member_off"]
+    B = int(jo.shape[0]) - 1
+    if B > 0 and (max_joint is None or max_member is None or max_free is None):
+        f = free_dofs_per_joint(dim, packed["support"])
+        cs = torch.cat([torch.zeros(1, dtype=torch.int64, device=f.device), torch.cumsum(f, 0)])
+        mx = torch.stack([(jo[1:] - jo[:-1]).max(), (mo[1:] - mo[:-1]).max(), (cs[jo[1:]] - cs[jo[:-1]]).max()]).tolist()
+    else:
+        mx = [0, 0, 0]
+    max_joint = mx[0] if max_joint is None else max_joint
+    max_member = mx[1] if max_member is None else max_member
+    if max_free is None:
+        max_free = min(max(mx[2], int(n_modes)), 160) if B > 0 else 0
+    return int(max_joint), int(max_member), int(max_free)
+
+
+def modes_ragged_device(dim, packed, n_modes, consistent=False, joint_mass=None, out=None, stream=None, max_joint=None,
+                        max_member=None, max_free=None):
+    """tb_modes_ragged on torch CUDA tensors: the ``n_modes`` lowest eigenpairs of every truss of a packed ragged batch
+    (``packed`` as for ``solve_ragged_device``; ``force`` is not read).  ``joint_mass`` [sum nJ] or None.  ``out`` may
+    hold preallocated "eigval" [B, n_modes], "modes" [n_modes d sum nJ] (skipped when present as None), "n_free" [B] and
+    "info" [B]; missing ones are allocated.  ``max_free`` (None: the largest truss's free-DOF count, at least n_modes)
+    sizes the launch.  Returns ``out``."""
+    import torch
+
+    mj, mm, mf = _modes_ragged_sizes(dim, packed, n_modes, max_joint, max_member, max_free)
+    ri = TbRaggedIn(int(dim), int(packed["joint_off"].shape[0]) - 1, _ptr(packed["joint_off"]), _ptr(packed["member_off"]),
+                    _ptr(packed["xyz"]), _ptr(packed["support"]), _ptr(packed["conn"]), _ptr(packed["aed"]), None, mj, mm)
+    dev, B, SJ = packed["xyz"].device, ri.batch, int(packed["support"].numel())
+    out = {} if out is None else out
+    for k, shape, dt in (("eigval", (B, int(n_modes)), torch.float64), ("modes", (int(n_modes) * dim * SJ,), torch.float64),
+                         ("n_free", (B,), torch.int32), ("info", (B,), torch.int32)):
+        if k not in out:
+            out[k] = torch.empty(shape, dtype=dt, device=dev)
+    mi = TbModesRaggedIn(int(n_modes), 1 if consistent else 0, _ptr(joint_mass), mf)
+    mo = TbModesRaggedOut(_ptr(out["eigval"]), _ptr(out.get("modes")), _ptr(out.get("n_free")), _ptr(out["info"]))
+    st = torch.cuda.current_stream() if stream is None else stream
+    check(lib().tb_modes_ragged(C.byref(ri), C.byref(mi), C.byref(mo), C.c_void_p(st.cuda_stream)))
+    return out
+
+
+def modes_ragged_host(dim, joint_off, member_off, xyz, support, conn, aed, n_modes, consistent=False, joint_mass=None,
+                      want_modes=True, max_free=None):
+    """tb_modes_ragged_host on numpy arrays (the packed layout of ``solve_ragged_host``).  Returns dict(eigval [B,
+    n_modes], modes [n_modes d sum nJ] (with ``want_modes``), n_free [B], info [B]).  ``max_free`` None: the largest
+    truss's free-DOF count (at least n_modes, at most 160)."""
+    joint_off, member_off = _np(joint_off, np.int64), _np(member_off, np.int64)
+    B = joint_off.shape[0] - 1
+    xyz, support, conn, aed = _np(xyz, np.float64), _np(support, np.uint8), _np(conn, np.int32), _np(aed, np.float64)
+    jm = None if joint_mass is None else _np(joint_mass, np.float64)
+    if jm is not None and jm.size != support.size:
+        raise ValueError(f"joint_mass must have {support.size} elements (one per joint), not {jm.size}")
+    SJ = int(joint_off[-1]) if B else 0
+    if max_free is None:
+        nf = 0
+        if B:
+            cs = np.concatenate([[0], np.cumsum(free_dofs_per_joint(dim, support))])
+            nf = int((cs[joint_off[1:]] - cs[joint_off[:-1]]).max())
+        max_free = min(max(nf, int(n_modes)), 160) if B else 0
+    ri = TbRaggedIn(int(dim), int(B), joint_off.ctypes.data, member_off.ctypes.data, xyz.ctypes.data, support.ctypes.data,
+                    conn.ctypes.data, aed.ctypes.data, None, int(np.diff(joint_off).max()) if B else 0,
+                    int(np.diff(member_off).max()) if B else 0)
+    out = {"eigval": np.empty((B, int(n_modes)), np.float64), "n_free": np.empty(B, np.int32), "info": np.empty(B, np.int32)}
+    if want_modes:
+        out["modes"] = np.empty(int(n_modes) * dim * SJ, np.float64)
+    mi = TbModesRaggedIn(int(n_modes), 1 if consistent else 0, _ptr(jm), int(max_free))
+    mo = TbModesRaggedOut(_ptr(out["eigval"]), _ptr(out.get("modes")), _ptr(out["n_free"]), _ptr(out["info"]))
+    check(lib().tb_modes_ragged_host(C.byref(ri), C.byref(mi), C.byref(mo)))
+    return out
+
+
+def modes_adjoint_ragged_device(dim, packed, fwd, g_eigval, out, consistent=False, stream=None, max_joint=None,
+                                max_member=None, max_free=None):
+    """Reverse mode of ``modes_ragged_device`` (tb_modes_adjoint_ragged) on torch CUDA tensors: the gradients of
+    sum_b,k g_eigval[b, k] lambda_bk.  ``fwd`` is the dict the forward returned (its "eigval", "modes" and "info" are
+    read); ``out`` maps "joint_xyz" [d sum nJ], "member_aed" [3 sum M] and "joint_mass" [sum nJ] to preallocated tensors
+    (missing or None = skipped).  ``consistent`` must be the forward's mass model."""
+    import torch
+
+    B, k = int(packed["joint_off"].shape[0]) - 1, int(fwd["eigval"].shape[-1])
+    SJ = int(packed["support"].numel())
+    for name, t, shape in (("fwd['eigval']", fwd.get("eigval"), (B, k)), ("fwd['modes']", fwd.get("modes"), (k * dim * SJ,)),
+                           ("fwd['info']", fwd.get("info"), (B,)), ("g_eigval", g_eigval, (B, k))):
+        if t is None or tuple(t.shape) != shape or not t.is_contiguous():
+            raise ValueError(f"{name} must be a contiguous tensor of shape {list(shape)}")
+    mj, mm, mf = _modes_ragged_sizes(dim, packed, k, max_joint, max_member, max_free)
+    ri = TbRaggedIn(int(dim), B, _ptr(packed["joint_off"]), _ptr(packed["member_off"]), _ptr(packed["xyz"]),
+                    _ptr(packed["support"]), _ptr(packed["conn"]), _ptr(packed["aed"]), None, mj, mm)
+    mi = TbModesRaggedIn(k, 1 if consistent else 0, None, mf)
+    ai = TbModesAdjIn(_ptr(fwd["eigval"]), _ptr(fwd["modes"]), _ptr(fwd["info"]), _ptr(g_eigval))
+    ao = TbModesAdjOut(_ptr(out.get("joint_xyz")), _ptr(out.get("member_aed")), _ptr(out.get("joint_mass")))
+    st = torch.cuda.current_stream() if stream is None else stream
+    check(lib().tb_modes_adjoint_ragged(C.byref(ri), C.byref(mi), C.byref(ai), C.byref(ao), C.c_void_p(st.cuda_stream)))
+    return out
 
 
 def solve_ragged_device(dim, packed, out=None, stream=None, max_joint=None, max_member=None, _entry="tb_solve_ragged"):

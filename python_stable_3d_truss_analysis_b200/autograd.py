@@ -23,6 +23,9 @@ over the members, nothing solved).  Example -- a frequency penalty for sizing, s
     out = autograd.modes(truss, aed=aed, n_modes=6)
     penalty = torch.relu(lam_min - out["eigval"]).pow(2).sum()
     penalty.backward()                                # aed.grad
+
+``modes_ragged(packed, xyz, aed, joint_mass)`` does the same for a ragged batch (``tb_modes_ragged`` /
+``tb_modes_adjoint_ragged``).
 """
 from __future__ import annotations
 
@@ -31,7 +34,7 @@ import torch
 
 from . import _lib
 
-__all__ = ["solve", "solve_ragged", "modes"]
+__all__ = ["solve", "solve_ragged", "modes", "modes_ragged"]
 
 
 def per_input(g, x):
@@ -282,3 +285,90 @@ def modes(truss, xyz=None, aed=None, joint_mass=None, n_modes=None, consistent=F
     if bx is None and ba is None and bm is None:
         out = {key: v[0] for key, v in out.items()}
     return out
+
+
+class _ModesRagged(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, xyz, aed, joint_mass, joint_off, member_off, support, conn, dim, n_modes, consistent, sizes):
+        p = dict(joint_off=joint_off, member_off=member_off, support=support, conn=conn, xyz=xyz, aed=aed)
+        mj, mm, mf = sizes
+        out = _lib.modes_ragged_device(dim, p, n_modes, consistent=consistent, joint_mass=joint_mass, max_joint=mj,
+                                       max_member=mm, max_free=mf)
+        ctx.save_for_backward(xyz, aed, joint_mass, out["eigval"], out["modes"], out["info"], joint_off, member_off,
+                              support, conn)
+        ctx.dim, ctx.consistent, ctx.sizes = dim, consistent, sizes
+        ctx.mark_non_differentiable(out["modes"], out["n_free"], out["info"])
+        ctx.set_materialize_grads(False)
+        return out["eigval"], out["modes"], out["n_free"], out["info"]
+
+    @staticmethod
+    def backward(ctx, g_eigval, _g_modes, _g_nfree, _g_info):
+        if g_eigval is None:
+            return (None,) * 11
+        xyz, aed, joint_mass, eigval, modes_, info, joint_off, member_off, support, conn = ctx.saved_tensors
+        need_x, need_a, need_m = ctx.needs_input_grad[:3]
+        res = {"joint_xyz": torch.empty_like(xyz) if need_x else None, "member_aed": torch.empty_like(aed) if need_a else None,
+               "joint_mass": torch.empty_like(joint_mass) if need_m else None}
+        p = dict(joint_off=joint_off, member_off=member_off, support=support, conn=conn, xyz=xyz, aed=aed)
+        mj, mm, mf = ctx.sizes
+        _lib.modes_adjoint_ragged_device(ctx.dim, p, {"eigval": eigval, "modes": modes_, "info": info}, g_eigval.contiguous(),
+                                         res, consistent=ctx.consistent, max_joint=mj, max_member=mm, max_free=mf)
+        return (res["joint_xyz"], res["member_aed"], res["joint_mass"]) + (None,) * 8
+
+
+def modes_ragged(packed, xyz=None, aed=None, joint_mass=None, n_modes=6, consistent=False, max_joint=None,
+                 max_member=None, max_free=None):
+    """Modal analysis of a ragged batch (every truss its own topology), with eigenvalues differentiable with respect to
+    ``xyz``, ``aed`` and ``joint_mass``.
+
+    ``packed`` is a dict of CUDA tensors in the layout of ``tb_ragged_in`` (as for ``solve_ragged``; ``force`` is not
+    used).  ``xyz`` [sum nJ, d] or [d sum nJ], ``aed`` [sum M, 3] or [3 sum M] and ``joint_mass`` [sum nJ] are float64
+    CUDA tensors; ``xyz`` / ``aed`` None mean the packed values held constant, ``joint_mass`` None no non-structural
+    mass.  ``n_modes`` lowest modes per truss; ``consistent`` selects the consistent mass matrix.  ``max_joint`` /
+    ``max_member`` / ``max_free`` size the kernels; None reads them from the offsets and support codes (one
+    device-to-host copy).  ``max_free`` defaults to the largest truss's free-DOF count (at least ``n_modes``).
+
+    Returns ``{"eigval": [B, k], "modes": [k d sum nJ], "n_free": [B] int32, "info": [B] int32}``: per truss lambda =
+    omega^2 ascending, its M-normalised mode shapes as the block ``[k][d nJ_b]`` starting at ``k d joint_off[b]``, its
+    free-DOF count and its status (``include/truss_b200.h``).  A truss with fewer than k free DOFs gets zeros past
+    ``n_free[b]``, which take no part in the gradient.  Only ``eigval`` is differentiable; a failed truss has zero outputs
+    and zero gradients.
+
+    Repeated eigenvalues: a single eigenvalue of a cluster is not differentiable, only functions symmetric in the
+    cluster's eigenvalues are.  A loss that treats every mode alike -- ``relu(lam_min - eigval).pow(2).sum()``,
+    ``(1 / eigval).sum()`` -- sends equal cotangents to a cluster and gets its exact gradient, whatever basis of the
+    cluster the forward returned.  A loss that singles out one eigenvalue of a cluster gets a basis-dependent
+    directional value; so does any loss when ``n_modes`` cuts a cluster in two.  Ask for enough modes to keep the
+    clusters you use whole."""
+    for k, dt in (("joint_off", torch.int64), ("member_off", torch.int64), ("support", torch.uint8), ("conn", torch.int32)):
+        t = packed.get(k)
+        if not isinstance(t, torch.Tensor) or t.dtype != dt or t.dim() != 1:
+            raise TypeError(f"packed[{k!r}] must be a 1-D {dt} CUDA tensor")
+    n_modes = int(n_modes)
+    if n_modes < 1:
+        raise ValueError(f"n_modes must be at least 1, not {n_modes}")
+    SJ, SM = int(packed["support"].numel()), int(packed["conn"].numel()) // 2
+    src = xyz if xyz is not None else packed.get("xyz")
+    if isinstance(src, torch.Tensor) and src.dim() == 2:
+        dim = int(src.shape[1])
+    elif isinstance(src, torch.Tensor) and SJ > 0 and src.numel() % SJ == 0:
+        dim = src.numel() // SJ
+    else:
+        raise ValueError("xyz must have shape [sum nJ, d] or [d * sum nJ] with d = 2 or 3")
+    if dim not in (2, 3):
+        raise ValueError(f"xyz must have d = 2 or 3 columns, not {dim}")
+    xyz = _packed_input(xyz, packed.get("xyz"), [(SJ, dim), (SJ * dim,)], "xyz")
+    aed = _packed_input(aed, packed.get("aed"), [(SM, 3), (SM * 3,)], "aed")
+    if joint_mass is not None:
+        joint_mass = _packed_input(joint_mass, None, [(SJ,)], "joint_mass")
+    base = {k: packed[k] for k in ("joint_off", "member_off", "support", "conn")}
+    for k, t in list(base.items()) + [("xyz", xyz), ("aed", aed), ("joint_mass", joint_mass)]:
+        if t is not None and (not t.is_cuda or t.device != xyz.device):
+            raise TypeError(f"{k} must be a CUDA tensor on the device of xyz")
+    xyz, aed = xyz.contiguous(), aed.contiguous()
+    joint_mass = joint_mass.contiguous() if joint_mass is not None else None
+    with torch.cuda.device(xyz.device):
+        sizes = _lib._modes_ragged_sizes(dim, base, n_modes, max_joint, max_member, max_free)
+        eigval, shapes, n_free, info = _ModesRagged.apply(xyz, aed, joint_mass, base["joint_off"], base["member_off"],
+                                                          base["support"], base["conn"], dim, n_modes, bool(consistent), sizes)
+    return {"eigval": eigval, "modes": shapes, "n_free": n_free, "info": info}

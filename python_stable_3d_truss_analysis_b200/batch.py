@@ -10,6 +10,7 @@ hand the whole batch to the CUDA library in one call:
   ``FitnessBatch(...)``                      GA.GetFitness for a population (ga.py:139-149)
   ``SolveWithFixedMemberType(trusses, t)``   the graph-data converter's double solve (data.py:17-44, 108-114)
   ``ModesBatch(truss, ...)``                 natural frequencies and mode shapes of many sizings of one truss
+  ``SolveModesBatch(trusses, ...)``          natural frequencies and mode shapes of trusses of any topologies
 
 All of them return dense numpy arrays (``u [B,N]``, ``ext [B,N]``, ``axial [B,M]``, ``weight [B]``,
 ``info [B]``); ``SolveBatch`` also stores the results back into the Truss objects.
@@ -101,6 +102,54 @@ def ModesBatch(truss: Truss, aed=None, genes=None, memberTypeList=None, nMode=No
         if bad.size:
             raise_for_modes_info(int(out["info"][bad[0]]))
     return out
+
+
+def SolveModesBatch(trusses, nMode=None, isConsistentMass=False, jointMasses=None, raise_on_error=True):
+    """``Truss.SolveModes`` for a list of Truss objects of any topologies in one ragged call (tb_modes_ragged_host); the
+    results are stored into each truss (``GetEigenvalues`` / ``GetNaturalFrequencies`` / ``GetModeShapes``).
+    ``nMode``: modes per truss, None = all modes of each truss (an ``nMode`` above a truss's free-DOF count raises, as
+    ``Truss.SolveModes`` does).  ``jointMasses``: None or one {jointID: mass} dict (or None) per truss.  Returns the
+    per-truss info codes; a failed truss keeps no modes (``raise_on_error`` raises for the first one)."""
+    trusses = list(trusses)
+    if not trusses:
+        return np.zeros(0, np.int32)
+    dim = trusses[0].dim
+    if any(t.dim != dim for t in trusses):
+        raise ValueError("all trusses of a batch must have the same dimension")
+    if jointMasses is not None and len(jointMasses) != len(trusses):
+        raise ValueError(f"jointMasses must hold one entry per truss ({len(trusses)}), not {len(jointMasses)}")
+    dim, jo, mo, xyz, sup, conn, aed, _ = pack_ragged(trusses)
+    cs = np.concatenate([[0], np.cumsum(_lib.free_dofs_per_joint(dim, sup))])
+    n_free = cs[jo[1:]] - cs[jo[:-1]]
+    if nMode is not None:
+        nMode = int(nMode)
+        short = np.nonzero(n_free < nMode)[0]
+        if nMode < 1 or short.size:
+            i = int(short[0]) if short.size else 0
+            raise ValueError(f"nMode = {nMode} is not in [1, {int(n_free[i])}], the free DOFs of truss {i}")
+    jm = None
+    if jointMasses is not None and any(jointMasses):
+        jm = np.zeros(int(jo[-1]))
+        for i, (t, masses) in enumerate(zip(trusses, jointMasses)):
+            for j, mass in (masses or {}).items():
+                if not 0 <= int(j) < t.nJoint:
+                    raise ValueError(f"truss {i}: no such joint [{j}], can't add a mass on it")
+                jm[jo[i] + int(j)] = float(mass)
+    k = int(n_free.max(initial=0)) if nMode is None else nMode
+    k = min(max(k, 1), 160)
+    out = _lib.modes_ragged_host(dim, jo, mo, xyz, sup, conn, aed, k, consistent=isConsistentMass, joint_mass=jm)
+    for i, t in enumerate(trusses):
+        if out["info"][i] != 0:
+            continue
+        q = int(out["n_free"][i]) if nMode is None else nMode
+        N = dim * int(jo[i + 1] - jo[i])
+        block = out["modes"][k * dim * jo[i]:k * dim * jo[i + 1]].reshape(k, N)
+        t._modes = {"eigval": out["eigval"][i, :q].copy(), "modes": block[:q].copy()}
+    if raise_on_error:
+        bad = np.nonzero(out["info"])[0]
+        if bad.size:
+            raise_for_modes_info(int(out["info"][bad[0]]))
+    return out["info"]
 
 
 def pack_ragged(trusses):

@@ -691,9 +691,37 @@ struct EnvScratch {
 };
 EnvScratch g_env[TB_MAX_DEVICES];
 
+// Makes the arena at least `need` bytes for a call on `st`, with S.mu held: it first waits for the previous call when that
+// ran on another stream, then grows stream-ordered (the previous call is ahead on st).  Inside a stream capture the arena
+// is never grown: TB_ERR_ALLOC with nothing enqueued (a warm-up call outside the capture grows it).
+int env_acquire(EnvScratch& S, size_t need, cudaStream_t st, bool* capturing) {
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
+  *capturing = cap != cudaStreamCaptureStatusNone;
+  if (S.bytes < need && *capturing) return TB_ERR_ALLOC;
+  if (!*capturing && S.used && S.last != st && S.ev) TB_CUDA(cudaStreamWaitEvent(st, S.ev, 0));
+  if (S.bytes < need) {
+    if (S.buf) TB_CUDA(cudaFreeAsync(S.buf, st));
+    S.buf = nullptr;
+    S.bytes = 0;
+    TB_CUDA(cudaMallocAsync(&S.buf, need, st));
+    S.bytes = need;
+  }
+  return TB_OK;
+}
+
+// After the call's last kernel on `st`: later calls on other streams wait for it (outside a capture)
+int env_release(EnvScratch& S, cudaStream_t st, bool capturing) {
+  if (capturing) return TB_OK;
+  if (!S.ev) TB_CUDA(cudaEventCreateWithFlags(&S.ev, cudaEventDisableTiming));
+  TB_CUDA(cudaEventRecord(S.ev, st));
+  S.last = st;
+  S.used = true;
+  return TB_OK;
+}
+
 // Envelope kernel over a batch: every truss (route = false), only the trusses above the fused launch's sizes (route:
-// those run first, in one fused launch of the batch), or the ordering mode (order != null).  Inside a stream capture
-// the arena is never grown: TB_ERR_ALLOC with nothing enqueued.
+// those run first, in one fused launch of the batch), or the ordering mode (order != null).
 int run_env(const tb_ragged_in* in, const tb_batch_out* out, bool route, int32_t* order, int64_t* envelope, cudaStream_t st) {
   const int d = in->dim;
   int dev = 0;
@@ -704,19 +732,9 @@ int run_env(const tb_ragged_in* in, const tb_batch_out* out, bool route, int32_t
   int rc = tb_rag_env_config(d, in->max_joint, in->max_member, in->batch, &grid, &smem, &env_smem);
   if (rc) return rc;
   const size_t slot = tb_rag_env_slot_bytes(d, in->max_joint, in->max_member);
-  const size_t need = slot * (size_t)grid;
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
-  const bool capturing = cap != cudaStreamCaptureStatusNone;
-  if (S.bytes < need && capturing) return TB_ERR_ALLOC;          // (a warm-up call outside the capture grows it)
-  if (!capturing && S.used && S.last != st && S.ev) TB_CUDA(cudaStreamWaitEvent(st, S.ev, 0));
-  if (S.bytes < need) {                                          // stream-ordered: the previous call is ahead on st
-    if (S.buf) TB_CUDA(cudaFreeAsync(S.buf, st));
-    S.buf = nullptr;
-    S.bytes = 0;
-    TB_CUDA(cudaMallocAsync(&S.buf, need, st));
-    S.bytes = need;
-  }
+  bool capturing = false;
+  rc = env_acquire(S, slot * (size_t)grid, st, &capturing);
+  if (rc) return rc;
   const int rj = d == 3 ? TB_RAGGED_ROUTE_J3 : TB_RAGGED_ROUTE_J2, rm = d == 3 ? TB_RAGGED_ROUTE_M3 : TB_RAGGED_ROUTE_M2;
   if (route) {                                   // the fused kernels first, sized at the routing limits (k_dense16)
     tb_ragged_in fin = *in;
@@ -740,13 +758,7 @@ int run_env(const tb_ragged_in* in, const tb_batch_out* out, bool route, int32_t
   a.env_smem = env_smem;
   rc = tb_launch_rag_env(a, grid, smem, st);
   if (rc) return rc;
-  if (!capturing) {
-    if (!S.ev) TB_CUDA(cudaEventCreateWithFlags(&S.ev, cudaEventDisableTiming));
-    TB_CUDA(cudaEventRecord(S.ev, st));
-    S.last = st;
-    S.used = true;
-  }
-  return TB_OK;
+  return env_release(S, st, capturing);
 }
 
 // The forward of a ragged batch: today's fused launch when the whole batch fits the fused kernels, else split by truss
@@ -1269,6 +1281,163 @@ extern "C" int tb_modes_host(tb_plan* p, const tb_batch_in* in, const tb_modes_i
   rc = body();
   if (rc) host_pipe_drain(hp);
   return rc;
+}
+
+// ---- modal analysis of ragged batches ---------------------------------------------------------------------------------
+namespace {
+
+// the launch's free-DOF bound: max_free, or every DOF of the largest truss up to the kernel's limit
+int modes_ragged_bound(const tb_ragged_in* in, const tb_modes_ragged_in* m) {
+  return m->max_free ? m->max_free : std::min(in->dim * in->max_joint, TB_SMALL_MAX_DOF);
+}
+
+// Argument checks shared by tb_modes_ragged, tb_modes_ragged_host and tb_modes_adjoint_ragged (in, m non-null): the
+// sizes, then (B > 0) n_modes against the bound, the packed arrays and the ragged size limits; the device last (as
+// tb_solve_ragged, also for B = 0)
+int check_modes_ragged_args(const tb_ragged_in* in, const tb_modes_ragged_in* m) {
+  if (in->dim != 2 && in->dim != 3) return TB_ERR_DIM;
+  if (in->batch < 0 || in->max_joint < 0 || in->max_member < 0) return TB_ERR_SIZE;
+  if (m->consistent != 0 && m->consistent != 1) return TB_ERR_SIZE;
+  if (m->max_free < 0 || m->max_free > TB_SMALL_MAX_DOF || m->n_modes < 1) return TB_ERR_SIZE;
+  if (in->batch > 0) {
+    if (m->n_modes > modes_ragged_bound(in, m)) return TB_ERR_SIZE;
+    if (!in->joint_off || !in->member_off || !in->joint_xyz || !in->support || !in->conn || !in->member_aed)
+      return TB_ERR_NULL;
+    if ((int64_t)in->max_joint * in->dim > TB_RAGGED_MAX_DOF || in->max_member > TB_RAGGED_MAX_MEMBER) return TB_ERR_TOO_LARGE;
+  }
+  if (!have_device()) return TB_ERR_NO_DEVICE;
+  return TB_OK;
+}
+
+int check_modes_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_ragged_out* out) {
+  if (!in || !m || !out) return TB_ERR_NULL;
+  if (!out->eigval || !out->info) return TB_ERR_NULL;
+  return check_modes_ragged_args(in, m);
+}
+
+// One k_modes_ragged launch over the batch (device pointers).  Consistent mass: one bound x bound slot per CTA in the
+// device's envelope arena (g_env: its lock, event and capture rule)
+int run_modes_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_ragged_out* out, cudaStream_t st) {
+  const int bound = modes_ragged_bound(in, m);
+  int threads = 0, smem = 0, per_sm = 0, dev = 0, sms = 0;
+  int rc = tb_modes_ragged_config(in->dim, bound, &threads, &smem, &per_sm);
+  if (rc) return rc;
+  TB_CUDA(cudaGetDevice(&dev));
+  TB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const int grid = (int)std::min<int64_t>(in->batch, (int64_t)sms * per_sm);
+  ModesRagArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.max_joint = in->max_joint; a.max_member = in->max_member; a.max_free = bound;
+  a.n_modes = m->n_modes; a.consistent = m->consistent;
+  a.joint_off = in->joint_off; a.member_off = in->member_off;
+  a.xyz = in->joint_xyz; a.support = in->support; a.conn = in->conn; a.aed = in->member_aed;
+  a.jmass = m->joint_mass;
+  a.eigval = out->eigval; a.modes = out->modes; a.n_free = out->n_free; a.info = out->info;
+  if (!m->consistent) return tb_launch_modes_ragged(a, in->dim, grid, threads, smem, st);
+  EnvScratch& S = g_env[dev & (TB_MAX_DEVICES - 1)];
+  std::lock_guard<std::mutex> lock(S.mu);
+  bool capturing = false;
+  rc = env_acquire(S, (size_t)grid * bound * bound * sizeof(double), st, &capturing);
+  if (rc) return rc;
+  a.slot = (double*)S.buf;
+  rc = tb_launch_modes_ragged(a, in->dim, grid, threads, smem, st);
+  if (rc) return rc;
+  return env_release(S, st, capturing);
+}
+
+}  // namespace
+
+extern "C" int tb_modes_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_ragged_out* out,
+                               void* cuda_stream) {
+  int rc = check_modes_ragged(in, m, out);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  return run_modes_ragged(in, m, out, (cudaStream_t)cuda_stream);
+}
+
+// Host buffers: the offsets are validated on the host, then staged through the ragged staging arena on the host pipe's
+// compute stream (plain cudaMemcpyAsync), as tb_solve_ragged_host
+extern "C" int tb_modes_ragged_host(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_ragged_out* out) {
+  int rc = check_modes_ragged(in, m, out);
+  if (rc) return rc;
+  const int B = in->batch, d = in->dim;
+  if (B == 0) return TB_OK;
+  if (in->joint_off[0] != 0 || in->member_off[0] != 0) return TB_ERR_SIZE;
+  for (int b = 0; b < B; ++b) {
+    const int64_t nj = in->joint_off[b + 1] - in->joint_off[b], nm = in->member_off[b + 1] - in->member_off[b];
+    if (nj < 0 || nm < 0) return TB_ERR_SIZE;
+    if (nj > in->max_joint || nm > in->max_member) return TB_ERR_TOO_LARGE;
+  }
+  const size_t SJ = (size_t)in->joint_off[B], SM = (size_t)in->member_off[B], nm = (size_t)m->n_modes;
+  std::lock_guard<std::mutex> lock(g_pipe_mu);
+  HostPipe* hp = host_pipe();
+  if (!hp) return TB_ERR_ALLOC;
+  int dev = 0;
+  TB_CUDA(cudaGetDevice(&dev));
+  void*& rag_dev = g_rag_dev[dev & (TB_MAX_DEVICES - 1)];
+  size_t& rag_bytes = g_rag_dev_bytes[dev & (TB_MAX_DEVICES - 1)];
+  auto body = [&]() -> int {
+    size_t need = 0;
+    for (size_t bytes : {(size_t)(B + 1) * 8, (size_t)(B + 1) * 8, SJ * d * 8, SJ, SM * 8, SM * 24, m->joint_mass ? SJ * 8 : 0,
+                         (size_t)B * nm * 8, out->modes ? nm * d * SJ * 8 : 0, (size_t)B * 4, (size_t)B * 4})
+      need += Arena::al(bytes);
+    int r2 = arena_reserve(&rag_dev, &rag_bytes, need + 4096);
+    if (r2) return r2;
+    cudaStream_t st = hp->comp;
+    char* cur = (char*)rag_dev;
+    tb_ragged_in din = *in;
+    din.joint_off = take<int64_t>(cur, B + 1);
+    din.member_off = take<int64_t>(cur, B + 1);
+    din.joint_xyz = take<double>(cur, SJ * d);
+    din.support = take<uint8_t>(cur, SJ);
+    din.conn = take<int32_t>(cur, SM * 2);
+    din.member_aed = take<double>(cur, SM * 3);
+    din.force = nullptr;
+    tb_modes_ragged_in dm = *m;
+    dm.joint_mass = m->joint_mass ? take<double>(cur, SJ) : nullptr;
+    tb_modes_ragged_out dout;
+    dout.eigval = take<double>(cur, (size_t)B * nm);
+    dout.modes = out->modes ? take<double>(cur, nm * d * SJ) : nullptr;
+    dout.n_free = take<int32_t>(cur, (size_t)B);
+    dout.info = take<int32_t>(cur, (size_t)B);
+    TB_CUDA(cudaMemcpyAsync((void*)din.joint_off, in->joint_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
+    TB_CUDA(cudaMemcpyAsync((void*)din.member_off, in->member_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
+    TB_CUDA(cudaMemcpyAsync((void*)din.joint_xyz, in->joint_xyz, SJ * d * 8, cudaMemcpyHostToDevice, st));
+    TB_CUDA(cudaMemcpyAsync((void*)din.support, in->support, SJ, cudaMemcpyHostToDevice, st));
+    TB_CUDA(cudaMemcpyAsync((void*)din.conn, in->conn, SM * 8, cudaMemcpyHostToDevice, st));
+    TB_CUDA(cudaMemcpyAsync((void*)din.member_aed, in->member_aed, SM * 24, cudaMemcpyHostToDevice, st));
+    if (m->joint_mass) TB_CUDA(cudaMemcpyAsync((void*)dm.joint_mass, m->joint_mass, SJ * 8, cudaMemcpyHostToDevice, st));
+    r2 = run_modes_ragged(&din, &dm, &dout, st);
+    if (r2) return r2;
+    TB_CUDA(cudaMemcpyAsync(out->eigval, dout.eigval, (size_t)B * nm * 8, cudaMemcpyDeviceToHost, st));
+    if (out->modes) TB_CUDA(cudaMemcpyAsync(out->modes, dout.modes, nm * d * SJ * 8, cudaMemcpyDeviceToHost, st));
+    if (out->n_free) TB_CUDA(cudaMemcpyAsync(out->n_free, dout.n_free, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaStreamSynchronize(st));
+    return TB_OK;
+  };
+  rc = body();
+  if (rc) host_pipe_drain(hp);
+  return rc;
+}
+
+// Reverse mode of tb_modes_ragged: one k_modes_sens_ragged launch, no scratch (always capturable)
+extern "C" int tb_modes_adjoint_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_adj_in* g,
+                                       const tb_modes_adj_out* out, void* cuda_stream) {
+  if (!in || !m || !g || !out) return TB_ERR_NULL;
+  if (!g->eigval || !g->modes || !g->info || !g->g_eigval) return TB_ERR_NULL;
+  int rc = check_modes_ragged_args(in, m);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  ModesSensRagArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.max_joint = in->max_joint; a.max_member = in->max_member;
+  a.n_modes = m->n_modes; a.consistent = m->consistent;
+  a.joint_off = in->joint_off; a.member_off = in->member_off;
+  a.xyz = in->joint_xyz; a.support = in->support; a.conn = in->conn; a.aed = in->member_aed;
+  a.eigval = g->eigval; a.modes = g->modes; a.info = g->info; a.g_eigval = g->g_eigval;
+  a.g_xyz = out->joint_xyz; a.g_aed = out->member_aed; a.g_jmass = out->joint_mass;
+  return tb_launch_modes_sens_ragged(a, in->dim, (cudaStream_t)cuda_stream);
 }
 
 // pinned host buffers for callers that want full-speed H2D/D2H through the *_host entry points

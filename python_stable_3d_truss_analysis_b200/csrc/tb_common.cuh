@@ -400,6 +400,29 @@ struct ModesSensArgs {
 };
 int tb_launch_modes_sens(const ModesSensArgs& a, int dim, cudaStream_t st);
 
+// Modal analysis of a ragged batch (tb_modes_ragged): packed layout of tb_ragged_in, one CTA per truss
+struct ModesRagArgs {
+  int batch, max_joint, max_member, max_free, n_modes, consistent;   // max_free: the launch's free-DOF bound
+  const int64_t* joint_off; const int64_t* member_off;
+  const double* xyz; const uint8_t* support; const int32_t* conn; const double* aed;
+  const double* jmass;                           // [sum nJ] non-structural joint mass, or null
+  double* eigval; double* modes; int32_t* n_free; int32_t* info;   // [B][n_modes], [n_modes d sum nJ] or null, [B] or null, [B]
+  double* slot;                                  // consistent mass: grid slots of max_free^2 doubles, else null
+};
+// CTA size, dynamic shared memory and resident CTAs per SM of k_modes_ragged for a free-DOF bound (1 <= bound <= 160)
+int tb_modes_ragged_config(int dim, int bound, int* threads, int* smem, int* per_sm);
+int tb_launch_modes_ragged(const ModesRagArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st);
+
+// Reverse mode of the ragged modal analysis (tb_modes_adjoint_ragged): one warp per truss, no scratch
+struct ModesSensRagArgs {
+  int batch, max_joint, max_member, n_modes, consistent;
+  const int64_t* joint_off; const int64_t* member_off;
+  const double* xyz; const uint8_t* support; const int32_t* conn; const double* aed;
+  const double* eigval; const double* modes; const int32_t* info; const double* g_eigval;   // packed as the forward's
+  double* g_xyz; double* g_aed; double* g_jmass;                                            // outputs, null = skipped
+};
+int tb_launch_modes_sens_ragged(const ModesSensRagArgs& a, int dim, cudaStream_t st);
+
 // fragment-major offset of element (r, c) inside one 64x64 tile:
 //   [k-half 2][row-block 8][k-slab 8][lane 32], lane = (r%8)*4 + c%4
 // so that one DMMA m8n8k4 operand fragment (8 rows x 4 k) is 32 consecutive doubles and a

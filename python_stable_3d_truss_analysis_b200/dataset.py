@@ -4,6 +4,7 @@ binary container instead of one JSON file per truss, plus the views back into th
 
 * ``PackedDataset.from_json_files``   N reference JSON files -> packed arrays through the native parser (no Truss objects);
 * ``PackedDataset.solve``             the whole container as one ragged GPU batch, results attached to the arrays;
+* ``PackedDataset.solve_modes``       natural frequencies and mode shapes of every truss in one ragged GPU batch;
 * ``PackedDataset.save / load``       one ``.npz`` (optionally compressed) holding every array;
 * ``PackedDataset.json(i)``           truss ``i`` as the reference's JSON dict (``Truss.Serialize``, truss.py:367-395 and
                                       ``detail/combine_with_JSON.md:71-163``: sparse ``displace / external / internal`` lists
@@ -25,6 +26,7 @@ from .utils import CheckDim, ZERO_EPS
 
 _ARRAYS = ("joint_off", "member_off", "xyz", "support", "conn", "aed", "force")
 _RESULTS = ("u", "ext", "axial", "weight", "info")
+_MODES = ("eigval", "modes", "n_free", "modes_info")   # solve_modes: [B, k], [k d sum nJ], [B], [B]
 _SUPPORT_NAMES = {int(v): SupportType.GetFromType(v) for v in (SupportType.NO, SupportType.PIN, SupportType.ROLLER_X,
                                                                SupportType.ROLLER_Y, SupportType.ROLLER_Z)}
 
@@ -36,7 +38,7 @@ class PackedDataset:
     def __init__(self, dim, arrays: dict, names=None):
         self.dim = int(dim)
         self.a = {k: np.asarray(arrays[k]) for k in _ARRAYS}
-        for k in _RESULTS + ("src",):
+        for k in _RESULTS + _MODES + ("src",):
             if k in arrays and arrays[k] is not None:
                 self.a[k] = np.asarray(arrays[k])
         self.names = list(names) if names is not None else None
@@ -124,6 +126,21 @@ class PackedDataset:
                 raise_for_info(int(out["info"][bad[0]]))
         return out["info"]
 
+    def solve_modes(self, nMode, isConsistentMass=False, jointMasses=None):
+        """The ``nMode`` lowest eigenpairs of every truss in one ragged GPU batch (tb_modes_ragged_host) -- labels for
+        surrogates of generated trusses -- attached as ``eigval`` [B, nMode] (lambda = omega^2, ascending), ``modes``
+        [nMode d sum nJ] (truss i's block [nMode][d nJ_i] starts at nMode d joint_off[i]), ``n_free`` [B] (entries past a
+        truss's free-DOF count are 0) and ``modes_info`` [B] (status codes of tb_modes).  ``jointMasses``: None or
+        [sum nJ] non-structural mass per joint.  Returns ``modes_info``."""
+        from . import _lib
+        a = self.a
+        out = _lib.modes_ragged_host(self.dim, a["joint_off"], a["member_off"], a["xyz"], a["support"], a["conn"], a["aed"],
+                                     int(nMode), consistent=isConsistentMass, joint_mass=jointMasses)
+        for k in ("eigval", "modes", "n_free"):
+            self.a[k] = out[k]
+        self.a["modes_info"] = out["info"]
+        return out["info"]
+
     # ------------------------------------------------------------------ binary container
     def save(self, path, compressed=False):
         payload = dict(self.a)
@@ -175,6 +192,10 @@ class PackedDataset:
         t = Truss(d).LoadFromJSON(data={k: v for k, v in self.json(i).items() if k in ("joint", "force", "member")})
         if self.solved and ("info" not in self.a or self.a["info"][i] == 0):
             t._set_dense_results(self.a["u"][d * j0:d * j1], self.a["ext"][d * j0:d * j1], self.a["axial"][m0:m1])
+        if "eigval" in self.a and self.a["modes_info"][i] == 0:
+            k, q = self.a["eigval"].shape[1], int(self.a["n_free"][i])
+            block = self.a["modes"][k * d * j0:k * d * j1].reshape(k, d * (j1 - j0))
+            t._modes = {"eigval": self.a["eigval"][i, :min(k, q)].copy(), "modes": block[:min(k, q)].copy()}
         return t
 
     def dump_json(self, folder, indices=None):
