@@ -303,6 +303,51 @@ typedef struct {
 int tb_modes_adjoint(tb_plan* plan, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_adj_in* a,
                      const tb_modes_adj_out* out, void* cuda_stream);
 
+/* ---- Linear buckling (DESIGN.md section 12) -------------------------------------------------------------------------
+ * For each system of a uniform batch under a given member-force state N (axial [B][M], tension positive: e.g. the
+ * `axial` output of tb_solve / tb_fitness on the same batch, one load case of several, or a prestress; nothing is solved
+ * here): the load factors lambda at which K_ff + lambda K_G,ff becomes singular, i.e. the generalised eigenproblem
+ *   K_ff phi = lambda (-K_G) phi
+ * over the free DOFs.  K_ff is the static solve's stiffness matrix (the same member geometry and ascending-member sums).
+ * K_G is the geometric stiffness in its transverse ("I - c c^T") form: member m from joint j0 to j1 with direction
+ * cosines c and length L adds, with g = N_m / L (correctly rounded),
+ *   +g (delta_ij - c_i c_j) to the blocks (j0, j0) and (j1, j1),  -g (delta_ij - c_i c_j) to (j0, j1) and (j1, j0),
+ * summed in ascending member order like K.  (The simpler form (N/L) I differs from it by a term of relative size N/(EA).)
+ * The solve: K_ff = L L^T (Cholesky), nu = eig(L^-1 K_G L^-T) ranked ascending.  Mode q is critical when nu_q <
+ * -1e-12 max_k |nu_k|; its load factor is lambda_q = -1 / nu_q.  factor[b] holds the n_modes critical factors in
+ * ascending order (factor[b][0] is the critical load factor: the state N times it buckles), then +inf for the modes that
+ * no positive multiple of N reaches.  Factors of the reversed load (nu > 0) are not reported: pass -N for those.
+ * Mode shapes are dense over the N DOFs (0 at supported DOFs, the layout of u), K-normalised (phi^T K_ff phi = 1), the
+ * component of largest magnitude positive (the sign rule of tb_modes); a mode with factor +inf has a zero row.  An
+ * all-zero N is not an error: every factor is +inf.
+ * info: 0, TB_INFO_NOT_STABLE (counting rule), TB_INFO_ZERO_LENGTH, TB_INFO_BAD_INDEX (a gene out of range) as tb_solve;
+ * j + 1 > 0 when the Cholesky factorisation of K_ff meets a pivot that is not > 0 at position j of the free DOFs (the
+ * reference's mask order): K_ff is not positive definite, e.g. a mechanism that passes the counting rule (tb_solve fails
+ * on such a system too); TB_INFO_NO_CONVERGENCE.  A failed system gets zero factors and zero modes.
+ * Plans with n <= 160 free DOFs (TB_SMALL_MAX_DOF); larger: TB_ERR_TOO_LARGE.  `in` as tb_modes (explicit member_aed or
+ * gene + type_table; in->force is ignored and may be NULL).  Argument errors come before TB_ERR_NO_DEVICE: TB_ERR_NULL for
+ * bk, bk->axial, out->factor, out->info; TB_ERR_SIZE for n_modes outside [1, n] or a negative axial_stride; then the
+ * checks of tb_modes.  tb_buckling enqueues on the stream and never synchronises.  Every call uses the plan's modal
+ * scratch (one n x n slot per CTA of the persistent grid, grow-only, grown stream-ordered on the caller's stream, shared
+ * with tb_modes' consistent mass); a call inside a stream capture never grows it: TB_ERR_ALLOC with nothing enqueued (a
+ * warm-up call outside the capture grows it).  tb_buckling_host stages host buffers through the plan (its strides must
+ * be 0 or one row). */
+typedef struct {
+  int32_t n_modes;            /* 1 <= n_modes <= n (free DOFs), else TB_ERR_SIZE */
+  const double* axial;        /* [B][M] member axial forces of the reference state, tension positive -- required */
+  int64_t axial_stride;       /* 0 = shared */
+} tb_buckling_in;
+
+typedef struct {
+  double* factor;             /* [B][n_modes] load factors, ascending, +inf past the critical modes -- required */
+  double* modes;              /* [B][n_modes][N] K-normalised buckling modes, 0 at supports -- or NULL */
+  int32_t* info;              /* [B] -- required */
+} tb_buckling_out;
+
+int tb_buckling(tb_plan* plan, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out,
+                void* cuda_stream);
+int tb_buckling_host(tb_plan* plan, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out);
+
 /* GA.GetFitness for B genes (ga.py:139-149); `full` may be NULL or receive the full results. */
 int tb_fitness(tb_plan* plan, const tb_batch_in* in, double allow_stress, double allow_displace,
                const tb_fit_out* fit, const tb_batch_out* full, void* cuda_stream);

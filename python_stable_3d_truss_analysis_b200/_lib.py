@@ -177,6 +177,14 @@ class TbModesAdjOut(C.Structure):
     _fields_ = [("joint_xyz", C.c_void_p), ("member_aed", C.c_void_p), ("joint_mass", C.c_void_p)]
 
 
+class TbBucklingIn(C.Structure):
+    _fields_ = [("n_modes", C.c_int32), ("axial", C.c_void_p), ("axial_stride", C.c_int64)]
+
+
+class TbBucklingOut(C.Structure):
+    _fields_ = [("factor", C.c_void_p), ("modes", C.c_void_p), ("info", C.c_void_p)]
+
+
 class TbModesRaggedIn(C.Structure):
     _fields_ = [("n_modes", C.c_int32), ("consistent", C.c_int32), ("joint_mass", C.c_void_p), ("max_free", C.c_int32)]
 
@@ -192,7 +200,7 @@ class TbRaggedIn(C.Structure):
 
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
-           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_modes_adjoint", "tb_modes_ragged", "tb_modes_ragged_host", "tb_modes_adjoint_ragged", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
+           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_modes_adjoint", "tb_modes_ragged", "tb_modes_ragged_host", "tb_modes_adjoint_ragged", "tb_buckling", "tb_buckling_host", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
            "tb_solve_ragged_host", "tb_solve_ragged_env", "tb_ragged_env_order", "tb_ragged_limits", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
@@ -232,6 +240,8 @@ def lib():
     L.tb_modes_ragged_host.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbModesRaggedIn), C.POINTER(TbModesRaggedOut)]
     L.tb_modes_adjoint_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbModesRaggedIn), C.POINTER(TbModesAdjIn),
                                           C.POINTER(TbModesAdjOut), vp]
+    L.tb_buckling.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBucklingIn), C.POINTER(TbBucklingOut), vp]
+    L.tb_buckling_host.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBucklingIn), C.POINTER(TbBucklingOut)]
     L.tb_fitness.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut), vp]
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
@@ -712,6 +722,65 @@ class Plan:
         ao = TbModesAdjOut(_ptr(out.get("joint_xyz")), _ptr(out.get("member_aed")), _ptr(out.get("joint_mass")))
         st = torch.cuda.current_stream() if stream is None else stream
         check(lib().tb_modes_adjoint(self._h, C.byref(bi), C.byref(mi), C.byref(ai), C.byref(ao), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def _buckling_in(self, B, axial, n_modes, axial_stride, keep):
+        """tb_buckling_in; ``axial`` is [M] (shared) or [B, M] unless ``axial_stride`` (elements between systems) is given;
+        ``n_modes=None`` asks for all n modes."""
+        ax = _np(axial, np.float64) if isinstance(axial, (np.ndarray, list, tuple)) else axial
+        total = int(np.prod(ax.shape))
+        if axial_stride is None:
+            if total not in (self.M, self.M * B):
+                raise ValueError(f"axial of {total} elements is neither [{self.M}] nor [{B},{self.M}]")
+            axial_stride = 0 if total == self.M else self.M
+        axial_stride = int(axial_stride)
+        if axial_stride < 0 or (B > 0 and total < (B - 1) * axial_stride + self.M):
+            raise ValueError(f"axial of {total} elements does not hold {B} rows of {self.M} at stride {axial_stride}")
+        keep.append(ax)
+        return TbBucklingIn(self.n if n_modes is None else int(n_modes), _ptr(ax), axial_stride)
+
+    def buckling_host(self, B, xyz, axial, aed=None, gene=None, type_table=None, n_modes=None, axial_stride=None,
+                      out=None, want_modes=True):
+        """Linear buckling of B systems under the member forces ``axial`` (tb_buckling_host), host (numpy) buffers:
+        ``factor`` [B, n_modes] (critical load factors ascending, inf for modes no positive multiple of the load reaches),
+        ``modes`` [B, n_modes, N] (K-normalised, 0 at supported DOFs and for inf factors; skipped with
+        ``want_modes=False``) and ``info`` [B].  ``axial`` is the ``axial`` output of a solve of the same batch, [M] or
+        [B, M]; ``n_modes=None`` = all n modes."""
+        keep = []
+        bi = self._batch_in(B, xyz, aed, gene, type_table, np.zeros(self.N), keep)
+        bi.force, bi.force_stride = None, 0            # (ignored by tb_buckling)
+        bk = self._buckling_in(B, axial, n_modes, axial_stride, keep)
+        nm = bk.n_modes
+        out = {} if out is None else out
+        out.setdefault("factor", np.empty((B, nm), np.float64))
+        if want_modes:
+            out.setdefault("modes", np.empty((B, nm, self.N), np.float64))
+        out.setdefault("info", np.empty(B, np.int32))
+        bo = TbBucklingOut(_ptr(out["factor"]), _ptr(out.get("modes")), _ptr(out["info"]))
+        check(lib().tb_buckling_host(self._h, C.byref(bi), C.byref(bk), C.byref(bo)))
+        return out
+
+    def buckling_device(self, B, xyz, axial, aed=None, gene=None, type_table=None, n_modes=None, axial_stride=None,
+                        out=None, stream=None):
+        """tb_buckling on torch CUDA tensors; enqueues on ``stream`` (a torch stream or None = current).  ``axial`` is a
+        CUDA tensor [M] or [B, M] (e.g. the "axial" output of ``solve_device`` / ``fitness_device`` on the same batch), or
+        any rows at ``axial_stride`` elements apart.  ``out`` maps "factor" [B, n_modes] and "info" [B] (allocated when
+        missing) and optionally "modes" [B, n_modes, N]."""
+        import torch
+
+        keep = []
+        bi = self._batch_in(B, xyz, aed, gene, type_table, np.zeros(self.N), keep)
+        bi.force, bi.force_stride = None, 0            # (ignored by tb_buckling)
+        bk = self._buckling_in(B, axial, n_modes, axial_stride, keep)
+        dev = xyz.device if hasattr(xyz, "device") else torch.device("cuda", torch.cuda.current_device())
+        out = {} if out is None else out
+        if out.get("factor") is None:
+            out["factor"] = torch.empty((B, bk.n_modes), dtype=torch.float64, device=dev)
+        if out.get("info") is None:
+            out["info"] = torch.empty(B, dtype=torch.int32, device=dev)
+        st = torch.cuda.current_stream() if stream is None else stream
+        bo = TbBucklingOut(_ptr(out["factor"]), _ptr(out.get("modes")), _ptr(out["info"]))
+        check(lib().tb_buckling(self._h, C.byref(bi), C.byref(bk), C.byref(bo), C.c_void_p(st.cuda_stream)))
         return out
 
     def fitness_device(self, B, xyz, force, gene, type_table, allow_stress, allow_displace, out, aed=None, stream=None):

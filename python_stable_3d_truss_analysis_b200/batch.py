@@ -11,6 +11,7 @@ hand the whole batch to the CUDA library in one call:
   ``SolveWithFixedMemberType(trusses, t)``   the graph-data converter's double solve (data.py:17-44, 108-114)
   ``ModesBatch(truss, ...)``                 natural frequencies and mode shapes of many sizings of one truss
   ``SolveModesBatch(trusses, ...)``          natural frequencies and mode shapes of trusses of any topologies
+  ``BucklingBatch(truss, ...)``              critical load factors and buckling modes of many sizings of one truss
 
 All of them return dense numpy arrays (``u [B,N]``, ``ext [B,N]``, ``axial [B,M]``, ``weight [B]``,
 ``info [B]``); ``SolveBatch`` also stores the results back into the Truss objects.
@@ -97,6 +98,37 @@ def ModesBatch(truss: Truss, aed=None, genes=None, memberTypeList=None, nMode=No
         genes = np.ascontiguousarray(genes, dtype=np.int32).reshape(-1, truss.nMember)
         out = plan.modes_host(genes.shape[0], xyz, gene=genes, type_table=type_table(memberTypeList), n_modes=nMode,
                               consistent=isConsistentMass, joint_mass=jm, want_modes=want_modes)
+    if raise_on_error:
+        bad = np.nonzero(out["info"])[0]
+        if bad.size:
+            raise_for_modes_info(int(out["info"][bad[0]]))
+    return out
+
+
+def BucklingBatch(truss: Truss, aed=None, genes=None, memberTypeList=None, nMode=None, raise_on_error=True,
+                  want_modes=True):
+    """Linear buckling of B sizings of one truss under its loads (``Truss.SolveBuckling`` per design, e.g. a stability
+    constraint on a GA population): one static call (tb_solve_host) for the member forces, then one buckling call
+    (tb_buckling_host) with them.  Member properties are either explicit, ``aed`` [B, M, 3] (a, e, density), or
+    ``genes`` int [B, M] of indices into ``memberTypeList``.  Returns dict(factor [B, k] (load factors ascending, inf for
+    modes no positive multiple of the loads reaches), modes [B, k, N] (K-normalised, 0 at supported DOFs and for inf
+    factors; with ``want_modes``), axial [B, M] (the member forces of the static solve), info [B] (the buckling call's:
+    it fails where the static solve does)); ``nMode=None`` = one per free DOF."""
+    xyz, support, conn, _, force = truss._pack()
+    plan = truss._get_plan(support, conn)
+    if (aed is None) == (genes is None):
+        raise ValueError("give either aed or genes (with memberTypeList)")
+    if aed is not None:
+        aed = np.ascontiguousarray(aed, dtype=np.float64).reshape(-1, truss.nMember * 3)
+        props = dict(aed=aed)
+        B = aed.shape[0]
+    else:
+        genes = np.ascontiguousarray(genes, dtype=np.int32).reshape(-1, truss.nMember)
+        props = dict(gene=genes, type_table=type_table(memberTypeList))
+        B = genes.shape[0]
+    st = plan.solve_host(B, xyz, force, want=("axial",), **props)
+    out = plan.buckling_host(B, xyz, st["axial"], n_modes=nMode, want_modes=want_modes, **props)
+    out["axial"] = st["axial"]
     if raise_on_error:
         bad = np.nonzero(out["info"])[0]
         if bad.size:

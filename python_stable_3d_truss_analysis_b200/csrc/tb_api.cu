@@ -1136,6 +1136,42 @@ int check_modes(const tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, c
   return check_modes_args(p, in, m);
 }
 
+// The plan's modal arena for a launch of `grid` CTAs: one n x n slot of doubles per CTA, grow-only, grown stream-ordered
+// on the caller's stream, never inside a stream capture (TB_ERR_ALLOC with nothing enqueued; a warm-up call outside the
+// capture grows it).  Orders the arena after the previous call's kernels (ws_acquire): the caller launches, then
+// ws_release.  With the plan lock held.
+int modes_slots(tb_plan* p, int grid, cudaStream_t st) {
+  const size_t need = (size_t)grid * p->n * p->n * sizeof(double);
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
+  if (p->modes_bytes < need && cap != cudaStreamCaptureStatusNone) return TB_ERR_ALLOC;
+  int rc = ws_acquire(p, st);
+  if (rc) return rc;
+  if (p->modes_bytes < need) {
+    if (p->modes_buf) TB_CUDA(cudaFreeAsync(p->modes_buf, st));
+    p->modes_buf = nullptr;
+    p->modes_bytes = 0;
+    TB_CUDA(cudaMallocAsync(&p->modes_buf, need, st));
+    p->modes_bytes = need;
+  }
+  return TB_OK;
+}
+
+// The batch and plan fields of a k_modes / k_buckling launch
+void modes_args(const tb_plan* p, const tb_batch_in* in, ModesArgs& a) {
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.nJ = p->nJ; a.M = p->M; a.N = p->N; a.n = p->n;
+  a.plan_stable = p->stable; a.n_type = in->n_type;
+  a.xyz = in->joint_xyz; a.xyz_stride = in->joint_stride;
+  a.aed = in->member_aed; a.aed_stride = in->member_stride;
+  a.gene = in->member_aed ? nullptr : in->gene; a.gene_stride = in->gene_stride;
+  a.type_table = in->type_table;
+  a.conn = p->d_conn; a.free_ref = p->d_free_ref; a.dof2free = p->d_dof2free;
+  a.ent_row = p->d_ent_row; a.ent_col = p->d_ent_col; a.ent_ptr = p->d_ent_ptr; a.nnz = (int64_t)p->ent_row.size();
+  a.ctr_member = p->d_ctr_member; a.ctr_local = p->d_ctr_local;
+  a.inc_ptr = p->d_inc_ptr; a.inc_mem = p->d_inc_mem;
+}
+
 // One k_modes launch over the batch (device pointers), with the plan lock held
 int run_modes(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_modes_out* out, cudaStream_t st) {
   int threads = 0, smem = 0, per_sm = 0;
@@ -1143,34 +1179,14 @@ int run_modes(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_
   if (rc) return rc;
   const int sms = p->num_sm > 0 ? p->num_sm : 148;
   const int grid = (int)std::min<int64_t>(in->batch, (int64_t)sms * per_sm);
-  if (m->consistent) {                           // the consistent mass's slots: grow-only, stream-ordered, never in a capture
-    const size_t need = (size_t)grid * p->n * p->n * sizeof(double);
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
-    if (p->modes_bytes < need && cap != cudaStreamCaptureStatusNone) return TB_ERR_ALLOC;
-    rc = ws_acquire(p, st);
+  if (m->consistent) {                           // the consistent mass's slots
+    rc = modes_slots(p, grid, st);
     if (rc) return rc;
-    if (p->modes_bytes < need) {
-      if (p->modes_buf) TB_CUDA(cudaFreeAsync(p->modes_buf, st));
-      p->modes_buf = nullptr;
-      p->modes_bytes = 0;
-      TB_CUDA(cudaMallocAsync(&p->modes_buf, need, st));
-      p->modes_bytes = need;
-    }
   }
   ModesArgs a;
-  memset(&a, 0, sizeof(a));
-  a.batch = in->batch; a.nJ = p->nJ; a.M = p->M; a.N = p->N; a.n = p->n;
-  a.n_modes = m->n_modes; a.consistent = m->consistent; a.plan_stable = p->stable; a.n_type = in->n_type;
-  a.xyz = in->joint_xyz; a.xyz_stride = in->joint_stride;
-  a.aed = in->member_aed; a.aed_stride = in->member_stride;
-  a.gene = in->member_aed ? nullptr : in->gene; a.gene_stride = in->gene_stride;
-  a.type_table = in->type_table;
+  modes_args(p, in, a);
+  a.n_modes = m->n_modes; a.consistent = m->consistent;
   a.jmass = m->joint_mass; a.jmass_stride = m->joint_mass_stride;
-  a.conn = p->d_conn; a.free_ref = p->d_free_ref; a.dof2free = p->d_dof2free;
-  a.ent_row = p->d_ent_row; a.ent_col = p->d_ent_col; a.ent_ptr = p->d_ent_ptr; a.nnz = (int64_t)p->ent_row.size();
-  a.ctr_member = p->d_ctr_member; a.ctr_local = p->d_ctr_local;
-  a.inc_ptr = p->d_inc_ptr; a.inc_mem = p->d_inc_mem;
   a.eigval = out->eigval; a.modes = out->modes; a.info = out->info;
   a.slot = m->consistent ? (double*)p->modes_buf : nullptr;
   rc = tb_launch_modes(a, p->dim, grid, threads, smem, st);
@@ -1273,6 +1289,124 @@ extern "C" int tb_modes_host(tb_plan* p, const tb_batch_in* in, const tb_modes_i
     r2 = run_modes(p, &din, &dm, &dout, st);
     if (r2) return r2;
     TB_CUDA(cudaMemcpyAsync(out->eigval, dout.eigval, nval * 8, cudaMemcpyDeviceToHost, st));
+    if (out->modes) TB_CUDA(cudaMemcpyAsync(out->modes, dout.modes, nmode * 8, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaStreamSynchronize(st));
+    return TB_OK;
+  };
+  rc = body();
+  if (rc) host_pipe_drain(hp);
+  return rc;
+}
+
+// ---- linear buckling (DESIGN.md section 12) ---------------------------------------------------------------------------
+namespace {
+
+// Argument checks of tb_buckling / tb_buckling_host: the pointers, the axial stride, then tb_modes' checks (sizes, the
+// free-DOF limit, the inputs, the device)
+int check_buckling(const tb_plan* p, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out) {
+  if (!p || !in || !bk || !out) return TB_ERR_NULL;
+  if (!bk->axial || !out->factor || !out->info) return TB_ERR_NULL;
+  if (bk->axial_stride < 0) return TB_ERR_SIZE;
+  const tb_modes_in m = {bk->n_modes, 0, nullptr, 0};
+  return check_modes_args(p, in, &m);
+}
+
+// One k_buckling launch over the batch (device pointers), with the plan lock held: K_ff and its factor take one slot
+// of the modal arena per CTA on every call
+int run_buckling(tb_plan* p, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out, cudaStream_t st) {
+  int threads = 0, smem = 0, per_sm = 0;
+  int rc = tb_buckling_config(p->dim, p->n, &threads, &smem, &per_sm);
+  if (rc) return rc;
+  const int sms = p->num_sm > 0 ? p->num_sm : 148;
+  const int grid = (int)std::min<int64_t>(in->batch, (int64_t)sms * per_sm);
+  rc = modes_slots(p, grid, st);
+  if (rc) return rc;
+  BucklingArgs a;
+  memset(&a, 0, sizeof(a));
+  modes_args(p, in, a.base);
+  a.base.n_modes = bk->n_modes; a.base.consistent = 1;
+  a.base.eigval = out->factor; a.base.modes = out->modes; a.base.info = out->info;
+  a.base.slot = (double*)p->modes_buf;
+  a.axial = bk->axial; a.axial_stride = bk->axial_stride;
+  rc = tb_launch_buckling(a, p->dim, grid, threads, smem, st);
+  if (rc) return rc;
+  return ws_release(p, st);
+}
+
+}  // namespace
+
+extern "C" int tb_buckling(tb_plan* p, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out,
+                           void* cuda_stream) {
+  int rc = check_buckling(p, in, bk, out);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  rc = check_device(p);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lock(p->mu);
+  return run_buckling(p, in, bk, out, (cudaStream_t)cuda_stream);
+}
+
+// Host buffers: staged through the plan's arena like tb_modes_host (plain cudaMemcpyAsync on the compute stream)
+extern "C" int tb_buckling_host(tb_plan* p, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out) {
+  int rc = check_buckling(p, in, bk, out);
+  if (rc) return rc;
+  const int B = in->batch;
+  if (B == 0) return TB_OK;
+  const int64_t rowJ = (int64_t)p->nJ * p->dim, rowM3 = (int64_t)p->M * 3, rowM = p->M, nm = bk->n_modes;
+  if (!stride_ok(in->joint_stride, rowJ)) return TB_ERR_SIZE;
+  if (in->member_aed && !stride_ok(in->member_stride, rowM3)) return TB_ERR_SIZE;
+  if (!in->member_aed && !stride_ok(in->gene_stride, rowM)) return TB_ERR_SIZE;
+  if (!stride_ok(bk->axial_stride, rowM)) return TB_ERR_SIZE;
+  rc = check_device(p);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> pipe_lock(g_pipe_mu);
+  std::lock_guard<std::mutex> plan_lock(p->mu);
+  HostPipe* hp = host_pipe();
+  if (!hp) return TB_ERR_ALLOC;
+  rc = async_drain(p);
+  if (rc) return rc;
+  auto cnt = [&](int64_t stride, int64_t row) { return (size_t)(stride == 0 ? row : row * B); };
+  const size_t nxyz = cnt(in->joint_stride, rowJ);
+  const size_t naed = in->member_aed ? cnt(in->member_stride, rowM3) : 0;
+  const size_t ngene = in->member_aed ? 0 : cnt(in->gene_stride, rowM);
+  const size_t ntab = in->member_aed ? 0 : (size_t)in->n_type * 3;
+  const size_t nax = cnt(bk->axial_stride, rowM);
+  const size_t nval = (size_t)B * nm, nmode = out->modes ? (size_t)B * nm * p->N : 0;
+  size_t need = 0;
+  for (size_t bytes : {nxyz * 8, naed * 8, ngene * 4, ntab * 8, nax * 8, nval * 8, nmode * 8, (size_t)B * 4}) need += Arena::al(bytes);
+  cudaStream_t st = hp->comp;
+  auto body = [&]() -> int {
+    int r2 = arena_reserve(&p->stage_dev, &p->stage_dev_bytes, need + 4096);
+    if (r2) return r2;
+    char* cur = (char*)p->stage_dev;
+    double* dxyz = take<double>(cur, nxyz);
+    double* daed = take<double>(cur, naed);
+    int32_t* dgene = take<int32_t>(cur, ngene);
+    double* dtab = take<double>(cur, ntab);
+    double* dax = take<double>(cur, nax);
+    tb_buckling_out dout = {take<double>(cur, nval), out->modes ? take<double>(cur, nmode) : nullptr,
+                            take<int32_t>(cur, (size_t)B)};
+    TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, nxyz * 8, cudaMemcpyHostToDevice, st));
+    tb_batch_in din = *in;
+    din.joint_xyz = dxyz;
+    din.force = nullptr;
+    if (in->member_aed) {
+      TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, naed * 8, cudaMemcpyHostToDevice, st));
+      din.member_aed = daed;
+      din.gene = nullptr;
+    } else {
+      TB_CUDA(cudaMemcpyAsync(dgene, in->gene, ngene * 4, cudaMemcpyHostToDevice, st));
+      TB_CUDA(cudaMemcpyAsync(dtab, in->type_table, ntab * 8, cudaMemcpyHostToDevice, st));
+      din.gene = dgene;
+      din.type_table = dtab;
+    }
+    TB_CUDA(cudaMemcpyAsync(dax, bk->axial, nax * 8, cudaMemcpyHostToDevice, st));
+    tb_buckling_in dbk = *bk;
+    dbk.axial = dax;
+    r2 = run_buckling(p, &din, &dbk, &dout, st);
+    if (r2) return r2;
+    TB_CUDA(cudaMemcpyAsync(out->factor, dout.factor, nval * 8, cudaMemcpyDeviceToHost, st));
     if (out->modes) TB_CUDA(cudaMemcpyAsync(out->modes, dout.modes, nmode * 8, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaStreamSynchronize(st));

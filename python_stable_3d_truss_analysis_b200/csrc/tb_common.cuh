@@ -175,7 +175,8 @@ struct tb_plan {
   // status [B], and the per-member vectors [B][M][d] when they do not fit shared memory
   void* adj_buf = nullptr;
   size_t adj_bytes = 0;
-  // tb_modes scratch of the consistent mass (grow-only, grown stream-ordered): one n x n slot per CTA of the launch
+  // modal scratch of tb_modes' consistent mass and of tb_buckling (grow-only, grown stream-ordered): one n x n slot per CTA
+  // of the launch
   void* modes_buf = nullptr;
   size_t modes_bytes = 0;
   // pipelined host calls (tb_solve_host_async): TB_ASYNC_SLOTS more staging arenas used in turn by consecutive calls,
@@ -388,6 +389,17 @@ struct ModesArgs {
 // CTA size, dynamic shared memory and resident CTAs per SM of k_modes for n free DOFs (1 <= n <= TB_SMALL_MAX_DOF)
 int tb_modes_config(int dim, int n, int* threads, int* smem, int* per_sm);
 int tb_launch_modes(const ModesArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st);
+
+// Linear buckling (tb_buckling, tb_modes.cu): k_modes' layout and plan maps in `base` (eigval = the load factors
+// [B][n_modes], modes = [B][n_modes][N] or null, slot = grid slots of n x n doubles: K_ff and its factor; jmass and
+// consistent are not read), plus the member axial forces of the reference state
+struct BucklingArgs {
+  ModesArgs base;
+  const double* axial; int64_t axial_stride;     // [B][M] tension positive, stride 0 = shared
+};
+// CTA size, dynamic shared memory and resident CTAs per SM of k_buckling for n free DOFs (1 <= n <= TB_SMALL_MAX_DOF)
+int tb_buckling_config(int dim, int n, int* threads, int* smem, int* per_sm);
+int tb_launch_buckling(const BucklingArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st);
 
 // Reverse mode of the modal analysis (tb_modes_adjoint): one warp per system, no scratch
 struct ModesSensArgs {

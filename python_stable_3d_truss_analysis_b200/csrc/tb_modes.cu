@@ -19,11 +19,13 @@
 // bits do not depend on its position in the batch, the batch size, the CTA size or the number of resident CTAs.
 //
 // Steps 2-5 are __device__ functions (modes_eigen, modes_order) shared with k_modes_ragged<DIM> (tb_modes_ragged), which
-// differs in step 1 and in where it writes; see there.
+// differs in step 1 and in where it writes, and with k_buckling<DIM> (tb_buckling, linear buckling: K_ff phi =
+// lambda (-K_G) phi), which differs in step 1 and in its output step; see there.
 //
 // k_modes_sens<DIM> is the reverse mode (tb_modes_adjoint): eigenvalue gradients from the forward's modes, below, and
 // k_modes_sens_ragged<DIM> its ragged form (tb_modes_adjoint_ragged).
 #include <cfloat>
+#include <math_constants.h>
 
 #include "tb_common.cuh"
 
@@ -34,6 +36,7 @@ constexpr int TQL_MAX_ITER = 30;   // QL sweeps per eigenvalue (EISPACK tql2's c
 struct ModesCtl {
   double h;
   int any, lo, status;
+  int piv;   // position (free-DOF row) of the pivot where the Cholesky of the slot stopped
 };
 
 // (a, e, density) of member m from the explicit rows or the gene / type table; ok = false for a gene out of range
@@ -99,7 +102,9 @@ __device__ __forceinline__ ModesSmem modes_smem(double* base, int n, int* perm) 
 
 // Steps 2-4 of one system (n >= 1): standard problem, tred2, tql2.  Entered with K_ff in Z (both triangles) and the mass
 // (lumped: s.sc; consistent: M_ff in L, row pitch n); returns the status (TB_INFO_MASS, TB_INFO_NO_CONVERGENCE or 0)
-// with the eigenvalues in s.dv and the eigenvectors of K~ in the columns of Z.  Shared by k_modes and k_modes_ragged.
+// with the eigenvalues in s.dv and the eigenvectors of K~ in the columns of Z.  Shared by k_modes, k_modes_ragged and
+// k_buckling (which enters with K_G in Z and K_ff in L).  TB_INFO_MASS means the Cholesky of L met a pivot that is not
+// > 0, at row ctl.piv.
 __device__ __forceinline__ int modes_eigen(const ModesSmem& s, int n, int consistent, double* L, ModesCtl& ctl,
                                            int status) {
   const int P = n | 1;
@@ -124,6 +129,7 @@ __device__ __forceinline__ int modes_eigen(const ModesSmem& s, int n, int consis
         double x = Lj[j];
         for (int k = 0; k < j; ++k) x -= Lj[k] * Lj[k];
         ctl.status = x > 0.0 ? 0 : TB_INFO_MASS;
+        if (!(x > 0.0)) ctl.piv = j;
         Lj[j] = x > 0.0 ? sqrt(x) : 0.0;
       }
       __syncthreads();
@@ -470,6 +476,121 @@ __global__ void __launch_bounds__(160) k_modes(const ModesArgs a) {
   }
 }
 
+// ---- linear buckling (tb_buckling): K_ff phi = lambda (-K_G) phi for a given member-force state N
+// k_buckling<DIM> is k_modes with its own step 1 and output step.  Step 1: the static solve's guards, then one pass over
+// the plan's scatter map assembles K_ff into the CTA's slot and the geometric stiffness K_G into Z, both triangles, both
+// in ascending member order.  Member m contributes to K_G, per block (A, B) and local (i, j),
+//   +-g (delta_ij - c_i c_j),  g = N_m / L_m (correctly rounded), + on the diagonal blocks, c_i c_j rounded as K's product
+// (the transverse "I - c c^T" form of the truss geometric stiffness).  Steps 2-5 are modes_eigen / modes_order with K_ff
+// as the "mass": nu = eig(L^-1 K_G L^-T), K_ff = L L^T, ascending, modes back-transformed by L^T y = z (so K-normalised).
+// Output step: mode q is critical when nu_q < -BUCKLING_TAU max_k |nu_k|; its load factor is -1 / nu_q (ascending with
+// q), any other mode gets +inf and a zero row.  A pivot of K_ff that is not > 0 at free-DOF row j gives info j + 1.
+// Registers: (160, 4) lets ptxas allocate 85 registers with no spills; with (160) alone it holds the kernel at 72-96
+// registers and spills 80-120 bytes.  85 registers and k_modes' shared memory give at least k_modes' residency at every n.
+constexpr double BUCKLING_TAU = 1e-12;   // relative threshold below which -nu counts as a critical eigenvalue
+
+template <int DIM>
+__global__ void __launch_bounds__(160, 4) k_buckling(const BucklingArgs ba) {
+  extern __shared__ __align__(16) double smem[];
+  __shared__ ModesCtl ctl;
+  const ModesArgs& a = ba.base;
+  const int n = a.n, P = n | 1, N = a.N, nm = a.n_modes;
+  const int tid = threadIdx.x, nth = blockDim.x;
+  int* i2r = (int*)(smem + (size_t)n * P + 8 * (size_t)n);   // internal row of the plan's scatter map -> free DOF in the reference's order
+  const ModesSmem s = modes_smem(smem, n, i2r + n);
+  double* Z = s.Z;
+  for (int r = tid; r < n; r += nth) i2r[a.dof2free[a.free_ref[r]]] = r;
+  double* L = a.slot + (size_t)blockIdx.x * n * n;           // K_ff, then its Cholesky factor
+
+  for (int b = blockIdx.x; b < a.batch; b += gridDim.x) {
+    const double* xyz = a.xyz + b * a.xyz_stride;
+    const double* aed = a.aed ? a.aed + b * a.aed_stride : nullptr;
+    const int32_t* gene = a.aed ? nullptr : a.gene + b * a.gene_stride;
+    __syncthreads();                           // the previous system's shared data is consumed (and i2r is complete)
+
+    // ---- status guards of the static solve, in its order of precedence
+    int bad = 0;
+    for (int m = tid; m < a.M; m += nth) {
+      double ar, e, rho;
+      bool ok;
+      member_props(a, aed, gene, m, ar, e, rho, ok);
+      if (!ok) {
+        bad |= 1;
+      } else {
+        double k, c[DIM], w;
+        if (!(member_kcw<DIM>(a, xyz, aed, gene, m, k, c, w) > 0.0)) bad |= 2;
+      }
+    }
+    const int anyidx = __syncthreads_or(bad & 1), anylen = __syncthreads_or(bad & 2);
+    int status = a.plan_stable ? 0 : TB_INFO_NOT_STABLE;
+    if (anyidx) status = min(status, TB_INFO_BAD_INDEX);
+    else if (anylen) status = min(status, TB_INFO_ZERO_LENGTH);
+
+    if (status == 0) {
+      // ---- K_ff into the slot, K_G into Z, densely, both triangles, one pass over the scatter map
+      const double* ax = ba.axial + b * ba.axial_stride;
+      for (int i = tid; i < n * P; i += nth) Z[i] = 0.0;
+      for (int i = tid; i < n * n; i += nth) L[i] = 0.0;
+      __syncthreads();
+      for (int64_t e = tid; e < a.nnz; e += nth) {
+        const int r = i2r[a.ent_row[e]], c = i2r[a.ent_col[e]];
+        double kv = 0.0, gv = 0.0;
+        for (int64_t q = a.ent_ptr[e]; q < a.ent_ptr[e + 1]; ++q) {
+          const int m = a.ctr_member[q], loc = a.ctr_local[q];
+          const int la = loc / (2 * DIM), lb = loc - la * (2 * DIM);
+          const int A = la / DIM, i = la - A * DIM, B = lb / DIM, j = lb - B * DIM;
+          double k, cs[DIM], w;
+          const double len = member_kcw<DIM>(a, xyz, aed, gene, m, k, cs, w);
+          const double g = __ddiv_rn(ax[m], len);
+          double pr = __dmul_rn(cs[i], cs[j]);   // truss.py:69,80
+          double t = i == j ? __dsub_rn(1.0, pr) : -pr;
+          if (A != B) {
+            pr = -pr;
+            t = -t;
+          }
+          kv = __dadd_rn(kv, __dmul_rn(k, pr));  // truss.py:70,314
+          gv = __dadd_rn(gv, __dmul_rn(g, t));
+        }
+        Z[r * P + c] = gv;
+        Z[c * P + r] = gv;
+        L[r * n + c] = kv;
+        L[c * n + r] = kv;
+      }
+      __syncthreads();
+    }
+
+    status = modes_eigen(s, n, 1, L, ctl, status);
+    if (status == TB_INFO_MASS) status = ctl.piv + 1;   // K_ff is not positive definite: the static solve's info
+
+    double* frow = a.eigval + (int64_t)b * nm;
+    double* mo = a.modes ? a.modes + (int64_t)b * nm * N : nullptr;
+    if (status == 0) {
+      modes_order(s, n, nm, 1, L, frow);
+      double vmax = 0.0;                       // (every thread, same value)
+      for (int j = 0; j < n; ++j) vmax = fmax(vmax, fabs(s.dv[j]));
+      const double thr = -BUCKLING_TAU * vmax;
+      for (int q = tid; q < nm; q += nth) {
+        const double nu = s.dv[s.perm[q]];
+        frow[q] = nu < thr ? -1.0 / nu : CUDART_INF;
+      }
+      if (mo) {
+        for (int64_t i = tid; i < (int64_t)nm * N; i += nth) mo[i] = 0.0;
+        __syncthreads();
+        for (int idx = tid; idx < nm * n; idx += nth) {
+          const int q = idx / n, r = idx - q * n;
+          const int col = s.perm[q];
+          if (s.dv[col] < thr) mo[(int64_t)q * N + a.free_ref[r]] = s.sg[q] * Z[r * P + col];
+        }
+      }
+    } else {                                   // failed system: zero outputs, never NaN
+      for (int q = tid; q < nm; q += nth) frow[q] = 0.0;
+      if (mo)
+        for (int64_t i = tid; i < (int64_t)nm * N; i += nth) mo[i] = 0.0;
+    }
+    if (tid == 0) a.info[b] = status;
+  }
+}
+
 
 // ---- ragged batches (tb_modes_ragged): one CTA per truss, every truss with its own topology
 // Only step 1 differs from k_modes: the static solve's guards on the truss, its free-DOF list (ascending DOF, the
@@ -638,13 +759,16 @@ __global__ void __launch_bounds__(160, 1) k_modes_ragged(const ModesRagArgs a) {
 }
 
 // CTA size and residency depend on the free-DOF bound n only: cached per device and n (the occupancy query costs more
-// than the launch).  RAG: k_modes_ragged, else k_modes.
-template <int DIM, bool RAG>
+// than the launch).  KERN: which kernel (MODES_PLAN k_modes, MODES_RAGGED k_modes_ragged, MODES_BUCKLING k_buckling).
+enum { MODES_PLAN, MODES_RAGGED, MODES_BUCKLING };
+
+template <int DIM, int KERN>
 int modes_config(int n, int* threads, int* smem, int* per_sm) {
   static int cache[64][TB_SMALL_MAX_DOF + 1];
   static int attr[64];   // the kernel's dynamic shared-memory limit set so far (only ever raised)
   static std::mutex mu;
-  const void* kern = RAG ? (const void*)k_modes_ragged<DIM> : (const void*)k_modes<DIM>;
+  const void* kern = KERN == MODES_RAGGED ? (const void*)k_modes_ragged<DIM>
+                     : KERN == MODES_BUCKLING ? (const void*)k_buckling<DIM> : (const void*)k_modes<DIM>;
   int dev = 0;
   TB_CUDA(cudaGetDevice(&dev));
   *threads = ((n < 32 ? 32 : n) + 31) / 32 * 32;
@@ -904,18 +1028,33 @@ int sens_grid(const void* kern, int batch, int* grid) {
 
 int tb_modes_config(int dim, int n, int* threads, int* smem, int* per_sm) {
   if (n < 1 || n > TB_SMALL_MAX_DOF) return (int)cudaErrorInvalidValue;
-  return dim == 3 ? modes_config<3, false>(n, threads, smem, per_sm) : modes_config<2, false>(n, threads, smem, per_sm);
+  return dim == 3 ? modes_config<3, MODES_PLAN>(n, threads, smem, per_sm) : modes_config<2, MODES_PLAN>(n, threads, smem, per_sm);
 }
 
 int tb_modes_ragged_config(int dim, int bound, int* threads, int* smem, int* per_sm) {
   if (bound < 1 || bound > TB_SMALL_MAX_DOF) return (int)cudaErrorInvalidValue;
-  return dim == 3 ? modes_config<3, true>(bound, threads, smem, per_sm) : modes_config<2, true>(bound, threads, smem, per_sm);
+  return dim == 3 ? modes_config<3, MODES_RAGGED>(bound, threads, smem, per_sm)
+                  : modes_config<2, MODES_RAGGED>(bound, threads, smem, per_sm);
+}
+
+int tb_buckling_config(int dim, int n, int* threads, int* smem, int* per_sm) {
+  if (n < 1 || n > TB_SMALL_MAX_DOF) return (int)cudaErrorInvalidValue;
+  return dim == 3 ? modes_config<3, MODES_BUCKLING>(n, threads, smem, per_sm)
+                  : modes_config<2, MODES_BUCKLING>(n, threads, smem, per_sm);
 }
 
 int tb_launch_modes(const ModesArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st) {
   if (a.batch <= 0) return 0;
   if (dim == 3) k_modes<3><<<grid, threads, smem, st>>>(a);
   else k_modes<2><<<grid, threads, smem, st>>>(a);
+  tb_count_launch();
+  return (int)cudaGetLastError();
+}
+
+int tb_launch_buckling(const BucklingArgs& a, int dim, int grid, int threads, int smem, cudaStream_t st) {
+  if (a.base.batch <= 0) return 0;
+  if (dim == 3) k_buckling<3><<<grid, threads, smem, st>>>(a);
+  else k_buckling<2><<<grid, threads, smem, st>>>(a);
   tb_count_launch();
   return (int)cudaGetLastError();
 }

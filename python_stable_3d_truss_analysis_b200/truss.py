@@ -169,10 +169,12 @@ class Truss:
         self._displace = self._external = self._internal = None
         self._solved = False
         self._modes = None                      # dict(eigval [k], modes [k, N]) of SolveModes()
+        self._buckling = None                   # dict(factor [k], modes [k, N]) of SolveBuckling()
 
     def _topology_changed(self):
         self._plan = None
         self._modes = None
+        self._buckling = None
 
     def _pack(self):
         """Flat arrays in the layout of include/truss_b200.h."""
@@ -275,6 +277,7 @@ class Truss:
             raise InvaildJointError(f"No such joint [{jointID}], can't add force on it.")
         if not IsZeroVector(vector):
             self._forces[jointID] = tuple(float(vector[i]) for i in range(self._dim))
+            self._buckling = None                   # (the buckling factors are those of the loads)
 
     def AddNewMember(self, jointID0, jointID1, memberType):
         member = Member(self._joints[jointID0][0], self._joints[jointID1][0], self._dim, memberType.Copy())
@@ -284,6 +287,7 @@ class Truss:
     def SetJointPosition(self, jointID, position):
         self._joints[jointID] = (position, self._joints[jointID][1])
         self._modes = None
+        self._buckling = None
         for j0, j1, member in self._members.values():
             if j0 == jointID: member.SetPosition(0, position)
             if j1 == jointID: member.SetPosition(1, position)
@@ -303,6 +307,7 @@ class Truss:
     def SetMemberType(self, memberID, memberType):
         self._members[memberID][2].memberType = memberType
         self._modes = None
+        self._buckling = None
 
     def SetMemberTypes(self, memberTypeDict, isCheckAllSet=False):
         if isCheckAllSet and self._members.keys() - memberTypeDict.keys():
@@ -471,6 +476,41 @@ class Truss:
         """One dict per mode, {jointID: displacement vector} over every joint (zero at supported DOFs), in the style of
         GetDisplacements; M-normalised, the component of largest magnitude positive."""
         modes = self._modes_or_raise()["modes"]
+        d = self._dim
+        return [{j: modes[k, j * d:(j + 1) * d].copy() for j in range(self.nJoint)} for k in range(modes.shape[0])]
+
+    # ------------------------------------------------------------------ linear buckling
+    def SolveBuckling(self, nMode=None):
+        """Linear buckling under the current loads on the GPU: the static solve (as ``Solve``, raising as it does), then
+        K_ff phi = lambda (-K_G) phi with the geometric stiffness of its member forces (tb_buckling, batch of one).  The
+        ``nMode`` lowest load factors (None = one per free DOF): the loads times ``GetBucklingFactors()[0]`` make the
+        truss unstable.  Modes no positive multiple of the loads reaches get an ``inf`` factor (e.g. every mode of a truss
+        without compressed members).  The static results are not stored (call ``Solve`` for those)."""
+        if not self.isStable:
+            raise TrussNotStableError("The truss is not stable !")
+        xyz, support, conn, aed, force = self._pack()
+        plan = self._get_plan(support, conn)
+        out = plan.solve_host(1, xyz, force, aed=aed, want=("axial",))
+        raise_for_info(int(out["info"][0]))
+        res = plan.buckling_host(1, xyz, out["axial"][0], aed=aed, n_modes=nMode)
+        raise_for_modes_info(int(res["info"][0]))
+        self._buckling = {"factor": res["factor"][0].copy(), "modes": res["modes"][0].copy()}
+
+    def _buckling_or_raise(self):
+        if self._buckling is None:
+            raise TrussNotSolvedError("Haven't done buckling analysis yet (SolveBuckling).")
+        return self._buckling
+
+    def GetBucklingFactors(self):
+        """Load factors of the solved buckling modes, ascending (numpy array; inf for modes no positive multiple of the
+        loads reaches).  The first one is the critical load factor."""
+        return self._buckling_or_raise()["factor"].copy()
+
+    def GetBucklingModes(self):
+        """One dict per buckling mode, {jointID: displacement vector} over every joint (zero at supported DOFs), in the
+        style of GetModeShapes; K-normalised (phi^T K_ff phi = 1), the component of largest magnitude positive, all zero
+        for a mode with an inf factor."""
+        modes = self._buckling_or_raise()["modes"]
         d = self._dim
         return [{j: modes[k, j * d:(j + 1) * d].copy() for j in range(self.nJoint)} for k in range(modes.shape[0])]
 
