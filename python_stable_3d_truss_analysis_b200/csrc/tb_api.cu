@@ -40,6 +40,68 @@ int check_batch_in(const tb_plan* p, const tb_batch_in* in) {
   return TB_OK;
 }
 
+// ---- grow-only device buffers ----------------------------------------------------------------------------------------
+// Grown after the whole device is idle (the workspace, the compact temporaries, the staging arenas), to need + slack bytes
+int reserve_sync(DevBuf& b, size_t need, size_t slack) {
+  if (b.bytes >= need) return TB_OK;
+  if (b.ptr) {
+    TB_CUDA(cudaDeviceSynchronize());
+    TB_CUDA(cudaFree(b.ptr));
+    b = DevBuf();
+  }
+  TB_CUDA(cudaMalloc(&b.ptr, need + slack));
+  b.bytes = need + slack;
+  return TB_OK;
+}
+
+// the staging arenas of the *_host calls: 4 KB of margin, and an eighth more when they grow
+int reserve_stage(DevBuf& b, size_t need) { return reserve_sync(b, need + 4096, (need + 4096) / 8); }
+
+// Grown stream-ordered on `st` (the scratch of tb_adjoint, the modal and the envelope kernels): the previous call's
+// kernels are ahead on st, StreamOrder::acquire put them there
+int reserve_async(DevBuf& b, size_t need, cudaStream_t st) {
+  if (b.bytes >= need) return TB_OK;
+  if (b.ptr) TB_CUDA(cudaFreeAsync(b.ptr, st));
+  b = DevBuf();
+  TB_CUDA(cudaMallocAsync(&b.ptr, need, st));
+  b.bytes = need;
+  return TB_OK;
+}
+
+bool capturing(cudaStream_t st) {
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
+  return cap != cudaStreamCaptureStatusNone;
+}
+
+}  // namespace
+
+// The previous call's kernels may still be running on another stream.  A captured step is single-stream by contract.
+int StreamOrder::acquire(cudaStream_t st) {
+  if (!capturing(st) && used && last != st && ev) TB_CUDA(cudaStreamWaitEvent(st, ev, 0));
+  return TB_OK;
+}
+int StreamOrder::release(cudaStream_t st) {
+  if (capturing(st)) return TB_OK;
+  if (!ev) TB_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+  TB_CUDA(cudaEventRecord(ev, st));
+  last = st;
+  used = true;
+  return TB_OK;
+}
+
+namespace {
+
+// Scratch of a call on `st` that kernels of earlier calls on other streams may still use: waits for them (ord), then grows
+// stream-ordered; the caller launches, then ord.release.  Inside a stream capture it is never grown: TB_ERR_ALLOC with
+// nothing enqueued (a warm-up call outside the capture grows it).
+int acquire_scratch(StreamOrder& ord, DevBuf& buf, size_t need, cudaStream_t st) {
+  if (buf.bytes < need && capturing(st)) return TB_ERR_ALLOC;
+  const int rc = ord.acquire(st);
+  if (rc) return rc;
+  return reserve_async(buf, need, st);
+}
+
 // Compact outputs (tb_batch_out.u_free / react): gathered from the dense rows of the same systems
 __global__ void __launch_bounds__(256) k_compact_out(const double* __restrict__ u, const double* __restrict__ ext,
                                                       double* __restrict__ u_free, double* __restrict__ react,
@@ -54,29 +116,14 @@ __global__ void __launch_bounds__(256) k_compact_out(const double* __restrict__ 
 }
 
 // dense temporaries of a call that wants the compact outputs without the dense ones (call before the ranges are enqueued)
-int ensure_compact_tmp(tb_plan* p, const tb_batch_out* out, int batch, cudaStream_t st) {
+int ensure_compact_tmp(tb_plan* p, const tb_batch_out* out, int batch) {
   if (!out || p->path != 0) return TB_OK;      // (the blocked pipelines' recovery kernel writes the compact outputs itself)
-  auto grow = [&](double** buf, size_t* cap) -> int {
-    if (*cap >= (size_t)batch) return TB_OK;
-    if (*buf) {
-      TB_CUDA(cudaStreamSynchronize(st));
-      TB_CUDA(cudaDeviceSynchronize());
-      TB_CUDA(cudaFree(*buf));
-      *buf = nullptr;
-      *cap = 0;
-    }
-    TB_CUDA(cudaMalloc((void**)buf, (size_t)batch * p->N * sizeof(double)));
-    *cap = (size_t)batch;
-    return TB_OK;
-  };
+  const size_t bytes = (size_t)batch * p->N * sizeof(double);
   if (out->u_free && !out->u) {
-    const int rc = grow(&p->compact_u, &p->compact_cap_u);
+    const int rc = reserve_sync(p->compact_u, bytes, 0);
     if (rc) return rc;
   }
-  if (out->react && !out->ext) {
-    const int rc = grow(&p->compact_ext, &p->compact_cap_ext);
-    if (rc) return rc;
-  }
+  if (out->react && !out->ext) return reserve_sync(p->compact_ext, bytes, 0);
   return TB_OK;
 }
 
@@ -89,8 +136,8 @@ int run_plan_range(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out, c
   if (!out->u_free && !out->react) return run_plan_range_dense(p, in, out, fit, allow_s, allow_d, st, b0, nb, ws, shared_k);
   if (p->path != 0) return run_plan_range_dense(p, in, out, fit, allow_s, allow_d, st, b0, nb, ws, shared_k);   // the recovery kernel writes them itself
   tb_batch_out eff = *out;
-  if (out->u_free && !eff.u) eff.u = p->compact_u;          // (ensure_compact_tmp sized them for the whole batch)
-  if (out->react && !eff.ext) eff.ext = p->compact_ext;
+  if (out->u_free && !eff.u) eff.u = (double*)p->compact_u.ptr;          // (ensure_compact_tmp sized them for the whole batch)
+  if (out->react && !eff.ext) eff.ext = (double*)p->compact_ext.ptr;
   if ((out->u_free && !eff.u) || (out->react && !eff.ext)) return TB_ERR_ALLOC;
   const int rc = run_plan_range_dense(p, in, &eff, fit, allow_s, allow_d, st, b0, nb, ws, shared_k);
   if (rc) return rc;
@@ -223,44 +270,11 @@ size_t plan_ws_bytes(const tb_plan* p, int batch) {
   return need;
 }
 
-int ensure_ws(tb_plan* p, size_t need, cudaStream_t st) {
-  if (p->ws_bytes >= need) return TB_OK;
-  if (p->ws) {
-    TB_CUDA(cudaStreamSynchronize(st));
-    TB_CUDA(cudaDeviceSynchronize());
-    TB_CUDA(cudaFree(p->ws));
-    p->ws = nullptr;
-    p->ws_bytes = 0;
-  }
-  TB_CUDA(cudaMalloc(&p->ws, need));
-  p->ws_bytes = need;
-  return TB_OK;
-}
-
 // The plan belongs to the device it was created on (its maps and workspace live there)
 int check_device(const tb_plan* p) {
   int dev = -1;
   if (cudaGetDevice(&dev) != cudaSuccess) return TB_ERR_NO_DEVICE;
   return dev == p->device ? TB_OK : TB_ERR_WRONG_DEVICE;
-}
-
-// Workspace ordering across streams: the previous call's kernels may still be running on another stream
-int ws_acquire(tb_plan* p, cudaStream_t st) {
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
-  if (cap != cudaStreamCaptureStatusNone) return TB_OK;          // a captured step is single-stream by contract
-  if (p->ws_used && p->ws_stream != st && p->ws_event) TB_CUDA(cudaStreamWaitEvent(st, p->ws_event, 0));
-  return TB_OK;
-}
-int ws_release(tb_plan* p, cudaStream_t st) {
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
-  if (cap != cudaStreamCaptureStatusNone) return TB_OK;
-  if (!p->ws_event) TB_CUDA(cudaEventCreateWithFlags(&p->ws_event, cudaEventDisableTiming));
-  TB_CUDA(cudaEventRecord(p->ws_event, st));
-  p->ws_stream = st;
-  p->ws_used = true;
-  return TB_OK;
 }
 
 int run_plan_unlocked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out, const tb_fit_out* fit, double allow_s,
@@ -273,11 +287,11 @@ int run_plan(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out, const t
   if (rc) return rc;
   std::lock_guard<std::mutex> lock(p->mu);
   if (p->path != 0) {
-    rc = ws_acquire(p, st);
+    rc = p->ws_order.acquire(st);
     if (rc) return rc;
   }
   rc = run_plan_unlocked(p, in, out, fit, allow_s, allow_d, st, shared_k);
-  if (!rc && p->path != 0) rc = ws_release(p, st);
+  if (!rc && p->path != 0) rc = p->ws_order.release(st);
   return rc;
 }
 
@@ -286,7 +300,7 @@ int run_plan_unlocked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out
   static const tb_batch_out none = {nullptr, nullptr, nullptr, nullptr, nullptr};
   if (!out) out = &none;
   {
-    const int rc0 = ensure_compact_tmp(p, out, in->batch, st);
+    const int rc0 = ensure_compact_tmp(p, out, in->batch);
     if (rc0) return rc0;
   }
   if (p->path == 0) {
@@ -296,10 +310,10 @@ int run_plan_unlocked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out
     // blocked paths: process the batch in chunks that fit the workspace cap
     const size_t per_sys = plan_ws_bytes(p, 1);
     int chunk = (int)std::min<size_t>((size_t)in->batch, std::max<size_t>(1, ws_cap_bytes() / per_sys));
-    int rc = ensure_ws(p, plan_ws_bytes(p, chunk), st);
+    int rc = reserve_sync(p->ws, plan_ws_bytes(p, chunk), 0);
     if (rc) return rc;
     for (int b0 = 0; b0 < in->batch; b0 += chunk) {
-      rc = run_plan_range(p, in, out, fit, allow_s, allow_d, st, b0, std::min(chunk, in->batch - b0), p->ws, shared_k);
+      rc = run_plan_range(p, in, out, fit, allow_s, allow_d, st, b0, std::min(chunk, in->batch - b0), p->ws.ptr, shared_k);
       if (rc) return rc;
     }
   }
@@ -309,28 +323,15 @@ int run_plan_unlocked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out
   return TB_OK;
 }
 
-// ---- bump allocator over a grow-only device arena -------------------------------------------
+// ---- bump allocation over a grow-only device arena: 256-byte aligned pieces ------------------------------------------
 struct Arena {
-  void** base;
-  size_t* cap;
-  size_t used = 0;
-  Arena(void** b, size_t* c) : base(b), cap(c) {}
   static size_t al(size_t x) { return (x + 255) & ~(size_t)255; }
-};
-
-int arena_reserve(void** base, size_t* cap, size_t need) {
-  if (*cap >= need) return 0;
-  if (*base) {
-    TB_CUDA(cudaDeviceSynchronize());
-    TB_CUDA(cudaFree(*base));
-    *base = nullptr;
-    *cap = 0;
+  static size_t sum(std::initializer_list<size_t> bytes) {
+    size_t s = 0;
+    for (size_t b : bytes) s += al(b);
+    return s;
   }
-  need += need / 8;
-  TB_CUDA(cudaMalloc(base, need));
-  *cap = need;
-  return 0;
-}
+};
 
 template <typename Tp>
 Tp* take(char*& cur, size_t count) {
@@ -379,6 +380,24 @@ void host_pipe_drain(HostPipe* hp) {           // after an error: nothing of the
   (void)cudaGetLastError();
 }
 int stride_ok(int64_t stride, int64_t row) { return stride == 0 || stride == row; }
+size_t rows(int64_t stride, int64_t row, int B) { return (size_t)(stride == 0 ? row : row * B); }   // elements to stage
+
+// The strides of a uniform batch's geometry and member inputs on the host: 0 (shared by the batch) or one system's row
+int check_in_strides(const tb_plan* p, const tb_batch_in* in) {
+  if (!stride_ok(in->joint_stride, (int64_t)p->nJ * p->dim)) return TB_ERR_SIZE;
+  if (in->member_aed ? !stride_ok(in->member_stride, (int64_t)p->M * 3) : !stride_ok(in->gene_stride, p->M)) return TB_ERR_SIZE;
+  return TB_OK;
+}
+
+// Elements of those inputs to stage
+struct InCounts {
+  size_t xyz, aed, gene, tab;
+  InCounts(const tb_plan* p, const tb_batch_in* in)
+      : xyz(rows(in->joint_stride, (int64_t)p->nJ * p->dim, in->batch)),
+        aed(in->member_aed ? rows(in->member_stride, (int64_t)p->M * 3, in->batch) : 0),
+        gene(in->member_aed ? 0 : rows(in->gene_stride, p->M, in->batch)),
+        tab(in->member_aed ? 0 : (size_t)in->n_type * 3) {}
+};
 
 int run_plan_host_locked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out, const tb_fit_out* fit, double allow_s,
                          double allow_d, int shared_k, HostPipe* hp, int async_slot = -1);
@@ -392,28 +411,66 @@ int async_drain(tb_plan* p) {
   return TB_OK;
 }
 
-// Host entry points: serialised per process (g_pipe_mu: helper streams, events) and per plan (p->mu: staging arena,
-// workspace); on an error the helper streams are drained before the code is returned.
+// The blocking host entry points run body(hp): serialised per process (g_pipe_mu: helper streams, events, the ragged
+// arenas) and per plan (p->mu: staging arena, workspace), after every pipelined call of the plan (they share the compute
+// stream and the workspace); on an error the helper streams are drained before the code is returned, so nothing of the
+// call may still be copying into the caller's buffers.  p: null for the ragged calls.
+template <class F>
+int host_call(tb_plan* p, F body) {
+  std::lock_guard<std::mutex> pipe_lock(g_pipe_mu);
+  std::unique_lock<std::mutex> plan_lock;
+  if (p) plan_lock = std::unique_lock<std::mutex>(p->mu);
+  HostPipe* hp = host_pipe();
+  if (!hp) return TB_ERR_ALLOC;
+  int rc = p ? async_drain(p) : TB_OK;
+  if (rc) return rc;
+  rc = body(hp);
+  if (rc) host_pipe_drain(hp);
+  return rc;
+}
+
+// Stages a uniform batch's geometry and member inputs (strides checked) at the start of the plan's staging arena, grown
+// to hold `extra` bytes more, with plain copies on `st`.  *din: the device-side batch (no load); *cur: the arena past them.
+int stage_in(tb_plan* p, const tb_batch_in* in, size_t extra, cudaStream_t st, tb_batch_in* din, char** cur) {
+  const InCounts c(p, in);
+  const int rc = reserve_stage(p->stage_dev, Arena::sum({c.xyz * 8, c.aed * 8, c.gene * 4, c.tab * 8}) + extra);
+  if (rc) return rc;
+  *cur = (char*)p->stage_dev.ptr;
+  *din = *in;
+  din->force = nullptr;
+  double* dxyz = take<double>(*cur, c.xyz);
+  TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, c.xyz * 8, cudaMemcpyHostToDevice, st));
+  din->joint_xyz = dxyz;
+  if (in->member_aed) {
+    double* daed = take<double>(*cur, c.aed);
+    TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, c.aed * 8, cudaMemcpyHostToDevice, st));
+    din->member_aed = daed;
+    din->gene = nullptr;
+  } else {
+    int32_t* dgene = take<int32_t>(*cur, c.gene);
+    double* dtab = take<double>(*cur, c.tab);
+    TB_CUDA(cudaMemcpyAsync(dgene, in->gene, c.gene * 4, cudaMemcpyHostToDevice, st));
+    TB_CUDA(cudaMemcpyAsync(dtab, in->type_table, c.tab * 8, cudaMemcpyHostToDevice, st));
+    din->gene = dgene;
+    din->type_table = dtab;
+  }
+  return TB_OK;
+}
+
 int run_plan_host(tb_plan* p, const tb_batch_in* in, const tb_batch_out* out, const tb_fit_out* fit, double allow_s,
                   double allow_d, int shared_k = 0) {
   int rc = check_batch_in(p, in);
   if (rc) return rc;
   rc = check_device(p);
   if (rc) return rc;
-  std::lock_guard<std::mutex> pipe_lock(g_pipe_mu);
-  std::lock_guard<std::mutex> plan_lock(p->mu);
-  HostPipe* hp = host_pipe();
-  if (!hp) return TB_ERR_ALLOC;
-  rc = async_drain(p);                          // (the blocking calls share the compute stream and the workspace with the pipelined ones)
-  if (rc) return rc;
-  if (p->path != 0) {
-    rc = ws_acquire(p, hp->comp);
-    if (rc) return rc;
-  }
-  rc = run_plan_host_locked(p, in, out, fit, allow_s, allow_d, shared_k, hp);
-  if (rc) host_pipe_drain(hp);
-  else if (p->path != 0) rc = ws_release(p, hp->comp);
-  return rc;
+  return host_call(p, [&](HostPipe* hp) -> int {
+    if (p->path != 0) {
+      const int r2 = p->ws_order.acquire(hp->comp);
+      if (r2) return r2;
+    }
+    const int r2 = run_plan_host_locked(p, in, out, fit, allow_s, allow_d, shared_k, hp);
+    return r2 || p->path == 0 ? r2 : p->ws_order.release(hp->comp);
+  });
 }
 
 // Pipelined host call: enqueue H2D (stream ain) -> kernels (comp) -> D2H (aout) and return; consecutive calls use the
@@ -436,7 +493,7 @@ int run_plan_host_async(tb_plan* p, const tb_batch_in* in, const tb_batch_out* o
   for (cudaEvent_t* e : {&p->async_in[slot], &p->async_k[slot], &p->async_done[slot]})
     if (!*e) TB_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
   if (p->path != 0) {
-    rc = ws_acquire(p, hp->comp);
+    rc = p->ws_order.acquire(hp->comp);
     if (rc) return rc;
   }
   rc = in->batch == 0 ? TB_OK : run_plan_host_locked(p, in, out, nullptr, 0.0, 0.0, 0, hp, slot);
@@ -445,7 +502,7 @@ int run_plan_host_async(tb_plan* p, const tb_batch_in* in, const tb_batch_out* o
     p->async_completed = p->async_submitted;
     return rc;
   }
-  if (p->path != 0) rc = ws_release(p, hp->comp);
+  if (p->path != 0) rc = p->ws_order.release(hp->comp);
   TB_CUDA(cudaEventRecord(p->async_done[slot], hp->aout));
   if (ticket) *ticket = p->async_submitted;
   p->async_submitted++;
@@ -459,37 +516,29 @@ int run_plan_host_locked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* 
   const int B = in->batch;
   if (B == 0) return TB_OK;
   const int64_t rowJ = (int64_t)p->nJ * p->dim, rowM3 = (int64_t)p->M * 3, rowM = p->M, rowN = p->N;
-  if (!stride_ok(in->joint_stride, rowJ) || !stride_ok(in->force_stride, rowN)) return TB_ERR_SIZE;
-  if (in->member_aed && !stride_ok(in->member_stride, rowM3)) return TB_ERR_SIZE;
-  if (!in->member_aed && !stride_ok(in->gene_stride, rowM)) return TB_ERR_SIZE;
-  auto cnt = [&](int64_t stride, int64_t row) { return (size_t)(stride == 0 ? row : row * B); };
-  const size_t nxyz = cnt(in->joint_stride, rowJ), nf = cnt(in->force_stride, rowN);
-  const size_t naed = in->member_aed ? cnt(in->member_stride, rowM3) : 0;
-  const size_t ngene = in->member_aed ? 0 : cnt(in->gene_stride, rowM);
-  const size_t ntab = in->member_aed ? 0 : (size_t)in->n_type * 3;
+  if (check_in_strides(p, in) || !stride_ok(in->force_stride, rowN)) return TB_ERR_SIZE;
+  const InCounts c(p, in);
+  const size_t nf = rows(in->force_stride, rowN, B);
   static const tb_batch_out none = {nullptr, nullptr, nullptr, nullptr, nullptr};
   if (!out) out = &none;
 
-  size_t need = 0;
-  auto add = [&](size_t bytes) { need += Arena::al(bytes); };
-  add(nxyz * 8); add(nf * 8); add(naed * 8); add(ngene * 4); add(ntab * 8);
-  add(out->u ? (size_t)B * rowN * 8 : 0); add(out->ext ? (size_t)B * rowN * 8 : 0);
-  add(out->axial ? (size_t)B * rowM * 8 : 0); add(out->weight ? (size_t)B * 8 : 0);
-  add((size_t)B * 4); add(fit ? (size_t)B * 8 : 0); add(fit ? (size_t)B * 2 : 0);
-  add(out->u_free ? (size_t)B * p->n * 8 : 0); add(out->react ? (size_t)B * p->s * 8 : 0);
-  void** arena = async ? &p->stage_async[async_slot] : &p->stage_dev;
-  size_t* arena_bytes = async ? &p->stage_async_bytes[async_slot] : &p->stage_dev_bytes;
-  rc = arena_reserve(arena, arena_bytes, need + 4096);
+  const size_t need = Arena::sum({c.xyz * 8, nf * 8, c.aed * 8, c.gene * 4, c.tab * 8,
+                                  out->u ? (size_t)B * rowN * 8 : 0, out->ext ? (size_t)B * rowN * 8 : 0,
+                                  out->axial ? (size_t)B * rowM * 8 : 0, out->weight ? (size_t)B * 8 : 0,
+                                  (size_t)B * 4, fit ? (size_t)B * 8 : 0, fit ? (size_t)B * 2 : 0,
+                                  out->u_free ? (size_t)B * p->n * 8 : 0, out->react ? (size_t)B * p->s * 8 : 0});
+  DevBuf& arena = async ? p->stage_async[async_slot] : p->stage_dev;
+  rc = reserve_stage(arena, need);
   if (rc) return rc;
 
   cudaStream_t st = hp->comp;
-  char* cur = (char*)*arena;
+  char* cur = (char*)arena.ptr;
   tb_batch_in din = *in;
-  double* dxyz = take<double>(cur, nxyz);
+  double* dxyz = take<double>(cur, c.xyz);
   double* df = take<double>(cur, nf);
-  double* daed = take<double>(cur, naed);
-  int32_t* dgene = take<int32_t>(cur, ngene);
-  double* dtab = take<double>(cur, ntab);
+  double* daed = take<double>(cur, c.aed);
+  int32_t* dgene = take<int32_t>(cur, c.gene);
+  double* dtab = take<double>(cur, c.tab);
   din.joint_xyz = dxyz;
   din.force = df;
   if (in->member_aed) {
@@ -507,7 +556,7 @@ int run_plan_host_locked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* 
   dout.info = take<int32_t>(cur, (size_t)B);
   dout.u_free = out->u_free ? take<double>(cur, (size_t)B * p->n) : nullptr;
   dout.react = out->react ? take<double>(cur, (size_t)B * p->s) : nullptr;
-  rc = ensure_compact_tmp(p, &dout, B, hp->comp);
+  rc = ensure_compact_tmp(p, &dout, B);
   if (rc) return rc;
   tb_fit_out dfit = {nullptr, nullptr, nullptr};
   if (fit) {
@@ -549,7 +598,7 @@ int run_plan_host_locked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* 
   int csz = 0;
   for (int j = 0; j < nch; ++j) csz = std::max(csz, cb[j + 1] - cb[j]);
   if (p->path != 0 && nch > 1) {
-    rc = ensure_ws(p, per_sys * (size_t)csz + 4096, st);       // chunks run one after the other: one workspace slice
+    rc = reserve_sync(p->ws, per_sys * (size_t)csz + 4096, 0);   // chunks run one after the other: one workspace slice
     if (rc) return rc;
   }
   cudaStream_t comp = st;                      // compute stream
@@ -561,13 +610,13 @@ int run_plan_host_locked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* 
   const bool sx = in->joint_stride == 0, sf = in->force_stride == 0;
   const bool sm_ = in->member_aed ? in->member_stride == 0 : in->gene_stride == 0;
   // shared inputs first, on the compute stream
-  if (sx) TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, nxyz * 8, cudaMemcpyHostToDevice, cin));
+  if (sx) TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, c.xyz * 8, cudaMemcpyHostToDevice, cin));
   if (sf) TB_CUDA(cudaMemcpyAsync(df, in->force, nf * 8, cudaMemcpyHostToDevice, cin));
   if (in->member_aed) {
-    if (sm_) TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, naed * 8, cudaMemcpyHostToDevice, cin));
+    if (sm_) TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, c.aed * 8, cudaMemcpyHostToDevice, cin));
   } else {
-    if (sm_) TB_CUDA(cudaMemcpyAsync(dgene, in->gene, ngene * 4, cudaMemcpyHostToDevice, cin));
-    TB_CUDA(cudaMemcpyAsync(dtab, in->type_table, ntab * 8, cudaMemcpyHostToDevice, cin));
+    if (sm_) TB_CUDA(cudaMemcpyAsync(dgene, in->gene, c.gene * 4, cudaMemcpyHostToDevice, cin));
+    TB_CUDA(cudaMemcpyAsync(dtab, in->type_table, c.tab * 8, cudaMemcpyHostToDevice, cin));
   }
   for (int j = 0; j < nch; ++j) {              // every chunk's inputs are queued at once, each on its copy stream
     const int b0 = cb[j], nb = cb[j + 1] - cb[j];
@@ -594,7 +643,7 @@ int run_plan_host_locked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* 
     if (nch == 1 && p->path != 0) {
       rc = run_plan_unlocked(p, &din, &dout, fit ? &dfit : nullptr, allow_s, allow_d, comp, shared_k);   // handles the workspace cap itself
     } else {
-      rc = run_plan_range(p, &din, &dout, fit ? &dfit : nullptr, allow_s, allow_d, comp, b0, nb, p->ws, shared_k);
+      rc = run_plan_range(p, &din, &dout, fit ? &dfit : nullptr, allow_s, allow_d, comp, b0, nb, p->ws.ptr, shared_k);
     }
     if (rc) return rc;
     if (nch > 1) {
@@ -625,14 +674,32 @@ int run_plan_host_locked(tb_plan* p, const tb_batch_in* in, const tb_batch_out* 
   return TB_OK;
 }
 
-int check_ragged(const tb_ragged_in* in) {
+bool ragged_fits_fused(const tb_ragged_in* in) {
+  return tb_small_fits(in->dim, in->max_joint, in->max_member, in->max_joint * in->dim);
+}
+
+// the launch's free-DOF bound of a modal ragged call: max_free, or every DOF of the largest truss up to the kernel's limit
+int modes_ragged_bound(const tb_ragged_in* in, const tb_modes_ragged_in* m) {
+  return m->max_free ? m->max_free : std::min(in->dim * in->max_joint, TB_SMALL_MAX_DOF);
+}
+
+// Argument checks of the ragged entry points, in this order: the layout and sizes; the modal arguments (m != null);
+// then, for a non-empty batch, the packed arrays (the load too, unless modal) and the size limit: the fused kernels'
+// (`fused`: tb_adjoint_ragged, whose solve runs on them) or the envelope kernel's
+int check_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, bool fused) {
   if (!in) return TB_ERR_NULL;
   if (in->dim != 2 && in->dim != 3) return TB_ERR_DIM;
   if (in->batch < 0 || in->max_joint < 0 || in->max_member < 0) return TB_ERR_SIZE;
+  if (m) {
+    if (m->consistent != 0 && m->consistent != 1) return TB_ERR_SIZE;
+    if (m->max_free < 0 || m->max_free > TB_SMALL_MAX_DOF || m->n_modes < 1) return TB_ERR_SIZE;
+    if (in->batch > 0 && m->n_modes > modes_ragged_bound(in, m)) return TB_ERR_SIZE;
+  }
   if (in->batch == 0) return TB_OK;
-  if (!in->joint_off || !in->member_off || !in->joint_xyz || !in->support || !in->conn || !in->member_aed || !in->force)
+  if (!in->joint_off || !in->member_off || !in->joint_xyz || !in->support || !in->conn || !in->member_aed || (!m && !in->force))
     return TB_ERR_NULL;
-  if (!tb_small_fits(in->dim, in->max_joint, in->max_member, in->max_joint * in->dim)) return TB_ERR_TOO_LARGE;
+  if (fused) return ragged_fits_fused(in) ? TB_OK : TB_ERR_TOO_LARGE;
+  if ((int64_t)in->max_joint * in->dim > TB_RAGGED_MAX_DOF || in->max_member > TB_RAGGED_MAX_MEMBER) return TB_ERR_TOO_LARGE;
   return TB_OK;
 }
 
@@ -658,67 +725,68 @@ int run_ragged(const tb_ragged_in* in, const tb_batch_out* out, cudaStream_t st)
   return tb_launch_small(a, in->dim, st);
 }
 
-// staging arena of the ragged host entry point: one per device (device memory), used under g_pipe_mu
-void* g_rag_dev[TB_MAX_DEVICES] = {};
-size_t g_rag_dev_bytes[TB_MAX_DEVICES] = {};
-
-// Argument checks of the ragged forward entry points: as check_ragged, up to the envelope kernel's limits
-int check_ragged_fwd(const tb_ragged_in* in) {
-  if (!in) return TB_ERR_NULL;
-  if (in->dim != 2 && in->dim != 3) return TB_ERR_DIM;
-  if (in->batch < 0 || in->max_joint < 0 || in->max_member < 0) return TB_ERR_SIZE;
-  if (in->batch == 0) return TB_OK;
-  if (!in->joint_off || !in->member_off || !in->joint_xyz || !in->support || !in->conn || !in->member_aed || !in->force)
-    return TB_ERR_NULL;
-  if ((int64_t)in->max_joint * in->dim > TB_RAGGED_MAX_DOF || in->max_member > TB_RAGGED_MAX_MEMBER) return TB_ERR_TOO_LARGE;
-  return TB_OK;
+// Argument checks of tb_solve_ragged, tb_solve_ragged_env and tb_solve_ragged_host: no compact outputs (they need one n
+// and s for the whole batch), check_ragged's, the outputs, then the device
+int check_ragged_fwd(const tb_ragged_in* in, const tb_batch_out* out) {
+  if (out && (out->u_free || out->react)) return TB_ERR_SIZE;
+  const int rc = check_ragged(in, nullptr, false);
+  if (rc) return rc;
+  if (!out) return TB_ERR_NULL;
+  return have_device() ? TB_OK : TB_ERR_NO_DEVICE;
 }
 
-bool ragged_fits_fused(const tb_ragged_in* in) {
-  return tb_small_fits(in->dim, in->max_joint, in->max_member, in->max_joint * in->dim);
-}
+// staging arena of the ragged host entry points: one per device (device memory), used under g_pipe_mu
+DevBuf g_rag_dev[TB_MAX_DEVICES];
 
-// Scratch of the envelope kernel: one grow-only arena per device (one slot per CTA of the persistent grid), grown
-// stream-ordered on the caller's stream.  `mu` serialises the calls on the device; `ev` orders the arena's use across
-// streams (recorded after a call's kernel; a call on another stream waits for it first).
-struct EnvScratch {
-  std::mutex mu;
-  void* buf = nullptr;
-  size_t bytes = 0;
-  cudaEvent_t ev = nullptr;
-  cudaStream_t last = nullptr;
-  bool used = false;
-};
-EnvScratch g_env[TB_MAX_DEVICES];
-
-// Makes the arena at least `need` bytes for a call on `st`, with S.mu held: it first waits for the previous call when that
-// ran on another stream, then grows stream-ordered (the previous call is ahead on st).  Inside a stream capture the arena
-// is never grown: TB_ERR_ALLOC with nothing enqueued (a warm-up call outside the capture grows it).
-int env_acquire(EnvScratch& S, size_t need, cudaStream_t st, bool* capturing) {
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
-  *capturing = cap != cudaStreamCaptureStatusNone;
-  if (S.bytes < need && *capturing) return TB_ERR_ALLOC;
-  if (!*capturing && S.used && S.last != st && S.ev) TB_CUDA(cudaStreamWaitEvent(st, S.ev, 0));
-  if (S.bytes < need) {
-    if (S.buf) TB_CUDA(cudaFreeAsync(S.buf, st));
-    S.buf = nullptr;
-    S.bytes = 0;
-    TB_CUDA(cudaMallocAsync(&S.buf, need, st));
-    S.bytes = need;
+// The offsets of a ragged batch on the host (the *_host entry points; batch > 0)
+int check_ragged_offsets_host(const tb_ragged_in* in) {
+  if (in->joint_off[0] != 0 || in->member_off[0] != 0) return TB_ERR_SIZE;
+  for (int b = 0; b < in->batch; ++b) {
+    const int64_t nj = in->joint_off[b + 1] - in->joint_off[b], nm = in->member_off[b + 1] - in->member_off[b];
+    if (nj < 0 || nm < 0) return TB_ERR_SIZE;
+    if (nj > in->max_joint || nm > in->max_member) return TB_ERR_TOO_LARGE;
   }
   return TB_OK;
 }
 
-// After the call's last kernel on `st`: later calls on other streams wait for it (outside a capture)
-int env_release(EnvScratch& S, cudaStream_t st, bool capturing) {
-  if (capturing) return TB_OK;
-  if (!S.ev) TB_CUDA(cudaEventCreateWithFlags(&S.ev, cudaEventDisableTiming));
-  TB_CUDA(cudaEventRecord(S.ev, st));
-  S.last = st;
-  S.used = true;
+// Stages the six packed arrays of a ragged batch (offsets checked) at the start of the device's ragged arena, grown to hold
+// `extra` bytes more, with plain copies on `st`.  *din: the device-side batch (no load); *cur: the arena past them.
+int stage_ragged_in(const tb_ragged_in* in, size_t extra, cudaStream_t st, tb_ragged_in* din, char** cur) {
+  const int B = in->batch, d = in->dim;
+  const size_t SJ = (size_t)in->joint_off[B], SM = (size_t)in->member_off[B];
+  int dev = 0;
+  TB_CUDA(cudaGetDevice(&dev));
+  DevBuf& arena = g_rag_dev[dev & (TB_MAX_DEVICES - 1)];
+  const int rc = reserve_stage(arena, Arena::sum({(size_t)(B + 1) * 8, (size_t)(B + 1) * 8, SJ * d * 8, SJ, SM * 8, SM * 24}) + extra);
+  if (rc) return rc;
+  *cur = (char*)arena.ptr;
+  int64_t* djo = take<int64_t>(*cur, B + 1);
+  int64_t* dmo = take<int64_t>(*cur, B + 1);
+  double* dxyz = take<double>(*cur, SJ * d);
+  uint8_t* dsup = take<uint8_t>(*cur, SJ);
+  int32_t* dconn = take<int32_t>(*cur, SM * 2);
+  double* daed = take<double>(*cur, SM * 3);
+  TB_CUDA(cudaMemcpyAsync(djo, in->joint_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
+  TB_CUDA(cudaMemcpyAsync(dmo, in->member_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
+  TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, SJ * d * 8, cudaMemcpyHostToDevice, st));
+  TB_CUDA(cudaMemcpyAsync(dsup, in->support, SJ, cudaMemcpyHostToDevice, st));
+  TB_CUDA(cudaMemcpyAsync(dconn, in->conn, SM * 8, cudaMemcpyHostToDevice, st));
+  TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, SM * 24, cudaMemcpyHostToDevice, st));
+  *din = *in;
+  din->joint_off = djo; din->member_off = dmo; din->joint_xyz = dxyz; din->support = dsup;
+  din->conn = dconn; din->member_aed = daed; din->force = nullptr;
   return TB_OK;
 }
+
+// Scratch of the envelope kernel: one grow-only arena per device (one slot per CTA of the persistent grid), grown
+// stream-ordered on the caller's stream.  `mu` serialises the calls on the device; `order` orders the arena's use across
+// streams.
+struct EnvScratch {
+  std::mutex mu;
+  DevBuf buf;
+  StreamOrder order;
+};
+EnvScratch g_env[TB_MAX_DEVICES];
 
 // Envelope kernel over a batch: every truss (route = false), only the trusses above the fused launch's sizes (route:
 // those run first, in one fused launch of the batch), or the ordering mode (order != null).
@@ -732,8 +800,7 @@ int run_env(const tb_ragged_in* in, const tb_batch_out* out, bool route, int32_t
   int rc = tb_rag_env_config(d, in->max_joint, in->max_member, in->batch, &grid, &smem, &env_smem);
   if (rc) return rc;
   const size_t slot = tb_rag_env_slot_bytes(d, in->max_joint, in->max_member);
-  bool capturing = false;
-  rc = env_acquire(S, slot * (size_t)grid, st, &capturing);
+  rc = acquire_scratch(S.order, S.buf, slot * (size_t)grid, st);
   if (rc) return rc;
   const int rj = d == 3 ? TB_RAGGED_ROUTE_J3 : TB_RAGGED_ROUTE_J2, rm = d == 3 ? TB_RAGGED_ROUTE_M3 : TB_RAGGED_ROUTE_M2;
   if (route) {                                   // the fused kernels first, sized at the routing limits (k_dense16)
@@ -753,12 +820,12 @@ int run_env(const tb_ragged_in* in, const tb_batch_out* out, bool route, int32_t
   if (out) { a.u = out->u; a.ext = out->ext; a.axial = out->axial; a.weight = out->weight; a.info = out->info; }
   a.order = order;
   a.envelope = envelope;
-  a.scratch = S.buf;
+  a.scratch = S.buf.ptr;
   a.slot_bytes = slot;
   a.env_smem = env_smem;
   rc = tb_launch_rag_env(a, grid, smem, st);
   if (rc) return rc;
-  return env_release(S, st, capturing);
+  return S.order.release(st);
 }
 
 // The forward of a ragged batch: today's fused launch when the whole batch fits the fused kernels, else split by truss
@@ -838,27 +905,21 @@ extern "C" int tb_fitness_host(tb_plan* plan, const tb_batch_in* in, double allo
 }
 
 extern "C" int tb_solve_ragged(const tb_ragged_in* in, const tb_batch_out* out, void* cuda_stream) {
-  if (out && (out->u_free || out->react)) return TB_ERR_SIZE;   // (the compact layout needs one n and s for the whole batch)
-  int rc = check_ragged_fwd(in);
+  int rc = check_ragged_fwd(in, out);
   if (rc) return rc;
-  if (!out) return TB_ERR_NULL;
-  if (!have_device()) return TB_ERR_NO_DEVICE;
   if (in->batch == 0) return TB_OK;
   return run_ragged_fwd(in, out, (cudaStream_t)cuda_stream);
 }
 
 extern "C" int tb_solve_ragged_env(const tb_ragged_in* in, const tb_batch_out* out, void* cuda_stream) {
-  if (out && (out->u_free || out->react)) return TB_ERR_SIZE;
-  int rc = check_ragged_fwd(in);
+  int rc = check_ragged_fwd(in, out);
   if (rc) return rc;
-  if (!out) return TB_ERR_NULL;
-  if (!have_device()) return TB_ERR_NO_DEVICE;
   if (in->batch == 0) return TB_OK;
   return run_env(in, out, false, nullptr, nullptr, (cudaStream_t)cuda_stream);
 }
 
 extern "C" int tb_ragged_env_order(const tb_ragged_in* in, int32_t* order, int64_t* envelope, void* cuda_stream) {
-  int rc = check_ragged_fwd(in);
+  int rc = check_ragged(in, nullptr, false);
   if (rc) return rc;
   if (in->batch == 0) return TB_OK;
   if (!order || !envelope) return TB_ERR_NULL;
@@ -875,75 +936,40 @@ extern "C" int tb_ragged_limits(int32_t dim, int32_t* max_joint, int32_t* max_me
 }
 
 extern "C" int tb_solve_ragged_host(const tb_ragged_in* in, const tb_batch_out* out) {
-  if (out && (out->u_free || out->react)) return TB_ERR_SIZE;
-  int rc = check_ragged_fwd(in);
+  int rc = check_ragged_fwd(in, out);
   if (rc) return rc;
-  if (!out) return TB_ERR_NULL;
-  if (!have_device()) return TB_ERR_NO_DEVICE;
   const int B = in->batch, d = in->dim;
   if (B == 0) return TB_OK;
-  // host-side validation of the offsets (they are host pointers here)
-  if (in->joint_off[0] != 0 || in->member_off[0] != 0) return TB_ERR_SIZE;
-  for (int b = 0; b < B; ++b) {
-    const int64_t nj = in->joint_off[b + 1] - in->joint_off[b], nm = in->member_off[b + 1] - in->member_off[b];
-    if (nj < 0 || nm < 0) return TB_ERR_SIZE;
-    if (nj > in->max_joint || nm > in->max_member) return TB_ERR_TOO_LARGE;
-  }
+  rc = check_ragged_offsets_host(in);
+  if (rc) return rc;
   const size_t SJ = (size_t)in->joint_off[B], SM = (size_t)in->member_off[B];
-  std::lock_guard<std::mutex> lock(g_pipe_mu);
-  HostPipe* hp = host_pipe();
-  if (!hp) return TB_ERR_ALLOC;
-  int dev = 0;
-  TB_CUDA(cudaGetDevice(&dev));
-  void*& rag_dev = g_rag_dev[dev & (TB_MAX_DEVICES - 1)];
-  size_t& rag_bytes = g_rag_dev_bytes[dev & (TB_MAX_DEVICES - 1)];
-  auto body = [&]() -> int {
-  size_t need = 0;
-  auto add = [&](size_t bytes) { need += Arena::al(bytes); };
-  add((B + 1) * 8); add((B + 1) * 8); add(SJ * d * 8); add(SJ); add(SM * 8); add(SM * 24); add(SJ * d * 8);
-  add(out->u ? SJ * d * 8 : 0); add(out->ext ? SJ * d * 8 : 0); add(out->axial ? SM * 8 : 0);
-  add(out->weight ? (size_t)B * 8 : 0); add((size_t)B * 4);
-  int rc = arena_reserve(&rag_dev, &rag_bytes, need + 4096);
-  if (rc) return rc;
-  cudaStream_t st = hp->comp;
-  char* cur = (char*)rag_dev;
-  tb_ragged_in din = *in;
-  int64_t* djo = take<int64_t>(cur, B + 1);
-  int64_t* dmo = take<int64_t>(cur, B + 1);
-  double* dxyz = take<double>(cur, SJ * d);
-  uint8_t* dsup = take<uint8_t>(cur, SJ);
-  int32_t* dconn = take<int32_t>(cur, SM * 2);
-  double* daed = take<double>(cur, SM * 3);
-  double* df = take<double>(cur, SJ * d);
-  TB_CUDA(cudaMemcpyAsync(djo, in->joint_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
-  TB_CUDA(cudaMemcpyAsync(dmo, in->member_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
-  TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, SJ * d * 8, cudaMemcpyHostToDevice, st));
-  TB_CUDA(cudaMemcpyAsync(dsup, in->support, SJ, cudaMemcpyHostToDevice, st));
-  TB_CUDA(cudaMemcpyAsync(dconn, in->conn, SM * 8, cudaMemcpyHostToDevice, st));
-  TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, SM * 24, cudaMemcpyHostToDevice, st));
-  TB_CUDA(cudaMemcpyAsync(df, in->force, SJ * d * 8, cudaMemcpyHostToDevice, st));
-  din.joint_off = djo; din.member_off = dmo; din.joint_xyz = dxyz; din.support = dsup;
-  din.conn = dconn; din.member_aed = daed; din.force = df;
-  tb_batch_out dout;
-  dout.u_free = dout.react = nullptr;
-  dout.u = out->u ? take<double>(cur, SJ * d) : nullptr;
-  dout.ext = out->ext ? take<double>(cur, SJ * d) : nullptr;
-  dout.axial = out->axial ? take<double>(cur, SM) : nullptr;
-  dout.weight = out->weight ? take<double>(cur, (size_t)B) : nullptr;
-  dout.info = take<int32_t>(cur, (size_t)B);
-  rc = run_ragged_fwd(&din, &dout, st);
-  if (rc) return rc;
-  if (out->u) TB_CUDA(cudaMemcpyAsync(out->u, dout.u, SJ * d * 8, cudaMemcpyDeviceToHost, st));
-  if (out->ext) TB_CUDA(cudaMemcpyAsync(out->ext, dout.ext, SJ * d * 8, cudaMemcpyDeviceToHost, st));
-  if (out->axial) TB_CUDA(cudaMemcpyAsync(out->axial, dout.axial, SM * 8, cudaMemcpyDeviceToHost, st));
-  if (out->weight) TB_CUDA(cudaMemcpyAsync(out->weight, dout.weight, (size_t)B * 8, cudaMemcpyDeviceToHost, st));
-  if (out->info) TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
-  TB_CUDA(cudaStreamSynchronize(st));
-  return TB_OK;
-  };
-  rc = body();
-  if (rc) host_pipe_drain(hp);                 // nothing of a failed call may still be copying into the caller's buffers
-  return rc;
+  return host_call(nullptr, [&](HostPipe* hp) -> int {
+    cudaStream_t st = hp->comp;
+    tb_ragged_in din;
+    char* cur = nullptr;
+    int r2 = stage_ragged_in(in, Arena::sum({SJ * d * 8, out->u ? SJ * d * 8 : 0, out->ext ? SJ * d * 8 : 0, out->axial ? SM * 8 : 0,
+                                             out->weight ? (size_t)B * 8 : 0, (size_t)B * 4}), st, &din, &cur);
+    if (r2) return r2;
+    double* df = take<double>(cur, SJ * d);
+    TB_CUDA(cudaMemcpyAsync(df, in->force, SJ * d * 8, cudaMemcpyHostToDevice, st));
+    din.force = df;
+    tb_batch_out dout;
+    dout.u_free = dout.react = nullptr;
+    dout.u = out->u ? take<double>(cur, SJ * d) : nullptr;
+    dout.ext = out->ext ? take<double>(cur, SJ * d) : nullptr;
+    dout.axial = out->axial ? take<double>(cur, SM) : nullptr;
+    dout.weight = out->weight ? take<double>(cur, (size_t)B) : nullptr;
+    dout.info = take<int32_t>(cur, (size_t)B);
+    r2 = run_ragged_fwd(&din, &dout, st);
+    if (r2) return r2;
+    if (out->u) TB_CUDA(cudaMemcpyAsync(out->u, dout.u, SJ * d * 8, cudaMemcpyDeviceToHost, st));
+    if (out->ext) TB_CUDA(cudaMemcpyAsync(out->ext, dout.ext, SJ * d * 8, cudaMemcpyDeviceToHost, st));
+    if (out->axial) TB_CUDA(cudaMemcpyAsync(out->axial, dout.axial, SM * 8, cudaMemcpyDeviceToHost, st));
+    if (out->weight) TB_CUDA(cudaMemcpyAsync(out->weight, dout.weight, (size_t)B * 8, cudaMemcpyDeviceToHost, st));
+    if (out->info) TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaStreamSynchronize(st));
+    return TB_OK;
+  });
 }
 
 // Debug export: the K_ff values the device assembles (the band path's program-order lists when the plan has the two-sided
@@ -960,31 +986,21 @@ extern "C" int tb_debug_assemble_host(tb_plan* p, const tb_batch_in* in, double*
   const bool ts = p->ts && p->ts->ok;
   const size_t nnz_map = p->ent_row.size();                      // scatter-map entries (the output's order)
   const size_t nnz = ts ? p->ts->epos.size() : nnz_map;          // device order: the band program's schedule has holes
-  const int64_t rowJ = (int64_t)p->nJ * p->dim, rowM3 = (int64_t)p->M * 3;
-  if (!stride_ok(in->joint_stride, rowJ) || !stride_ok(in->member_stride, rowM3)) return TB_ERR_SIZE;
-  std::lock_guard<std::mutex> pipe_lock(g_pipe_mu);
-  std::lock_guard<std::mutex> plan_lock(p->mu);
-  HostPipe* hp = host_pipe();
-  if (!hp) return TB_ERR_ALLOC;
-  cudaStream_t st = hp->comp;
-  const size_t nxyz = (size_t)(in->joint_stride == 0 ? rowJ : rowJ * B), naed = (size_t)(in->member_stride == 0 ? rowM3 : rowM3 * B);
-  const int nv = p->dim * (p->dim + 1) / 2;
-  double *dxyz = nullptr, *daed = nullptr, *dkv = nullptr, *dscr = nullptr;
-  int32_t* dstat = nullptr;
-  std::vector<double> host((size_t)B * nnz);
-  auto body = [&]() -> int {
-    TB_CUDA(cudaMalloc(&dxyz, nxyz * 8));
-    TB_CUDA(cudaMalloc(&daed, naed * 8));
-    TB_CUDA(cudaMalloc(&dkv, (size_t)B * nnz * 8));
-    TB_CUDA(cudaMalloc(&dscr, (size_t)B * p->M * (2 + p->dim + nv) * 8));     // k_geom arrays (only used for very many members)
-    TB_CUDA(cudaMalloc(&dstat, (size_t)B * 4));
-    TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, nxyz * 8, cudaMemcpyHostToDevice, st));
-    TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, naed * 8, cudaMemcpyHostToDevice, st));
+  rc = check_in_strides(p, in);
+  if (rc) return rc;
+  const size_t nkv = (size_t)B * nnz, nscr = (size_t)B * p->M * (2 + p->dim + p->dim * (p->dim + 1) / 2);
+  std::vector<double> host(nkv);
+  rc = host_call(p, [&](HostPipe* hp) -> int {
+    cudaStream_t st = hp->comp;
+    tb_batch_in din;
+    char* cur = nullptr;
+    int r2 = stage_in(p, in, Arena::sum({nkv * 8, nscr * 8, (size_t)B * 4}), st, &din, &cur);
+    if (r2) return r2;
     LargeArgs a;
     memset(&a, 0, sizeof(a));
     a.batch = B; a.dim = p->dim; a.nJ = p->nJ; a.M = p->M; a.N = p->N; a.n = p->n;
-    a.xyz = dxyz; a.xyz_stride = in->joint_stride;
-    a.aed = daed; a.aed_stride = in->member_stride;
+    a.xyz = din.joint_xyz; a.xyz_stride = in->joint_stride;
+    a.aed = din.member_aed; a.aed_stride = in->member_stride;
     a.conn = p->d_conn;
     a.nnz = (int64_t)nnz;
     a.q_first = ts ? p->ts->d_tq_first : p->d_q_first;
@@ -992,22 +1008,19 @@ extern "C" int tb_debug_assemble_host(tb_plan* p, const tb_batch_in* in, double*
     a.q_ptr = ts ? p->ts->d_tq_ptr : p->d_q_ptr;
     a.q_pack = ts ? p->ts->d_tq_pack : p->d_q_pack;
     a.n_multi = (int)(ts ? p->ts->tq_multi.size() : p->q_multi.size());
-    a.kv = dkv;
-    a.status = dstat;
-    double* q = dscr;
+    a.kv = take<double>(cur, nkv);
+    double* q = take<double>(cur, nscr);     // k_geom arrays (only used for very many members)
+    a.status = take<int32_t>(cur, (size_t)B);
     a.mk = q; q += (size_t)B * p->M;
     a.mc = q; q += (size_t)B * p->M * p->dim;
     a.mw = q; q += (size_t)B * p->M;
     a.mkc = q;
-    int r2 = tb_launch_assemble_only(a, p->num_sm, st);
+    r2 = tb_launch_assemble_only(a, p->num_sm, st);
     if (r2) return r2;
-    TB_CUDA(cudaMemcpyAsync(host.data(), dkv, (size_t)B * nnz * 8, cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaMemcpyAsync(host.data(), a.kv, nkv * 8, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaStreamSynchronize(st));
     return TB_OK;
-  };
-  rc = body();
-  if (rc) host_pipe_drain(hp);
-  cudaFree(dxyz); cudaFree(daed); cudaFree(dkv); cudaFree(dscr); cudaFree(dstat);
+  });
   if (rc) return rc;
   const std::vector<int32_t>& src = ts ? p->ts->ent_src : p->tile_ent;      // device order -> scatter-map entry
   for (int b = 0; b < B; ++b)
@@ -1035,19 +1048,14 @@ extern "C" int tb_adjoint(tb_plan* p, const tb_batch_in* in, const double* u, co
   cudaStream_t st = (cudaStream_t)cuda_stream;
   const int B = in->batch;
   std::lock_guard<std::mutex> lock(p->mu);
-  rc = ws_acquire(p, st);
+  rc = p->ws_order.acquire(st);
   if (rc) return rc;
   const bool smem = tb_adjoint_vec_in_smem(p->dim, p->M);
   const size_t rowN = (size_t)B * p->N * 8, nvec = smem ? 0 : (size_t)B * p->M * p->dim * 8;
   const size_t need = 2 * Arena::al(rowN) + Arena::al((size_t)B * 4) + nvec;
-  if (p->adj_bytes < need) {                    // stream-ordered: the previous call's kernels are ahead on this stream
-    if (p->adj_buf) TB_CUDA(cudaFreeAsync(p->adj_buf, st));
-    p->adj_buf = nullptr;
-    p->adj_bytes = 0;
-    TB_CUDA(cudaMallocAsync(&p->adj_buf, need, st));
-    p->adj_bytes = need;
-  }
-  char* cur = (char*)p->adj_buf;
+  rc = reserve_async(p->adj_buf, need, st);
+  if (rc) return rc;
+  char* cur = (char*)p->adj_buf.ptr;
   double* r = take<double>(cur, (size_t)B * p->N);
   double* lam = take<double>(cur, (size_t)B * p->N);
   int32_t* info_tmp = take<int32_t>(cur, (size_t)B);
@@ -1075,7 +1083,7 @@ extern "C" int tb_adjoint(tb_plan* p, const tb_batch_in* in, const double* u, co
   if (rc) return rc;
   rc = tb_launch_sens(a, num_sm, st);
   if (rc) return rc;
-  return ws_release(p, st);
+  return p->ws_order.release(st);
 }
 
 // Reverse mode of tb_solve_ragged: adjoint load, the adjoint solve through run_ragged (the same kernel as the forward of
@@ -1084,7 +1092,7 @@ extern "C" int tb_adjoint(tb_plan* p, const tb_batch_in* in, const double* u, co
 // warp (or CTA), so the host never needs the device-resident total joint count to place a second array.
 extern "C" int tb_adjoint_ragged(const tb_ragged_in* in, const double* u, const tb_adj_in* grad, const tb_adj_out* out,
                                  double* work, void* cuda_stream) {
-  int rc = check_ragged(in);
+  int rc = check_ragged(in, nullptr, true);
   if (rc) return rc;
   if (in->batch == 0) return TB_OK;
   if (!u || !grad || !out || !out->member_aed || !out->info || !work) return TB_ERR_NULL;
@@ -1136,27 +1144,6 @@ int check_modes(const tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, c
   return check_modes_args(p, in, m);
 }
 
-// The plan's modal arena for a launch of `grid` CTAs: one n x n slot of doubles per CTA, grow-only, grown stream-ordered
-// on the caller's stream, never inside a stream capture (TB_ERR_ALLOC with nothing enqueued; a warm-up call outside the
-// capture grows it).  Orders the arena after the previous call's kernels (ws_acquire): the caller launches, then
-// ws_release.  With the plan lock held.
-int modes_slots(tb_plan* p, int grid, cudaStream_t st) {
-  const size_t need = (size_t)grid * p->n * p->n * sizeof(double);
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) (void)cudaGetLastError();
-  if (p->modes_bytes < need && cap != cudaStreamCaptureStatusNone) return TB_ERR_ALLOC;
-  int rc = ws_acquire(p, st);
-  if (rc) return rc;
-  if (p->modes_bytes < need) {
-    if (p->modes_buf) TB_CUDA(cudaFreeAsync(p->modes_buf, st));
-    p->modes_buf = nullptr;
-    p->modes_bytes = 0;
-    TB_CUDA(cudaMallocAsync(&p->modes_buf, need, st));
-    p->modes_bytes = need;
-  }
-  return TB_OK;
-}
-
 // The batch and plan fields of a k_modes / k_buckling launch
 void modes_args(const tb_plan* p, const tb_batch_in* in, ModesArgs& a) {
   memset(&a, 0, sizeof(a));
@@ -1179,8 +1166,8 @@ int run_modes(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_
   if (rc) return rc;
   const int sms = p->num_sm > 0 ? p->num_sm : 148;
   const int grid = (int)std::min<int64_t>(in->batch, (int64_t)sms * per_sm);
-  if (m->consistent) {                           // the consistent mass's slots
-    rc = modes_slots(p, grid, st);
+  if (m->consistent) {                           // the consistent mass's slots: one n x n slot per CTA
+    rc = acquire_scratch(p->ws_order, p->modes_buf, (size_t)grid * p->n * p->n * sizeof(double), st);
     if (rc) return rc;
   }
   ModesArgs a;
@@ -1188,10 +1175,10 @@ int run_modes(tb_plan* p, const tb_batch_in* in, const tb_modes_in* m, const tb_
   a.n_modes = m->n_modes; a.consistent = m->consistent;
   a.jmass = m->joint_mass; a.jmass_stride = m->joint_mass_stride;
   a.eigval = out->eigval; a.modes = out->modes; a.info = out->info;
-  a.slot = m->consistent ? (double*)p->modes_buf : nullptr;
+  a.slot = m->consistent ? (double*)p->modes_buf.ptr : nullptr;
   rc = tb_launch_modes(a, p->dim, grid, threads, smem, st);
   if (rc) return rc;
-  return m->consistent ? ws_release(p, st) : TB_OK;
+  return m->consistent ? p->ws_order.release(st) : TB_OK;
 }
 
 }  // namespace
@@ -1234,58 +1221,24 @@ extern "C" int tb_modes_host(tb_plan* p, const tb_batch_in* in, const tb_modes_i
   if (rc) return rc;
   const int B = in->batch;
   if (B == 0) return TB_OK;
-  const int64_t rowJ = (int64_t)p->nJ * p->dim, rowM3 = (int64_t)p->M * 3, rowM = p->M, nm = m->n_modes;
-  if (!stride_ok(in->joint_stride, rowJ)) return TB_ERR_SIZE;
-  if (in->member_aed && !stride_ok(in->member_stride, rowM3)) return TB_ERR_SIZE;
-  if (!in->member_aed && !stride_ok(in->gene_stride, rowM)) return TB_ERR_SIZE;
-  if (m->joint_mass && !stride_ok(m->joint_mass_stride, p->nJ)) return TB_ERR_SIZE;
+  if (check_in_strides(p, in) || (m->joint_mass && !stride_ok(m->joint_mass_stride, p->nJ))) return TB_ERR_SIZE;
   rc = check_device(p);
   if (rc) return rc;
-  std::lock_guard<std::mutex> pipe_lock(g_pipe_mu);
-  std::lock_guard<std::mutex> plan_lock(p->mu);
-  HostPipe* hp = host_pipe();
-  if (!hp) return TB_ERR_ALLOC;
-  rc = async_drain(p);
-  if (rc) return rc;
-  auto cnt = [&](int64_t stride, int64_t row) { return (size_t)(stride == 0 ? row : row * B); };
-  const size_t nxyz = cnt(in->joint_stride, rowJ);
-  const size_t naed = in->member_aed ? cnt(in->member_stride, rowM3) : 0;
-  const size_t ngene = in->member_aed ? 0 : cnt(in->gene_stride, rowM);
-  const size_t ntab = in->member_aed ? 0 : (size_t)in->n_type * 3;
-  const size_t njm = m->joint_mass ? cnt(m->joint_mass_stride, p->nJ) : 0;
-  const size_t nval = (size_t)B * nm, nmode = out->modes ? (size_t)B * nm * p->N : 0;
-  size_t need = 0;
-  for (size_t bytes : {nxyz * 8, naed * 8, ngene * 4, ntab * 8, njm * 8, nval * 8, nmode * 8, (size_t)B * 4}) need += Arena::al(bytes);
-  cudaStream_t st = hp->comp;
-  auto body = [&]() -> int {
-    int r2 = arena_reserve(&p->stage_dev, &p->stage_dev_bytes, need + 4096);
+  const size_t njm = m->joint_mass ? rows(m->joint_mass_stride, p->nJ, B) : 0;
+  const size_t nval = (size_t)B * m->n_modes, nmode = out->modes ? nval * p->N : 0;
+  return host_call(p, [&](HostPipe* hp) -> int {
+    cudaStream_t st = hp->comp;
+    tb_batch_in din;
+    char* cur = nullptr;
+    int r2 = stage_in(p, in, Arena::sum({njm * 8, nval * 8, nmode * 8, (size_t)B * 4}), st, &din, &cur);
     if (r2) return r2;
-    char* cur = (char*)p->stage_dev;
-    double* dxyz = take<double>(cur, nxyz);
-    double* daed = take<double>(cur, naed);
-    int32_t* dgene = take<int32_t>(cur, ngene);
-    double* dtab = take<double>(cur, ntab);
-    double* djm = take<double>(cur, njm);
-    tb_modes_out dout = {take<double>(cur, nval), out->modes ? take<double>(cur, nmode) : nullptr, take<int32_t>(cur, (size_t)B)};
-    TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, nxyz * 8, cudaMemcpyHostToDevice, st));
-    tb_batch_in din = *in;
-    din.joint_xyz = dxyz;
-    din.force = nullptr;
-    if (in->member_aed) {
-      TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, naed * 8, cudaMemcpyHostToDevice, st));
-      din.member_aed = daed;
-      din.gene = nullptr;
-    } else {
-      TB_CUDA(cudaMemcpyAsync(dgene, in->gene, ngene * 4, cudaMemcpyHostToDevice, st));
-      TB_CUDA(cudaMemcpyAsync(dtab, in->type_table, ntab * 8, cudaMemcpyHostToDevice, st));
-      din.gene = dgene;
-      din.type_table = dtab;
-    }
     tb_modes_in dm = *m;
     if (m->joint_mass) {
+      double* djm = take<double>(cur, njm);
       TB_CUDA(cudaMemcpyAsync(djm, m->joint_mass, njm * 8, cudaMemcpyHostToDevice, st));
       dm.joint_mass = djm;
     }
+    tb_modes_out dout = {take<double>(cur, nval), out->modes ? take<double>(cur, nmode) : nullptr, take<int32_t>(cur, (size_t)B)};
     r2 = run_modes(p, &din, &dm, &dout, st);
     if (r2) return r2;
     TB_CUDA(cudaMemcpyAsync(out->eigval, dout.eigval, nval * 8, cudaMemcpyDeviceToHost, st));
@@ -1293,10 +1246,7 @@ extern "C" int tb_modes_host(tb_plan* p, const tb_batch_in* in, const tb_modes_i
     TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaStreamSynchronize(st));
     return TB_OK;
-  };
-  rc = body();
-  if (rc) host_pipe_drain(hp);
-  return rc;
+  });
 }
 
 // ---- linear buckling (DESIGN.md section 12) ---------------------------------------------------------------------------
@@ -1320,18 +1270,18 @@ int run_buckling(tb_plan* p, const tb_batch_in* in, const tb_buckling_in* bk, co
   if (rc) return rc;
   const int sms = p->num_sm > 0 ? p->num_sm : 148;
   const int grid = (int)std::min<int64_t>(in->batch, (int64_t)sms * per_sm);
-  rc = modes_slots(p, grid, st);
+  rc = acquire_scratch(p->ws_order, p->modes_buf, (size_t)grid * p->n * p->n * sizeof(double), st);
   if (rc) return rc;
   BucklingArgs a;
   memset(&a, 0, sizeof(a));
   modes_args(p, in, a.base);
   a.base.n_modes = bk->n_modes; a.base.consistent = 1;
   a.base.eigval = out->factor; a.base.modes = out->modes; a.base.info = out->info;
-  a.base.slot = (double*)p->modes_buf;
+  a.base.slot = (double*)p->modes_buf.ptr;
   a.axial = bk->axial; a.axial_stride = bk->axial_stride;
   rc = tb_launch_buckling(a, p->dim, grid, threads, smem, st);
   if (rc) return rc;
-  return ws_release(p, st);
+  return p->ws_order.release(st);
 }
 
 }  // namespace
@@ -1353,57 +1303,23 @@ extern "C" int tb_buckling_host(tb_plan* p, const tb_batch_in* in, const tb_buck
   if (rc) return rc;
   const int B = in->batch;
   if (B == 0) return TB_OK;
-  const int64_t rowJ = (int64_t)p->nJ * p->dim, rowM3 = (int64_t)p->M * 3, rowM = p->M, nm = bk->n_modes;
-  if (!stride_ok(in->joint_stride, rowJ)) return TB_ERR_SIZE;
-  if (in->member_aed && !stride_ok(in->member_stride, rowM3)) return TB_ERR_SIZE;
-  if (!in->member_aed && !stride_ok(in->gene_stride, rowM)) return TB_ERR_SIZE;
-  if (!stride_ok(bk->axial_stride, rowM)) return TB_ERR_SIZE;
+  if (check_in_strides(p, in) || !stride_ok(bk->axial_stride, p->M)) return TB_ERR_SIZE;
   rc = check_device(p);
   if (rc) return rc;
-  std::lock_guard<std::mutex> pipe_lock(g_pipe_mu);
-  std::lock_guard<std::mutex> plan_lock(p->mu);
-  HostPipe* hp = host_pipe();
-  if (!hp) return TB_ERR_ALLOC;
-  rc = async_drain(p);
-  if (rc) return rc;
-  auto cnt = [&](int64_t stride, int64_t row) { return (size_t)(stride == 0 ? row : row * B); };
-  const size_t nxyz = cnt(in->joint_stride, rowJ);
-  const size_t naed = in->member_aed ? cnt(in->member_stride, rowM3) : 0;
-  const size_t ngene = in->member_aed ? 0 : cnt(in->gene_stride, rowM);
-  const size_t ntab = in->member_aed ? 0 : (size_t)in->n_type * 3;
-  const size_t nax = cnt(bk->axial_stride, rowM);
-  const size_t nval = (size_t)B * nm, nmode = out->modes ? (size_t)B * nm * p->N : 0;
-  size_t need = 0;
-  for (size_t bytes : {nxyz * 8, naed * 8, ngene * 4, ntab * 8, nax * 8, nval * 8, nmode * 8, (size_t)B * 4}) need += Arena::al(bytes);
-  cudaStream_t st = hp->comp;
-  auto body = [&]() -> int {
-    int r2 = arena_reserve(&p->stage_dev, &p->stage_dev_bytes, need + 4096);
+  const size_t nax = rows(bk->axial_stride, p->M, B);
+  const size_t nval = (size_t)B * bk->n_modes, nmode = out->modes ? nval * p->N : 0;
+  return host_call(p, [&](HostPipe* hp) -> int {
+    cudaStream_t st = hp->comp;
+    tb_batch_in din;
+    char* cur = nullptr;
+    int r2 = stage_in(p, in, Arena::sum({nax * 8, nval * 8, nmode * 8, (size_t)B * 4}), st, &din, &cur);
     if (r2) return r2;
-    char* cur = (char*)p->stage_dev;
-    double* dxyz = take<double>(cur, nxyz);
-    double* daed = take<double>(cur, naed);
-    int32_t* dgene = take<int32_t>(cur, ngene);
-    double* dtab = take<double>(cur, ntab);
+    tb_buckling_in dbk = *bk;
     double* dax = take<double>(cur, nax);
+    TB_CUDA(cudaMemcpyAsync(dax, bk->axial, nax * 8, cudaMemcpyHostToDevice, st));
+    dbk.axial = dax;
     tb_buckling_out dout = {take<double>(cur, nval), out->modes ? take<double>(cur, nmode) : nullptr,
                             take<int32_t>(cur, (size_t)B)};
-    TB_CUDA(cudaMemcpyAsync(dxyz, in->joint_xyz, nxyz * 8, cudaMemcpyHostToDevice, st));
-    tb_batch_in din = *in;
-    din.joint_xyz = dxyz;
-    din.force = nullptr;
-    if (in->member_aed) {
-      TB_CUDA(cudaMemcpyAsync(daed, in->member_aed, naed * 8, cudaMemcpyHostToDevice, st));
-      din.member_aed = daed;
-      din.gene = nullptr;
-    } else {
-      TB_CUDA(cudaMemcpyAsync(dgene, in->gene, ngene * 4, cudaMemcpyHostToDevice, st));
-      TB_CUDA(cudaMemcpyAsync(dtab, in->type_table, ntab * 8, cudaMemcpyHostToDevice, st));
-      din.gene = dgene;
-      din.type_table = dtab;
-    }
-    TB_CUDA(cudaMemcpyAsync(dax, bk->axial, nax * 8, cudaMemcpyHostToDevice, st));
-    tb_buckling_in dbk = *bk;
-    dbk.axial = dax;
     r2 = run_buckling(p, &din, &dbk, &dout, st);
     if (r2) return r2;
     TB_CUDA(cudaMemcpyAsync(out->factor, dout.factor, nval * 8, cudaMemcpyDeviceToHost, st));
@@ -1411,36 +1327,18 @@ extern "C" int tb_buckling_host(tb_plan* p, const tb_batch_in* in, const tb_buck
     TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaStreamSynchronize(st));
     return TB_OK;
-  };
-  rc = body();
-  if (rc) host_pipe_drain(hp);
-  return rc;
+  });
 }
 
 // ---- modal analysis of ragged batches ---------------------------------------------------------------------------------
 namespace {
 
-// the launch's free-DOF bound: max_free, or every DOF of the largest truss up to the kernel's limit
-int modes_ragged_bound(const tb_ragged_in* in, const tb_modes_ragged_in* m) {
-  return m->max_free ? m->max_free : std::min(in->dim * in->max_joint, TB_SMALL_MAX_DOF);
-}
-
-// Argument checks shared by tb_modes_ragged, tb_modes_ragged_host and tb_modes_adjoint_ragged (in, m non-null): the
-// sizes, then (B > 0) n_modes against the bound, the packed arrays and the ragged size limits; the device last (as
-// tb_solve_ragged, also for B = 0)
+// Argument checks shared by tb_modes_ragged, tb_modes_ragged_host and tb_modes_adjoint_ragged (in, m non-null):
+// check_ragged's, then the device (as tb_solve_ragged, also for B = 0)
 int check_modes_ragged_args(const tb_ragged_in* in, const tb_modes_ragged_in* m) {
-  if (in->dim != 2 && in->dim != 3) return TB_ERR_DIM;
-  if (in->batch < 0 || in->max_joint < 0 || in->max_member < 0) return TB_ERR_SIZE;
-  if (m->consistent != 0 && m->consistent != 1) return TB_ERR_SIZE;
-  if (m->max_free < 0 || m->max_free > TB_SMALL_MAX_DOF || m->n_modes < 1) return TB_ERR_SIZE;
-  if (in->batch > 0) {
-    if (m->n_modes > modes_ragged_bound(in, m)) return TB_ERR_SIZE;
-    if (!in->joint_off || !in->member_off || !in->joint_xyz || !in->support || !in->conn || !in->member_aed)
-      return TB_ERR_NULL;
-    if ((int64_t)in->max_joint * in->dim > TB_RAGGED_MAX_DOF || in->max_member > TB_RAGGED_MAX_MEMBER) return TB_ERR_TOO_LARGE;
-  }
-  if (!have_device()) return TB_ERR_NO_DEVICE;
-  return TB_OK;
+  const int rc = check_ragged(in, m, false);
+  if (rc) return rc;
+  return have_device() ? TB_OK : TB_ERR_NO_DEVICE;
 }
 
 int check_modes_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const tb_modes_ragged_out* out) {
@@ -1470,13 +1368,12 @@ int run_modes_ragged(const tb_ragged_in* in, const tb_modes_ragged_in* m, const 
   if (!m->consistent) return tb_launch_modes_ragged(a, in->dim, grid, threads, smem, st);
   EnvScratch& S = g_env[dev & (TB_MAX_DEVICES - 1)];
   std::lock_guard<std::mutex> lock(S.mu);
-  bool capturing = false;
-  rc = env_acquire(S, (size_t)grid * bound * bound * sizeof(double), st, &capturing);
+  rc = acquire_scratch(S.order, S.buf, (size_t)grid * bound * bound * sizeof(double), st);
   if (rc) return rc;
-  a.slot = (double*)S.buf;
+  a.slot = (double*)S.buf.ptr;
   rc = tb_launch_modes_ragged(a, in->dim, grid, threads, smem, st);
   if (rc) return rc;
-  return env_release(S, st, capturing);
+  return S.order.release(st);
 }
 
 }  // namespace
@@ -1496,51 +1393,27 @@ extern "C" int tb_modes_ragged_host(const tb_ragged_in* in, const tb_modes_ragge
   if (rc) return rc;
   const int B = in->batch, d = in->dim;
   if (B == 0) return TB_OK;
-  if (in->joint_off[0] != 0 || in->member_off[0] != 0) return TB_ERR_SIZE;
-  for (int b = 0; b < B; ++b) {
-    const int64_t nj = in->joint_off[b + 1] - in->joint_off[b], nm = in->member_off[b + 1] - in->member_off[b];
-    if (nj < 0 || nm < 0) return TB_ERR_SIZE;
-    if (nj > in->max_joint || nm > in->max_member) return TB_ERR_TOO_LARGE;
-  }
-  const size_t SJ = (size_t)in->joint_off[B], SM = (size_t)in->member_off[B], nm = (size_t)m->n_modes;
-  std::lock_guard<std::mutex> lock(g_pipe_mu);
-  HostPipe* hp = host_pipe();
-  if (!hp) return TB_ERR_ALLOC;
-  int dev = 0;
-  TB_CUDA(cudaGetDevice(&dev));
-  void*& rag_dev = g_rag_dev[dev & (TB_MAX_DEVICES - 1)];
-  size_t& rag_bytes = g_rag_dev_bytes[dev & (TB_MAX_DEVICES - 1)];
-  auto body = [&]() -> int {
-    size_t need = 0;
-    for (size_t bytes : {(size_t)(B + 1) * 8, (size_t)(B + 1) * 8, SJ * d * 8, SJ, SM * 8, SM * 24, m->joint_mass ? SJ * 8 : 0,
-                         (size_t)B * nm * 8, out->modes ? nm * d * SJ * 8 : 0, (size_t)B * 4, (size_t)B * 4})
-      need += Arena::al(bytes);
-    int r2 = arena_reserve(&rag_dev, &rag_bytes, need + 4096);
-    if (r2) return r2;
+  rc = check_ragged_offsets_host(in);
+  if (rc) return rc;
+  const size_t SJ = (size_t)in->joint_off[B], nm = (size_t)m->n_modes;
+  return host_call(nullptr, [&](HostPipe* hp) -> int {
     cudaStream_t st = hp->comp;
-    char* cur = (char*)rag_dev;
-    tb_ragged_in din = *in;
-    din.joint_off = take<int64_t>(cur, B + 1);
-    din.member_off = take<int64_t>(cur, B + 1);
-    din.joint_xyz = take<double>(cur, SJ * d);
-    din.support = take<uint8_t>(cur, SJ);
-    din.conn = take<int32_t>(cur, SM * 2);
-    din.member_aed = take<double>(cur, SM * 3);
-    din.force = nullptr;
+    tb_ragged_in din;
+    char* cur = nullptr;
+    int r2 = stage_ragged_in(in, Arena::sum({m->joint_mass ? SJ * 8 : 0, (size_t)B * nm * 8, out->modes ? nm * d * SJ * 8 : 0,
+                                             (size_t)B * 4, (size_t)B * 4}), st, &din, &cur);
+    if (r2) return r2;
     tb_modes_ragged_in dm = *m;
-    dm.joint_mass = m->joint_mass ? take<double>(cur, SJ) : nullptr;
+    if (m->joint_mass) {
+      double* djm = take<double>(cur, SJ);
+      TB_CUDA(cudaMemcpyAsync(djm, m->joint_mass, SJ * 8, cudaMemcpyHostToDevice, st));
+      dm.joint_mass = djm;
+    }
     tb_modes_ragged_out dout;
     dout.eigval = take<double>(cur, (size_t)B * nm);
     dout.modes = out->modes ? take<double>(cur, nm * d * SJ) : nullptr;
     dout.n_free = take<int32_t>(cur, (size_t)B);
     dout.info = take<int32_t>(cur, (size_t)B);
-    TB_CUDA(cudaMemcpyAsync((void*)din.joint_off, in->joint_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
-    TB_CUDA(cudaMemcpyAsync((void*)din.member_off, in->member_off, (B + 1) * 8, cudaMemcpyHostToDevice, st));
-    TB_CUDA(cudaMemcpyAsync((void*)din.joint_xyz, in->joint_xyz, SJ * d * 8, cudaMemcpyHostToDevice, st));
-    TB_CUDA(cudaMemcpyAsync((void*)din.support, in->support, SJ, cudaMemcpyHostToDevice, st));
-    TB_CUDA(cudaMemcpyAsync((void*)din.conn, in->conn, SM * 8, cudaMemcpyHostToDevice, st));
-    TB_CUDA(cudaMemcpyAsync((void*)din.member_aed, in->member_aed, SM * 24, cudaMemcpyHostToDevice, st));
-    if (m->joint_mass) TB_CUDA(cudaMemcpyAsync((void*)dm.joint_mass, m->joint_mass, SJ * 8, cudaMemcpyHostToDevice, st));
     r2 = run_modes_ragged(&din, &dm, &dout, st);
     if (r2) return r2;
     TB_CUDA(cudaMemcpyAsync(out->eigval, dout.eigval, (size_t)B * nm * 8, cudaMemcpyDeviceToHost, st));
@@ -1549,10 +1422,7 @@ extern "C" int tb_modes_ragged_host(const tb_ragged_in* in, const tb_modes_ragge
     TB_CUDA(cudaMemcpyAsync(out->info, dout.info, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
     TB_CUDA(cudaStreamSynchronize(st));
     return TB_OK;
-  };
-  rc = body();
-  if (rc) host_pipe_drain(hp);
-  return rc;
+  });
 }
 
 // Reverse mode of tb_modes_ragged: one k_modes_sens_ragged launch, no scratch (always capturable)

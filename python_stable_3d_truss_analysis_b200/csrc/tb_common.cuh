@@ -67,6 +67,17 @@ void tb_prof_end(int slot, cudaStream_t st);
 // calls of tb_solve_host_async in flight per plan: one uploading, one computing, one downloading
 constexpr int TB_ASYNC_SLOTS = 3;
 
+struct DevBuf { void* ptr = nullptr; size_t bytes = 0; };   // grow-only device buffer (tb_api.cu: reserve_sync / _async)
+// Cross-stream order of a scratch buffer (tb_api.cu): acquire makes a call on another stream than the last user's wait
+// for its event, release records it after the call's last kernel; neither does anything inside a stream capture.
+struct StreamOrder {
+  cudaEvent_t ev = nullptr;
+  cudaStream_t last = nullptr;   // stream of the last call that used the buffer
+  bool used = false;
+  int acquire(cudaStream_t st);
+  int release(cudaStream_t st);
+};
+
 struct tb_plan {
   int dim = 0, nJ = 0, M = 0, N = 0, n = 0, s = 0;
   int n_resist = 0, stable = 0, path = 0, n_pad = 0, nt = 0;
@@ -154,35 +165,24 @@ struct tb_plan {
   TsPlan* ts = nullptr;
 
   // grow-only device workspace of the blocked path.  One workspace per plan: `mu` serialises the calls that enqueue work
-  // on it (and the growth of the arenas), `ws_event` orders its use across streams (recorded after the last kernel of a
-  // call; a call on another stream waits for it first).  See the threading contract in truss_b200.h.
-  void* ws = nullptr;
-  size_t ws_bytes = 0;
+  // on it (and the growth of the arenas), `ws_order` orders its use, and that of adj_buf and modes_buf, across streams.
+  // See the threading contract in truss_b200.h.
+  DevBuf ws;
   std::mutex mu;
-  cudaEvent_t ws_event = nullptr;
-  cudaStream_t ws_stream = nullptr;   // stream of the last call that used the workspace
-  bool ws_used = false;
+  StreamOrder ws_order;
   // grow-only staging for the *_host entry points
-  void* stage_dev = nullptr;
-  size_t stage_dev_bytes = 0;
-  void* stage_pinned = nullptr;
-  size_t stage_pinned_bytes = 0;
+  DevBuf stage_dev;
   // dense u / ext of a call that asks for the compact outputs only (grow-only, [capacity][N] each)
-  double* compact_u = nullptr;
-  double* compact_ext = nullptr;
-  size_t compact_cap_u = 0, compact_cap_ext = 0;   // systems
+  DevBuf compact_u, compact_ext;
   // tb_adjoint scratch (grow-only, grown stream-ordered on the caller's stream): adjoint load and solution [B][N] each,
   // status [B], and the per-member vectors [B][M][d] when they do not fit shared memory
-  void* adj_buf = nullptr;
-  size_t adj_bytes = 0;
+  DevBuf adj_buf;
   // modal scratch of tb_modes' consistent mass and of tb_buckling (grow-only, grown stream-ordered): one n x n slot per CTA
   // of the launch
-  void* modes_buf = nullptr;
-  size_t modes_bytes = 0;
+  DevBuf modes_buf;
   // pipelined host calls (tb_solve_host_async): TB_ASYNC_SLOTS more staging arenas used in turn by consecutive calls,
   // the events that chain a call's copies and kernels, and the ticket counters (submitted / known to be complete)
-  void* stage_async[TB_ASYNC_SLOTS] = {};
-  size_t stage_async_bytes[TB_ASYNC_SLOTS] = {};
+  DevBuf stage_async[TB_ASYNC_SLOTS];
   cudaEvent_t async_in[TB_ASYNC_SLOTS] = {}, async_k[TB_ASYNC_SLOTS] = {}, async_done[TB_ASYNC_SLOTS] = {};
   uint64_t async_submitted = 0, async_completed = 0;
 };

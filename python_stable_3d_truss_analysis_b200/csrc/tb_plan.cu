@@ -501,6 +501,7 @@ extern "C" int tb_plan_create(const tb_topology* topo, tb_plan** plan_out) {
 
 extern "C" void tb_plan_destroy(tb_plan* p) {
   if (!p) return;
+  auto free_buf = [](DevBuf& b) { cudaFree(b.ptr); };
   tb_ts_destroy(p->ts, p->device >= 0);
   p->ts = nullptr;
   if (p->device < 0) {
@@ -513,8 +514,8 @@ extern "C" void tb_plan_destroy(tb_plan* p) {
   cudaFree(p->d_dof2free);
   cudaFree(p->d_sup_idx);
   cudaFree(p->d_free_ref);
-  cudaFree(p->compact_u);
-  cudaFree(p->compact_ext);
+  free_buf(p->compact_u);
+  free_buf(p->compact_ext);
   cudaFree(p->d_ent_row);
   cudaFree(p->d_ent_col);
   cudaFree(p->d_ent_ptr);
@@ -539,22 +540,21 @@ extern "C" void tb_plan_destroy(tb_plan* p) {
   cudaFree(p->d_prod_k);
   cudaFree(p->d_inc_ptr);
   cudaFree(p->d_inc_mem);
-  if (p->ws_event) {
-    cudaEventSynchronize(p->ws_event);          // (the last call's kernels may still read the adjoint scratch)
-    cudaEventDestroy(p->ws_event);
+  if (p->ws_order.ev) {
+    cudaEventSynchronize(p->ws_order.ev);       // (the last call's kernels may still read the adjoint scratch)
+    cudaEventDestroy(p->ws_order.ev);
   }
-  cudaFree(p->adj_buf);
-  cudaFree(p->modes_buf);
-  cudaFree(p->ws);
-  cudaFree(p->stage_dev);
+  free_buf(p->adj_buf);
+  free_buf(p->modes_buf);
+  free_buf(p->ws);
+  free_buf(p->stage_dev);
   for (int i = 0; i < TB_ASYNC_SLOTS; ++i) {
     if (p->async_done[i]) cudaEventSynchronize(p->async_done[i]);     // (a pipelined call may still be in flight)
-    cudaFree(p->stage_async[i]);
+    free_buf(p->stage_async[i]);
     if (p->async_in[i]) cudaEventDestroy(p->async_in[i]);
     if (p->async_k[i]) cudaEventDestroy(p->async_k[i]);
     if (p->async_done[i]) cudaEventDestroy(p->async_done[i]);
   }
-  if (p->stage_pinned) cudaFreeHost(p->stage_pinned);
   delete p;
 }
 
