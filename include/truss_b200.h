@@ -348,6 +348,31 @@ int tb_buckling(tb_plan* plan, const tb_batch_in* in, const tb_buckling_in* bk, 
                 void* cuda_stream);
 int tb_buckling_host(tb_plan* plan, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out);
 
+/* Reverse mode of tb_buckling (DESIGN.md section 12): the gradients of L = sum_q g_eigval[q] lambda_q with respect to the
+ * joint positions, the member properties and the member forces N, from the forward's K-normalised modes:
+ *   dlambda/dp = lambda phi^T (dK/dp) phi + lambda^2 phi^T (dK_G/dp) phi     (simple factor, phi^T K_ff phi = 1)
+ * with N held fixed; out->axial is dL/dN.  One pass over the members per system; nothing is solved.  To differentiate
+ * through a static solve that produced N, pass out->axial as grad->axial to tb_adjoint with that solve's u.  `g` is the
+ * forward's output in tb_modes_adj_in: eigval = the factors, modes (required here), info, and g_eigval the cotangent of
+ * the factors.  `in` and `bk` are the forward's arguments (bk->n_modes, bk->axial and its stride are read).  Explicit
+ * member properties only (member_aed; a gene / type-table batch returns TB_ERR_NULL: pass type_table[gene]).  Argument
+ * errors come before TB_ERR_NO_DEVICE, in tb_buckling's order: TB_ERR_NULL for bk, g, out, bk->axial or any array of g,
+ * TB_ERR_SIZE for a negative axial_stride, then the checks of tb_modes (TB_ERR_SIZE for n_modes outside [1, n],
+ * TB_ERR_TOO_LARGE for n > 160); B = 0 is a no-op.  A mode with g_eigval[q] == 0 or a factor that is not finite (+inf:
+ * not critical) is skipped whatever its cotangent: its gradient is 0, never NaN.  The density gradient is 0 (density
+ * enters neither K nor K_G).  A system whose forward info is not 0 gets zero gradients.  Gradients are written per system
+ * even for an input shared with stride 0 (reducing them is the caller's job).  Enqueues on the stream, never
+ * synchronises and uses no scratch (always capturable).  Repeated factors (e.g. a symmetric column braced alike in two
+ * directions): as tb_modes_adjoint, only a cotangent equal across a cluster gives a basis-independent gradient. */
+typedef struct {
+  double* joint_xyz;          /* [B][nJ][d]  any may be NULL to skip it */
+  double* member_aed;         /* [B][M][3]   (a, e, density) */
+  double* axial;              /* [B][M]      dL/dN */
+} tb_buckling_adj_out;
+
+int tb_buckling_adjoint(tb_plan* plan, const tb_batch_in* in, const tb_buckling_in* bk, const tb_modes_adj_in* g,
+                        const tb_buckling_adj_out* out, void* cuda_stream);
+
 /* GA.GetFitness for B genes (ga.py:139-149); `full` may be NULL or receive the full results. */
 int tb_fitness(tb_plan* plan, const tb_batch_in* in, double allow_stress, double allow_displace,
                const tb_fit_out* fit, const tb_batch_out* full, void* cuda_stream);

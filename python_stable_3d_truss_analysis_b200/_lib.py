@@ -185,6 +185,10 @@ class TbBucklingOut(C.Structure):
     _fields_ = [("factor", C.c_void_p), ("modes", C.c_void_p), ("info", C.c_void_p)]
 
 
+class TbBucklingAdjOut(C.Structure):
+    _fields_ = [("joint_xyz", C.c_void_p), ("member_aed", C.c_void_p), ("axial", C.c_void_p)]
+
+
 class TbModesRaggedIn(C.Structure):
     _fields_ = [("n_modes", C.c_int32), ("consistent", C.c_int32), ("joint_mass", C.c_void_p), ("max_free", C.c_int32)]
 
@@ -200,7 +204,7 @@ class TbRaggedIn(C.Structure):
 
 
 EXPORTS = ["tb_plan_create", "tb_plan_destroy", "tb_plan_query", "tb_plan_set_path", "tb_plan_get_maps",
-           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_modes_adjoint", "tb_modes_ragged", "tb_modes_ragged_host", "tb_modes_adjoint_ragged", "tb_buckling", "tb_buckling_host", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
+           "tb_plan_get_scatter", "tb_solve", "tb_solve_host", "tb_solve_host_async", "tb_host_wait", "tb_solve_loadcases", "tb_solve_loadcases_host", "tb_adjoint", "tb_modes", "tb_modes_host", "tb_modes_adjoint", "tb_modes_ragged", "tb_modes_ragged_host", "tb_modes_adjoint_ragged", "tb_buckling", "tb_buckling_host", "tb_buckling_adjoint", "tb_fitness", "tb_fitness_host", "tb_solve_ragged",
            "tb_solve_ragged_host", "tb_solve_ragged_env", "tb_ragged_env_order", "tb_ragged_limits", "tb_adjoint_ragged", "tb_ga_init", "tb_ga_step", "tb_augment_ragged", "tb_json_scan", "tb_json_fill", "tb_gencube_limits", "tb_gencube", "tb_gencube_pack", "tb_pinned_alloc", "tb_pinned_free", "tb_small_path_limits", "tb_fp64_peak", "tb_rsqrt_probe", "tb_div_probe", "tb_profile_enable", "tb_profile_read",
            "tb_launch_count", "tb_strerror", "tb_version", "tb_small_path_fits", "tb_debug_assemble_host", "tb_plan_ts_info", "tb_plan_ts_array", "tb_ts_phase_read"]
 
@@ -242,6 +246,8 @@ def lib():
                                           C.POINTER(TbModesAdjOut), vp]
     L.tb_buckling.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBucklingIn), C.POINTER(TbBucklingOut), vp]
     L.tb_buckling_host.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBucklingIn), C.POINTER(TbBucklingOut)]
+    L.tb_buckling_adjoint.argtypes = [vp, C.POINTER(TbBatchIn), C.POINTER(TbBucklingIn), C.POINTER(TbModesAdjIn),
+                                      C.POINTER(TbBucklingAdjOut), vp]
     L.tb_fitness.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut), vp]
     L.tb_fitness_host.argtypes = [vp, C.POINTER(TbBatchIn), dbl, dbl, C.POINTER(TbFitOut), C.POINTER(TbBatchOut)]
     L.tb_solve_ragged.argtypes = [C.POINTER(TbRaggedIn), C.POINTER(TbBatchOut), vp]
@@ -781,6 +787,35 @@ class Plan:
         st = torch.cuda.current_stream() if stream is None else stream
         bo = TbBucklingOut(_ptr(out["factor"]), _ptr(out.get("modes")), _ptr(out["info"]))
         check(lib().tb_buckling(self._h, C.byref(bi), C.byref(bk), C.byref(bo), C.c_void_p(st.cuda_stream)))
+        return out
+
+    def buckling_adjoint_device(self, B, xyz, aed, axial, fwd, g_factor, out, n_modes=None, axial_stride=None,
+                                stream=None):
+        """Reverse mode of ``buckling_device`` (tb_buckling_adjoint) on torch CUDA tensors: the gradients of
+        sum_q g_factor[:, q] * lambda_q with the member forces held fixed, and their gradient dL/dN.  ``axial`` (and
+        ``axial_stride``) are the forward's; ``fwd`` is the dict ``buckling_device`` returned for the same inputs (its
+        "factor", "modes" and "info" are read); ``g_factor`` is [B, n_modes]; ``out`` maps "joint_xyz" [B, nJ, d],
+        "member_aed" [B, M, 3] and "axial" [B, M] to preallocated tensors (missing or None = skipped).  ``n_modes=None``
+        takes the forward's count.  Gradients are per system, also for shared inputs.  Pass ``out["axial"]`` as the
+        "axial" cotangent of ``adjoint_device`` to differentiate through the static solve that produced ``axial``."""
+        import torch
+
+        if aed is None:
+            raise ValueError("aed is required: there are no gradients with respect to a gene type table")
+        k = int(fwd["factor"].shape[-1]) if n_modes is None else int(n_modes)
+        for name, t, shape in (("fwd['factor']", fwd.get("factor"), (B, k)), ("fwd['modes']", fwd.get("modes"), (B, k, self.N)),
+                               ("fwd['info']", fwd.get("info"), (B,)), ("g_factor", g_factor, (B, k))):
+            if t is None or tuple(t.shape) != shape or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous tensor of shape {list(shape)}")
+        keep = []
+        bi = self._batch_in(B, xyz, aed, None, None, np.zeros(self.N), keep)
+        bi.force, bi.force_stride = None, 0            # (not read)
+        bk = self._buckling_in(B, axial, k, axial_stride, keep)
+        ai = TbModesAdjIn(_ptr(fwd["factor"]), _ptr(fwd["modes"]), _ptr(fwd["info"]), _ptr(g_factor))
+        ao = TbBucklingAdjOut(_ptr(out.get("joint_xyz")), _ptr(out.get("member_aed")), _ptr(out.get("axial")))
+        st = torch.cuda.current_stream() if stream is None else stream
+        check(lib().tb_buckling_adjoint(self._h, C.byref(bi), C.byref(bk), C.byref(ai), C.byref(ao),
+                                        C.c_void_p(st.cuda_stream)))
         return out
 
     def fitness_device(self, B, xyz, force, gene, type_table, allow_stress, allow_displace, out, aed=None, stream=None):

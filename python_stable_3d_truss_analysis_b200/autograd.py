@@ -26,6 +26,17 @@ over the members, nothing solved).  Example -- a frequency penalty for sizing, s
 
 ``modes_ragged(packed, xyz, aed, joint_mass)`` does the same for a ragged batch (``tb_modes_ragged`` /
 ``tb_modes_adjoint_ragged``).
+
+``buckling(truss, xyz, aed, force=force)`` runs the static solve and then linear buckling (``tb_buckling``, DESIGN.md
+section 12) under its member forces, and returns load factors that backpropagate to the joint coordinates, the member
+properties and the loads (``tb_buckling_adjoint``, then ``tb_adjoint`` for the member forces' share).  Example -- a
+weight-minimising sizing step with the stability constraint "critical load factor >= 1.5" as a penalty::
+
+    aed = torch.cat([area[:, None], aed0[:, 1:]], 1)  # area: the design variables, requires_grad=True
+    weight = autograd.solve(truss, aed=aed)["weight"]
+    factor = autograd.buckling(truss, aed=aed, n_modes=6)["factor"]
+    loss = weight + c * torch.relu(1.5 - factor[..., 0])
+    loss.backward()                                   # area.grad
 """
 from __future__ import annotations
 
@@ -34,7 +45,7 @@ import torch
 
 from . import _lib
 
-__all__ = ["solve", "solve_ragged", "modes", "modes_ragged"]
+__all__ = ["solve", "solve_ragged", "modes", "modes_ragged", "buckling"]
 
 
 def per_input(g, x):
@@ -284,6 +295,90 @@ def modes(truss, xyz=None, aed=None, joint_mass=None, n_modes=None, consistent=F
     out = {"eigval": eigval, "modes": shapes, "info": info}
     if bx is None and ba is None and bm is None:
         out = {key: v[0] for key, v in out.items()}
+    return out
+
+
+class _Buckling(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, xyz, aed, axial, plan, B, n_modes):
+        out = {"modes": torch.empty(B, n_modes, plan.N, dtype=torch.float64, device=xyz.device)}   # (the backward needs them)
+        plan.buckling_device(B, xyz, axial, aed=aed, n_modes=n_modes, out=out)
+        ctx.save_for_backward(xyz, aed, axial, out["factor"], out["modes"], out["info"])
+        ctx.plan, ctx.B, ctx.n_modes = plan, B, n_modes
+        ctx.mark_non_differentiable(out["modes"], out["info"])
+        ctx.set_materialize_grads(False)
+        return out["factor"], out["modes"], out["info"]
+
+    @staticmethod
+    def backward(ctx, g_factor, _g_modes, _g_info):
+        if g_factor is None:
+            return (None,) * 6
+        xyz, aed, axial, factor, modes_, info = ctx.saved_tensors
+        plan, B = ctx.plan, ctx.B
+        f64 = dict(dtype=torch.float64, device=xyz.device)
+        need_x, need_a, need_n = ctx.needs_input_grad[:3]
+        res = {"joint_xyz": torch.empty(B, plan.nJ, plan.dim, **f64) if need_x else None,
+               "member_aed": torch.empty(B, plan.M, 3, **f64) if need_a else None,
+               "axial": torch.empty(B, plan.M, **f64) if need_n else None}
+        fwd = {"factor": factor, "modes": modes_, "info": info}
+        plan.buckling_adjoint_device(B, xyz, aed, axial, fwd, g_factor.contiguous(), res, n_modes=ctx.n_modes)
+        return (per_input(res["joint_xyz"], xyz), per_input(res["member_aed"], aed), per_input(res["axial"], axial),
+                None, None, None)
+
+
+def buckling(truss, xyz=None, aed=None, axial=None, force=None, n_modes=None):
+    """Linear buckling (``Truss.SolveBuckling``) for a uniform batch, with load factors differentiable with respect to
+    ``xyz``, ``aed`` and the loads or the member forces.
+
+    Inputs are float64 CUDA tensors: ``xyz`` [nJ, d] joint positions, ``aed`` [M, 3] (a, e, density) per member, and
+    either ``axial`` [M], the member forces N of the reference state (tension positive), or ``force`` [N], dense loads
+    (index joint * d + axis); each either unbatched (shared by every system) or with a leading batch dimension B.
+    ``xyz`` / ``aed`` / ``force`` None mean the truss's own values, held constant.  With ``axial`` None the member forces
+    come from ``solve(truss, xyz, aed, force)``, so the gradients also flow through the static solve (one adjoint solve)
+    and reach the loads.  ``n_modes`` (None = all n free DOFs) lowest factors.
+
+    Returns ``{"factor": [B, k], "modes": [B, k, N], "info": [B] int32, "axial": [B, M]}`` (without the batch dimension
+    when no input has one): the load factors ascending (+inf for modes no positive multiple of N reaches), the
+    K-normalised buckling modes (0 at supported DOFs), the per-system status of ``include/truss_b200.h`` and the member
+    forces used.  Only ``factor`` (and ``axial``, when it comes from the solve) is differentiable
+    (dlambda/dp = lambda phi^T dK/dp phi + lambda^2 phi^T dK_G/dp phi); a failed system has zero outputs and zero
+    gradients, and a factor at +inf has zero gradient whatever its cotangent.
+
+    Repeated factors (symmetric structures such as a column braced alike in two directions have exactly repeated
+    critical pairs): a single factor of a cluster is not differentiable, only functions symmetric in the cluster's
+    factors are.  A loss that treats every factor alike -- ``relu(1.5 - factor).sum()`` -- sends equal cotangents to a
+    cluster and gets its exact gradient, whatever basis of the cluster the forward returned.  A loss that singles out
+    one factor of a cluster (``factor[..., 0]`` when the lowest factor is a pair) gets a basis-dependent directional
+    value; so does any loss when ``n_modes`` cuts a cluster in two.  Ask for enough modes to keep the clusters you use
+    whole."""
+    if axial is not None and force is not None:
+        raise ValueError("give the member forces (axial) or the loads (force), not both")
+    pxyz, psup, pconn, paed, pforce = truss._pack()
+    plan = truss._get_plan(psup, pconn)
+    given = [t for t in (xyz, aed, axial, force) if isinstance(t, torch.Tensor)]
+    device = given[0].device if given else torch.device("cuda", torch.cuda.current_device())
+    xyz, bx = _input(xyz, pxyz, (plan.nJ, plan.dim), device, "xyz")
+    aed, ba = _input(aed, paed, (plan.M, 3), device, "aed")
+    if axial is not None:
+        axial, bl = _input(axial, None, (plan.M,), device, "axial")
+    else:
+        force, bl = _input(force, pforce, (plan.N,), device, "force")
+    for name, t in (("xyz", xyz), ("aed", aed), ("axial", axial), ("force", force)):
+        if t is not None and t.device != device:
+            raise TypeError(f"{name} must be on the device of the other inputs ({device})")
+    sizes = {b for b in (bx, ba, bl) if b is not None}
+    if len(sizes) > 1:
+        raise ValueError(f"batched inputs disagree on the batch size: {sorted(sizes)}")
+    B = sizes.pop() if sizes else 1
+    k = plan.n if n_modes is None else int(n_modes)
+    with torch.cuda.device(device):
+        if axial is None:
+            axial = solve(truss, xyz, aed, force)["axial"]
+        factor, shapes, info = _Buckling.apply(xyz, aed, axial, plan, B, k)
+    out = {"factor": factor, "modes": shapes, "info": info}
+    if bx is None and ba is None and bl is None:
+        out = {key: v[0] for key, v in out.items()}
+    out["axial"] = axial
     return out
 
 

@@ -1297,6 +1297,32 @@ extern "C" int tb_buckling(tb_plan* p, const tb_batch_in* in, const tb_buckling_
   return run_buckling(p, in, bk, out, (cudaStream_t)cuda_stream);
 }
 
+// Reverse mode of tb_buckling: one k_buckling_sens launch, no scratch (so no plan lock and always capturable).  Argument
+// errors in check_buckling's order: the pointers (a gene batch has no member gradient), the axial stride, tb_modes' checks
+extern "C" int tb_buckling_adjoint(tb_plan* p, const tb_batch_in* in, const tb_buckling_in* bk, const tb_modes_adj_in* g,
+                                   const tb_buckling_adj_out* out, void* cuda_stream) {
+  if (!p || !in || !bk || !g || !out) return TB_ERR_NULL;
+  if (!bk->axial || !g->eigval || !g->modes || !g->info || !g->g_eigval) return TB_ERR_NULL;
+  if (in->batch > 0 && !in->member_aed) return TB_ERR_NULL;      // (no gradients with respect to a type table)
+  if (bk->axial_stride < 0) return TB_ERR_SIZE;
+  const tb_modes_in m = {bk->n_modes, 0, nullptr, 0};
+  int rc = check_modes_args(p, in, &m);
+  if (rc) return rc;
+  if (in->batch == 0) return TB_OK;
+  rc = check_device(p);
+  if (rc) return rc;
+  BucklingSensArgs a;
+  memset(&a, 0, sizeof(a));
+  a.batch = in->batch; a.nJ = p->nJ; a.M = p->M; a.N = p->N; a.n_modes = bk->n_modes;
+  a.xyz = in->joint_xyz; a.xyz_stride = in->joint_stride;
+  a.aed = in->member_aed; a.aed_stride = in->member_stride;
+  a.axial = bk->axial; a.axial_stride = bk->axial_stride;
+  a.conn = p->d_conn; a.dof2free = p->d_dof2free; a.inc_ptr = p->d_inc_ptr; a.inc_mem = p->d_inc_mem;
+  a.factor = g->eigval; a.modes = g->modes; a.info = g->info; a.g_factor = g->g_eigval;
+  a.g_xyz = out->joint_xyz; a.g_aed = out->member_aed; a.g_axial = out->axial;
+  return tb_launch_buckling_sens(a, p->dim, (cudaStream_t)cuda_stream);
+}
+
 // Host buffers: staged through the plan's arena like tb_modes_host (plain cudaMemcpyAsync on the compute stream)
 extern "C" int tb_buckling_host(tb_plan* p, const tb_batch_in* in, const tb_buckling_in* bk, const tb_buckling_out* out) {
   int rc = check_buckling(p, in, bk, out);

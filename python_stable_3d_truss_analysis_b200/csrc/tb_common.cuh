@@ -412,6 +412,18 @@ struct ModesSensArgs {
 };
 int tb_launch_modes_sens(const ModesSensArgs& a, int dim, cudaStream_t st);
 
+// Reverse mode of linear buckling (tb_buckling_adjoint): one warp per system, no scratch
+struct BucklingSensArgs {
+  int batch, nJ, M, N, n_modes;
+  const double* xyz; int64_t xyz_stride;
+  const double* aed; int64_t aed_stride;
+  const double* axial; int64_t axial_stride;     // [B][M] the forward's member forces, stride 0 = shared
+  const int32_t* conn; const int32_t* dof2free; const int32_t* inc_ptr; const int32_t* inc_mem;
+  const double* factor; const double* modes; const int32_t* info; const double* g_factor;   // [B][k], [B][k][N], [B], [B][k]
+  double* g_xyz; double* g_aed; double* g_axial;                                            // outputs, null = skipped
+};
+int tb_launch_buckling_sens(const BucklingSensArgs& a, int dim, cudaStream_t st);
+
 // Modal analysis of a ragged batch (tb_modes_ragged): packed layout of tb_ragged_in, one CTA per truss
 struct ModesRagArgs {
   int batch, max_joint, max_member, max_free, n_modes, consistent;   // max_free: the launch's free-DOF bound

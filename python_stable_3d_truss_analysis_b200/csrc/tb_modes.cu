@@ -23,7 +23,8 @@
 // lambda (-K_G) phi), which differs in step 1 and in its output step; see there.
 //
 // k_modes_sens<DIM> is the reverse mode (tb_modes_adjoint): eigenvalue gradients from the forward's modes, below, and
-// k_modes_sens_ragged<DIM> its ragged form (tb_modes_adjoint_ragged).
+// k_modes_sens_ragged<DIM> its ragged form (tb_modes_adjoint_ragged); k_buckling_sens<DIM> is the reverse mode of
+// tb_buckling (tb_buckling_adjoint): load-factor gradients from the forward's modes, in the same shape.
 #include <cfloat>
 #include <math_constants.h>
 
@@ -1000,6 +1001,110 @@ __global__ void __launch_bounds__(32 * SENS_WARPS, 3) k_modes_sens_ragged(const 
   }
 }
 
+// ---- reverse mode of linear buckling (tb_buckling_adjoint): for a simple critical mode with phi^T K_ff phi = 1,
+//   dlambda/dp = lambda phi^T (dK/dp) phi + lambda^2 phi^T (dK_G/dp) phi,
+// the member forces N held fixed (their own gradient is an output: the caller closes the chain through the static
+// solve's adjoint).  k_buckling_sens<DIM> has k_modes_sens' shape: one warp per system, lanes over members write the
+// (a, e, density) row and the dL/dN row, then lanes over joints gather the geometry vector over the plan's incidence
+// lists, recomputing the member body.  Modes are summed in ascending q; a mode with a zero cotangent or a factor that is
+// not finite (+inf: not critical, its row is zero) is skipped whatever its cotangent, so lambda 0 inf never turns into
+// NaN.  No atomics, no shared memory, no scratch.
+
+// Member m of one system over its first nq modes: ga = dL/d(a, e), gn = dL/dN_m and v = dL/d(x_j1) = -dL/d(x_j0), with
+// t = c.dphi, s = |dphi|^2 and g = N / L (phi^T K_m phi = k t^2, phi^T K_G,m phi = g (s - t^2)):
+//   dlambda/da = lambda (e/L) t^2,  dlambda/de = lambda (a/L) t^2,  dlambda/dN = lambda^2 (s - t^2) / L,
+//   dlambda/dd = lambda (k/L) (2 t dphi - 3 t^2 c) + lambda^2 (g/L) (3 t^2 c - 2 t dphi - s c)
+template <int DIM>
+__device__ __forceinline__ void buckling_sens_member(const PlanFree<DIM>& fr, const int32_t* conn, int N, int nq,
+                                                     const double* xyz, const double* aed_m, double axial_m,
+                                                     const double* lam, const double* gl, const double* phi, int m,
+                                                     double ga[2], double& gn, double v[DIM]) {
+  const int j0 = conn[2 * m], j1 = conn[2 * m + 1];
+  const double ar = aed_m[0], e = aed_m[1];
+  double dx[DIM], c[DIM], k, w;
+  const double len = tb_member_geom<DIM>(xyz, j0, j1, ar, e, aed_m[2], dx, c, k, w);
+  const double il = 1.0 / len, el = e * il, al = ar * il, kl = k * il, gll = axial_m * il * il;
+  ga[0] = ga[1] = gn = 0.0;
+#pragma unroll
+  for (int i = 0; i < DIM; ++i) v[i] = 0.0;
+  for (int q = 0; q < nq; ++q) {
+    const double g = gl[q], lq = lam[q];
+    if (g == 0.0 || !isfinite(lq)) continue;
+    const double* ph = phi + (int64_t)q * N;
+    double p0[DIM], p1[DIM], dp[DIM], t = 0.0, s = 0.0;
+    mode_at<DIM>(fr, ph, j0, p0);
+    mode_at<DIM>(fr, ph, j1, p1);
+#pragma unroll
+    for (int i = 0; i < DIM; ++i) {
+      dp[i] = p1[i] - p0[i];
+      t = fma(c[i], dp[i], t);
+      s = fma(dp[i], dp[i], s);
+    }
+    const double gq = g * lq, gq2 = gq * lq, t2 = t * t;
+    ga[0] += gq * (el * t2);
+    ga[1] += gq * (al * t2);
+    gn += gq2 * ((s - t2) * il);
+#pragma unroll
+    for (int i = 0; i < DIM; ++i) {
+      const double a2 = 2.0 * t * dp[i] - 3.0 * t2 * c[i];
+      v[i] += gq * (kl * a2) - gq2 * (gll * (a2 + s * c[i]));
+    }
+  }
+}
+
+template <int DIM>
+__global__ void __launch_bounds__(32 * SENS_WARPS, 3) k_buckling_sens(const BucklingSensArgs a) {
+  const int lane = threadIdx.x & 31;
+  const int nm = a.n_modes;
+  const PlanFree<DIM> fr{a.dof2free};
+  for (int b = blockIdx.x * SENS_WARPS + (threadIdx.x >> 5); b < a.batch; b += gridDim.x * SENS_WARPS) {
+    double* gx = a.g_xyz ? a.g_xyz + (int64_t)b * a.N : nullptr;
+    double* ga = a.g_aed ? a.g_aed + (int64_t)b * a.M * 3 : nullptr;
+    double* gn = a.g_axial ? a.g_axial + (int64_t)b * a.M : nullptr;
+    if (a.info[b] != 0) {                      // failed system: zero gradients, never NaN
+      for (int i = lane; i < a.N; i += 32)
+        if (gx) gx[i] = 0.0;
+      for (int i = lane; i < 3 * a.M; i += 32)
+        if (ga) ga[i] = 0.0;
+      for (int i = lane; i < a.M; i += 32)
+        if (gn) gn[i] = 0.0;
+      continue;
+    }
+    const double* xyz = a.xyz + b * a.xyz_stride;
+    const double* aed = a.aed + b * a.aed_stride;
+    const double* ax = a.axial + b * a.axial_stride;
+    const double* lam = a.factor + (int64_t)b * nm;
+    const double* gl = a.g_factor + (int64_t)b * nm;
+    const double* phi = a.modes + (int64_t)b * nm * a.N;
+    if (ga || gn)
+      for (int m = lane; m < a.M; m += 32) {
+        double r[2], rn, v[DIM];
+        buckling_sens_member<DIM>(fr, a.conn, a.N, nm, xyz, aed + 3 * m, ax[m], lam, gl, phi, m, r, rn, v);
+        if (ga) {
+          ga[3 * m] = r[0];
+          ga[3 * m + 1] = r[1];
+          ga[3 * m + 2] = 0.0;                 // the density enters neither K nor K_G
+        }
+        if (gn) gn[m] = rn;
+      }
+    if (!gx) continue;
+    for (int J = lane; J < a.nJ; J += 32) {
+      double s[DIM];
+#pragma unroll
+      for (int i = 0; i < DIM; ++i) s[i] = 0.0;
+      for (int p = a.inc_ptr[J]; p < a.inc_ptr[J + 1]; ++p) {   // (+) at the member's joint 1, (-) at its joint 0
+        const int me = a.inc_mem[p], m = me >> 1;
+        double r[2], rn, v[DIM];
+        buckling_sens_member<DIM>(fr, a.conn, a.N, nm, xyz, aed + 3 * m, ax[m], lam, gl, phi, m, r, rn, v);
+#pragma unroll
+        for (int i = 0; i < DIM; ++i) s[i] += (me & 1) ? v[i] : -v[i];
+      }
+#pragma unroll
+      for (int i = 0; i < DIM; ++i) gx[J * DIM + i] = s[i];
+    }
+  }
+}
+
 // persistent grid of a warp-per-system kernel: the resident CTAs of the device (the occupancy query costs more than the
 // launch: cached per device and kernel)
 template <int WHICH>
@@ -1087,6 +1192,18 @@ int tb_launch_modes_sens_ragged(const ModesSensRagArgs& a, int dim, cudaStream_t
   if (rc) return rc;
   if (dim == 3) k_modes_sens_ragged<3><<<grid, 32 * SENS_WARPS, 0, st>>>(a);
   else k_modes_sens_ragged<2><<<grid, 32 * SENS_WARPS, 0, st>>>(a);
+  tb_count_launch();
+  return (int)cudaGetLastError();
+}
+
+int tb_launch_buckling_sens(const BucklingSensArgs& a, int dim, cudaStream_t st) {
+  if (a.batch <= 0) return 0;
+  int grid = 0;
+  int rc = dim == 3 ? sens_grid<23>((const void*)k_buckling_sens<3>, a.batch, &grid)
+                    : sens_grid<22>((const void*)k_buckling_sens<2>, a.batch, &grid);
+  if (rc) return rc;
+  if (dim == 3) k_buckling_sens<3><<<grid, 32 * SENS_WARPS, 0, st>>>(a);
+  else k_buckling_sens<2><<<grid, 32 * SENS_WARPS, 0, st>>>(a);
   tb_count_launch();
   return (int)cudaGetLastError();
 }
